@@ -112,7 +112,7 @@ def run_reference(args):
     synth = importlib.import_module(PKG + ".synth")
     from oracle import refbind
     if not refbind.available("f64"):
-        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/libref_f64.so not built (needs /root/reference at build time)"}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/libref_f64.so not built (needs B200RT_REFERENCE at build time)"}))
         return
     scn, locs, dirs = make_workload(synth, args.ref_los)
     R = refbind.RefModel(scn, "f64")
@@ -153,6 +153,29 @@ def cuda_array(ptr, shape, dtype="<f8"):
     a = _A()
     a.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": dtype, "data": (int(ptr), False), "version": 2}
     return a
+
+
+DUMP_K_ROWS = 256            # rows of K written by --dump-outputs: 256 x 5841 x 8 B = 12 MB
+DUMP_MAX_LOS = 1 << 20       # lines of sight written by --dump-outputs: 4 results x 2^20 x 8 B = 32 MB
+DUMP_SEED = 1234
+
+
+def dump_outputs(out_dir, ctx, K_t, n_vox):
+    """What the last timed step computed, as a caller of that path receives it, as out_dir/<name>.npy (float64): the
+    solution vectors in full, a fixed seeded sample of the rows of K and, above DUMP_MAX_LOS lines of sight, a fixed
+    seeded sample of them.  The same arguments give the same inputs, so two builds can be compared file for file."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(DUMP_SEED)
+    out = ctx.solution(0)                                       # S, S0, tau_species_ss, tau_absorber_ss
+    rows = np.sort(rng.choice(n_vox, min(DUMP_K_ROWS, n_vox), replace=False))
+    out["influence_matrix_rows"] = K_t[torch.from_numpy(rows).to(K_t.device)].cpu().numpy()
+    los = ctx.los_download()                                    # brightness, optical depths, column density: (1, n_los)
+    n_los = ctx.n_los
+    pick = np.sort(rng.choice(n_los, DUMP_MAX_LOS, replace=False)) if n_los > DUMP_MAX_LOS else slice(None)
+    out.update({k: v[0, pick] for k, v in los.items()})
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def run_ours(args):
@@ -331,6 +354,8 @@ def run_ours(args):
             recs.append(rec)
     if sampler:
         sampler.stop_flag = True
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ctx, K_t, n_vox)
 
     def reduce_max(x):
         if world == 1:
@@ -359,12 +384,12 @@ def run_ours(args):
 
     # ---- e2e arm (host buffers)
     erecs = []
-    for it in range(1 + max(1, min(args.steps, 3))):
+    for it in range(args.warmup + args.steps):
         flush.zero_()
         barrier()
         r = e2e_step()
         barrier()
-        if it >= 1:
+        if it >= args.warmup:
             erecs.append(r)
     Ke = len(erecs)
     e_infl = reduce_max(sum(r["w_influence"] for r in erecs))
@@ -498,7 +523,7 @@ def run_ours(args):
     # binding use): rank 0 drives all N GPUs, host buffers in and out; the other ranks' GPUs are free by now
     if world > 1 and not args.no_in_process:
         try:
-            line["in_process"] = run_in_process(binding, torch, scn, tabs, (b_, T_, s_, g_), los_all, world, max(2, min(args.steps, 3)))
+            line["in_process"] = run_in_process(binding, torch, scn, tabs, (b_, T_, s_, g_), los_all, world, args.warmup, args.steps)
         except Exception as ex:
             line["in_process"] = {"error": str(ex)}
 
@@ -552,7 +577,7 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def run_in_process(binding, torch, scn, tabs, scalars, los_all, n_dev, reps):
+def run_in_process(binding, torch, scn, tabs, scalars, los_all, n_dev, warmup, reps):
     """source function + brightness through ONE handle over n_dev GPUs of this process, host buffers in and out"""
     b_, T_, s_, g_ = scalars
     ctx = binding.Context(precision=binding.F64, devices=list(range(n_dev)))
@@ -562,7 +587,7 @@ def run_in_process(binding, torch, scn, tabs, scalars, los_all, n_dev, reps):
     los_pin = [torch.from_numpy(np.ascontiguousarray(a)).pin_memory().numpy() for a in los_all]
     out_pin = [torch.empty((1, n_los), dtype=torch.float64).pin_memory().numpy() for _ in range(4)]
     rec = []
-    for it in range(1 + reps):
+    for it in range(warmup + reps):
         w0 = time.perf_counter()
         ctx.set_singlet(0, 1, b_, T_, s_, g_, tabs)             # H2D: 8 tables, every device
         ctx.generate_S()                                        # rows on every device -> device 0's K, solve, S to all
@@ -575,7 +600,7 @@ def run_in_process(binding, torch, scn, tabs, scalars, los_all, n_dev, reps):
         w2 = time.perf_counter()
         ph.update({k: ctx.kernel_ms(p)[0] for k, p in (("los_traverse", binding.PH_TRAVERSE), ("brightness", binding.PH_BRIGHTNESS))})
         assert np.isfinite(out["brightness"]).all() and sol["S0"].max() <= 1.0
-        if it >= 1:
+        if it >= warmup:
             rec.append(dict(source_function_ms=(w1 - w0) * 1e3, brightness_ms=(w2 - w1) * 1e3, job_ms=(w2 - w0) * 1e3, steps=steps, **ph))
     ctx.close()
     m = lambda k: sum(r[k] for r in rec) / len(rec)
@@ -601,7 +626,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the IPH and sweep measurements")
     ap.add_argument("--no-in-process", action="store_true", help="N > 1: skip the one-handle in-process arm on rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (one process only)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs writes the results of one process; run it without torchrun")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

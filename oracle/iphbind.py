@@ -9,7 +9,8 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "libiph_oracle.so")
-REF_TABLE = "/root/reference/src/quemerais_IPH_model/fsm99td12v20t80"   # only in the build container
+_REF = os.environ.get("B200RT_REFERENCE")                      # the reference's source tree, where one is at hand
+REF_TABLE = os.path.join(_REF, "src", "quemerais_IPH_model", "fsm99td12v20t80") if _REF else None
 
 _fp = np.ctypeslib.ndpointer(dtype=np.float32, flags="C_CONTIGUOUS")
 _dp = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")

@@ -37,5 +37,5 @@ def refbind():
     """the reference's own hot-path source built in place (oracle/_ref); absent => skip"""
     from oracle import refbind as rb
     if not rb.available("f64"):
-        pytest.skip("oracle/_ref not built (needs /root/reference; see oracle/Makefile)")
+        pytest.skip("oracle/_ref not built (needs the reference's source: B200RT_REFERENCE, see oracle/Makefile)")
     return rb

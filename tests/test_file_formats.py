@@ -7,12 +7,15 @@ facade's writers (host/observation_fit.cpp write_S_file / write_influence) are g
 same bytes.  Number formatting on the reference side is Eigen's operator<< (default IOFormat): Eigen is not vendored in
 the reference tree, so oracle/standin/Eigen/Dense restates Eigen 3.4.0's print_matrix (src/Core/IO.h: every coefficient
 printed at the stream's precision, all of them right-aligned to the widest) -- that one algorithm is restated, everything
-else in the files is the reference's own code."""
+else in the files is the reference's own code.  Without the reference build, test_save_S_and_influence_bytes_pins holds
+the writers to the bytes of tests/golden/ref_pins.json on the oracle's arrays (pinned bit for bit to the reference's)."""
 import filecmp
 import importlib
 
 import numpy as np
 import pytest
+
+import ref_pins
 
 
 @pytest.fixture(scope="module")
@@ -47,3 +50,10 @@ def test_save_S_and_influence_bytes(synth, refbind, hb, tmp_path, shape, n_em):
     assert filecmp.cmp(ref_K, our_K, shallow=False), "save_influence bytes differ"
     txt = open(our_S).read()
     assert txt.startswith("radial boundaries [cm]: ") and "  For SZA = " in txt and "    Source function: " in txt
+
+
+@pytest.mark.parametrize("shape,n_em", ref_pins.FILE_CASES)
+def test_save_S_and_influence_bytes_pins(synth, oraclebind, hb, shape, n_em):
+    scn = synth.make_scenario(*shape, n_em=n_em, sza_T_contrast=0.1)
+    out = ref_pins.file_case(scn, oraclebind.OracleModel(scn, "f64"), hb)
+    ref_pins.Pins.load().check(f"file_{'x'.join(map(str, shape))}_{n_em}", out)

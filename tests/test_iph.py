@@ -33,9 +33,9 @@ def test_oracle_reproduces_golden_fixture():
 
 
 def table_file(tmp_path):
-    """the reference's own table file where it exists (the build container), else the same READ sequence written
-    from the committed fixture tables"""
-    if os.path.exists(iphbind.REF_TABLE):
+    """the reference's own table file where B200RT_REFERENCE names its tree, else the same READ sequence written from
+    the committed fixture tables"""
+    if iphbind.REF_TABLE and os.path.exists(iphbind.REF_TABLE):
         return iphbind.REF_TABLE
     from util import write_iph_table_file
     path = str(tmp_path / "iph_table_from_fixture")

@@ -2,13 +2,15 @@
 H_lyman_multiplet_test.hpp; BASELINE.json configs[4] (ii)/(iii)).
 
 CPU: the oracle restatement (oracle/multiplet_oracle.inc.c) against the reference's own source built in place
-(bit for bit, double and float) and against golden fixtures made from it.
+(bit for bit, double and float), against what that comparison compared against (tests/golden/ref_pins.*, for machines
+without the reference build) and against golden fixtures made from it.
 GPU: the CUDA path (b200rt_set_multiplet ...) against the oracle and the fixtures, 1e-6 (double) / 1e-4 (float)."""
 import os
 
 import numpy as np
 import pytest
 
+import ref_pins
 from util import TOL, UNDERFLOW, rel_err, same_bits
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -31,7 +33,7 @@ def bits_equal(a, b):
 @pytest.mark.parametrize("shape", [(8, 6, 4, 4), (12, 8, 5, 6)])
 def test_oracle_matches_reference(synth, multbind, prec, kind, shape):
     if not multbind.ref_available(prec):
-        pytest.skip("oracle/_ref/libref_mult_*.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libref_mult_*.so not built (needs B200RT_REFERENCE)")
     scn = synth.make_multiplet_scenario(kind, *shape, sza_T_contrast=0.1)
     R, O = multbind.RefMultiplet(scn, prec), multbind.OracleMultiplet(scn, prec)
     assert (R.n_lines, R.n_mult, R.n_lower, R.n_upper, R.n_lambda) == synth.MULT_DIMS[kind]
@@ -70,7 +72,7 @@ def test_oracle_matches_reference(synth, multbind, prec, kind, shape):
 def test_oracle_matches_reference_default_grid(synth, multbind):
     """reference default grid 40x20x7x12 (observation_fit.hpp:44-47), O I 102.6: a strided subset of rows"""
     if not multbind.ref_available("f64"):
-        pytest.skip("oracle/_ref/libref_mult_*.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libref_mult_*.so not built (needs B200RT_REFERENCE)")
     scn = synth.make_multiplet_scenario(0, 40, 20, 7, 12)
     R, O = multbind.RefMultiplet(scn), multbind.OracleMultiplet(scn)
     _, ns_r = R.build_rows(0, scn.n_vox, 97)
@@ -80,6 +82,26 @@ def test_oracle_matches_reference_default_grid(synth, multbind):
     rows = np.concatenate([np.arange(v * NUP, (v + 1) * NUP) for v in range(0, scn.n_vox, 97)])
     assert same_bits(R.K()[rows], O.K()[rows])
     assert same_bits(R.vectors()["S0"][rows], O.vectors()["S0"][rows])
+
+
+@pytest.mark.parametrize("prec", ["f64", "f32"])
+@pytest.mark.parametrize("kind", KINDS)
+@pytest.mark.parametrize("shape", [(8, 6, 4, 4), (12, 8, 5, 6)])
+def test_oracle_matches_reference_pins(synth, multbind, prec, kind, shape):
+    pins = ref_pins.Pins.load()
+    case = f"mult{kind}_{'x'.join(map(str, shape))}_{prec}"
+    Sr = pins.sourcefns[case][0]
+    O = multbind.OracleMultiplet(synth.make_multiplet_scenario(kind, *shape, sza_T_contrast=0.1), prec)
+    out, own, res = ref_pins.mult_case(synth, O, Sr)       # brightness with the stored source function, as above
+    pins.check(case, out)
+    assert res < 1e-12 if prec == "f64" else res < 1e-4
+    floor = 1e-30 if prec == "f64" else float(np.abs(Sr).max())
+    assert rel_err(Sr, own, floor=floor) < (1e-7 if prec == "f64" else 1e-3)
+
+
+def test_oracle_matches_reference_default_grid_pins(synth, multbind):
+    O = multbind.OracleMultiplet(synth.make_multiplet_scenario(0, 40, 20, 7, 12))
+    ref_pins.Pins.load().check("mult0_D", ref_pins.mult_grid_D_case(synth, O))
 
 
 def test_singlet_through_multiplet_is_the_singlet(synth, multbind, oraclebind):

@@ -1,10 +1,12 @@
 """Pin oracle/rt_oracle.c against the reference's own source built in place (oracle/_ref).
 
-Runs only where oracle/_ref/*.so exists (this container, or a box it was shipped to).
+The live comparisons run only where oracle/_ref/*.so is built; the *_pins tests hold the oracle to what those
+comparisons compared against, stored in tests/golden/ref_pins.* (tests/ref_pins.py), everywhere.
 """
 import numpy as np
 import pytest
 
+import ref_pins
 from util import assert_lists_equal, rel_err, same_bits
 
 SHAPES = [(8, 6, 4, 4), (12, 8, 5, 6), (20, 12, 6, 8)]
@@ -76,3 +78,33 @@ def test_default_grid_D(synth, oraclebind, refbind):
         assert rel_err(R.vectors(e)["S0"], O.vectors(e)["S0"]) == 0.0
         assert rel_err(R.vectors(e)["S"], O.vectors(e)["S"], floor=1e-30) < 1e-7
     assert t > 0
+
+
+@pytest.fixture(scope="module")
+def pins():
+    return ref_pins.Pins.load()
+
+
+@pytest.mark.parametrize("prec", ["f64", "f32"])
+@pytest.mark.parametrize("shape", SHAPES)
+def test_oracle_matches_reference_pins(synth, oraclebind, pins, prec, shape):
+    case = f"singlet_{'x'.join(map(str, shape))}_{prec}"
+    S = pins.sourcefns[case]
+    O = oraclebind.OracleModel(synth.make_scenario(*shape, n_em=2, sza_T_contrast=0.1), prec)
+    out, own, res = ref_pins.singlet_case(synth, O, S)      # brightness with the stored source functions, as above
+    pins.check(case, out)
+    for e in range(2):
+        assert res[e] < (1e-12 if prec == "f64" else 1e-4)
+        floor = 1e-30 if prec == "f64" else float(np.abs(S[e]).max())
+        assert rel_err(S[e], own[e], floor=floor) < (1e-7 if prec == "f64" else 1e-3)
+
+
+def test_reference_rmethod_altitude_pins(synth, pins):
+    pins.check("rmethod_altitude", {"radial_boundaries": synth.make_scenario(12, 8, 5, 6, n_em=1).rb})
+
+
+def test_default_grid_D_pins(synth, oraclebind, pins):
+    out, own = ref_pins.grid_D_case(synth, oraclebind.OracleModel(synth.make_scenario(40, 20, 7, 12, n_em=2), "f64"))
+    pins.check("singlet_D", out)
+    for e in range(2):
+        assert rel_err(pins.sourcefns["singlet_D"][e], own[e], floor=1e-30) < 1e-7

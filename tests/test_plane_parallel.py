@@ -2,12 +2,14 @@
 source function only -- the reference has no interp_weights on this grid (:304-311).
 
 CPU: the oracle restatement against the reference's own source built in place and against the
-golden fixture made from it.  GPU: the CUDA path (b200rt_set_grid_pp) against oracle and fixture."""
+golden fixture made from it (and, without the reference build, against what the comparison with it compared against:
+tests/golden/ref_pins.*).  GPU: the CUDA path (b200rt_set_grid_pp) against oracle and fixture."""
 import os
 
 import numpy as np
 import pytest
 
+import ref_pins
 from util import TOL, UNDERFLOW, assert_lists_equal, rel_err, same_bits
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -45,6 +47,20 @@ def test_oracle_matches_reference_pp(synth, oraclebind, refbind, prec, shape):
         Sr = R.vectors(e)["S"]
         floor = 1e-30 if prec == "f64" else float(np.abs(Sr).max())
         assert rel_err(Sr, O.vectors(e)["S"], floor=floor) < (1e-7 if prec == "f64" else 1e-3)
+
+
+@pytest.mark.parametrize("prec", ["f64", "f32"])
+@pytest.mark.parametrize("shape", SHAPES)
+def test_oracle_matches_reference_pp_pins(synth, oraclebind, prec, shape):
+    pins = ref_pins.Pins.load()
+    case = f"pp_{'x'.join(map(str, shape))}_{prec}"
+    out, own, res = ref_pins.pp_case(oraclebind.OracleModel(synth.make_scenario_pp(*shape, n_em=2), prec))
+    pins.check(case, out)
+    for e in range(2):
+        assert res[e] < (1e-12 if prec == "f64" else 1e-4)
+        Sr = pins.sourcefns[case][e]
+        floor = 1e-30 if prec == "f64" else float(np.abs(Sr).max())
+        assert rel_err(Sr, own[e], floor=floor) < (1e-7 if prec == "f64" else 1e-3)
 
 
 def underflow_floor(Ka, Kb, prec):

@@ -1,8 +1,8 @@
 """Drop-in check of SURVEY.md 8(b): the reference's OWN Cython binding (python/py_corona_sim.pyx), compiled unchanged and
 in place against this repository's observation_fit facade (oracle/build_pyx.py -> oracle/_ref/py_corona_sim/, module name
 py_corona_sim_gpu as the reference's CUDA build), must build, expose every method of Pyobservation_fit, and -- on the
-GPU box -- give the numbers of the facade's C handles.  Needs /root/reference to build; the GPU box uses the prebuilt
-module that travels with the snapshot."""
+GPU -- give the numbers of the facade's C handles.  Built where B200RT_REFERENCE names the reference's source tree;
+otherwise a module built before is used."""
 import glob
 import importlib
 import os
@@ -14,6 +14,7 @@ import pytest
 from util import rel_err
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = os.environ.get("B200RT_REFERENCE")     # the reference's source tree, where one is at hand
 OUT = os.path.join(ROOT, "oracle", "_ref", "py_corona_sim")
 PKG = "3d_planetary_rt_model_b200"
 
@@ -32,12 +33,12 @@ lyman_singlet_brightness corona_model_git_hash""".split()
 
 @pytest.fixture(scope="module")
 def module():
-    if os.path.exists("/root/reference/python/py_corona_sim.pyx"):
+    if REF and os.path.exists(os.path.join(REF, "python", "py_corona_sim.pyx")):
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import build_pyx
         build_pyx.build(verbose=False)
     if not glob.glob(os.path.join(OUT, "py_corona_sim_gpu*.so")):
-        pytest.skip("oracle/_ref/py_corona_sim not built (needs /root/reference; python oracle/build_pyx.py)")
+        pytest.skip("oracle/_ref/py_corona_sim not built (needs B200RT_REFERENCE; python oracle/build_pyx.py)")
     if OUT not in sys.path:
         sys.path.insert(0, OUT)
     return importlib.import_module("py_corona_sim_gpu")

@@ -10,11 +10,12 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = os.environ.get("B200RT_REFERENCE")     # the reference's source tree, where one is at hand
 OUT = os.path.join(ROOT, "oracle", "_ref", "py_corona_sim_fast")
 
 
 def built():
-    if os.path.exists("/root/reference/python/py_corona_sim.pyx"):
+    if REF and os.path.exists(os.path.join(REF, "python", "py_corona_sim.pyx")):
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import build_pyx
         build_pyx.build(verbose=False, fast=True)
@@ -23,7 +24,7 @@ def built():
 
 def test_fast_binding_builds_and_keeps_the_reference_class():
     if not built():
-        pytest.skip("oracle/_ref/py_corona_sim_fast not built (needs /root/reference; python oracle/build_pyx.py)")
+        pytest.skip("oracle/_ref/py_corona_sim_fast not built (needs B200RT_REFERENCE; python oracle/build_pyx.py)")
     code = ("import sys; sys.path.insert(0, %r); import py_corona_sim_gpu as m; "
             "assert issubclass(m.Pyobservation_fit_b200, m.Pyobservation_fit); "
             "print(len([x for x in dir(m.Pyobservation_fit) if not x.startswith('_')]))" % OUT)

@@ -18,7 +18,7 @@ pytestmark = pytest.mark.gpu
 def test_reference_gpu_members_match_its_cpu_members(synth, prec, shape, n_em):
     from oracle import refbind
     if not refbind.available(prec, "b200"):
-        pytest.skip("oracle/_ref/libref_b200_*.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libref_b200_*.so not built (needs B200RT_REFERENCE at build time)")
     tol = TOL[prec]
     scn = synth.make_scenario(*shape, n_em=n_em, sza_T_contrast=0.1)
     cpu = refbind.RefModel(scn, prec, variant="b200")
