@@ -563,9 +563,19 @@ class GpuMultiplet:
         self.ctx.influence(v0, v1)
         return self.ctx.kernel_ms(PH_INFLUENCE)[0] * 1e-3, self.ctx.last_step_count()
 
+    def build_ranges(self, ranges):
+        """the element rows of the source voxels in `ranges` (ascending, disjoint: multi.partition_interleaved), as one
+        rank of a distributed solve holds them"""
+        self.ctx.influence_ranges(ranges)
+        return self.ctx.kernel_ms(PH_INFLUENCE)[0] * 1e-3, self.ctx.last_step_count()
+
     def solve(self):
         self.ctx.solve()
         return self.ctx.residual(0)
+
+    def last_solve_steps(self):
+        """GMRES steps of the last distributed (or GMRES-chosen) solve"""
+        return self.ctx.last_solve_steps()
 
     def K(self):
         return self.ctx.influence_matrix(0)

@@ -167,6 +167,10 @@ inline bool is64(const b200rt_ctx *c) { return c->precision == B200RT_F64; }
 int influence(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges);
 int solve(b200rt_ctx *c, bool reset_timer);
 int solve_emission(b200rt_ctx *c, int e);   // one singlet emission only (device group: emission e on its owner device)
+// b200rt_solve's choice of the GMRES (solve_krylov.cu) over the LU: a grid of B200RT_KRYLOV_MIN_N voxels or more (default
+// 2048) whose rows were all built by this context; B200RT_SOLVER = lu | gmres overrides the size.  The caller adds the
+// capacity limit (B200RT_KRYLOV_MAX_N unknowns) and that the rows exist.
+bool use_gmres(const b200rt_ctx *c);
 int set_singlet(b200rt_ctx *c, int e, const double *const arr[8]);
 // ---- api_brightness.cu  (los_download_slice / brightness_slice are declared in common.hpp)
 int brightness_resident(b200rt_ctx *c, int n_subsamples);
@@ -178,7 +182,7 @@ int traverse_los(b200rt_ctx *c, long long capacity, int *len, int *exits_bottom,
                  long long *n_entries);
 // ---- api_multiplet.cu
 int set_multiplet(b200rt_ctx *c, const double *const arr[6]);
-int mult_influence(b200rt_ctx *c, int v_begin, int v_end);
+int mult_influence(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges);
 int mult_solve(b200rt_ctx *c, bool reset_timer);
 int mult_brightness(b200rt_ctx *c, int n_subsamples);
 int mult_los_download(b200rt_ctx *c, double *const dst[4], long long stride, long long offset);

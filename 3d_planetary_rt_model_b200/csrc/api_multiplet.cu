@@ -61,8 +61,10 @@ int set_multiplet_impl(b200rt_ctx *c, const double *const arr[6]) {
   return rc;
 }
 
+// ranges: the source-voxel ranges [begin, end) this call builds the rows of (all n_upper element rows of each voxel);
+// several ranges are the interleaved shards of a distributed solve, marched as one list as in influence_impl
 template <class Real>
-int mult_influence_impl(b200rt_ctx *c, int v_begin, int v_end) {
+int mult_influence_impl(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges) {
   GridView<Real> &g = gv<Real>(c);
   Multiplet &M = c->mult;
   const b200rt_multiplet_desc &d = M.d;
@@ -71,26 +73,43 @@ int mult_influence_impl(b200rt_ctx *c, int v_begin, int v_end) {
   PhaseTimer::reset(c);
   B200RT_CUDA(c, cudaMemsetAsync(c->work_counter.p, 0, 2 * sizeof(int), c->stream));
   B200RT_CUDA(c, cudaMemsetAsync(c->step_counter.p, 0, sizeof(unsigned long long), c->stream));
-  if (v_end > v_begin)
-    B200RT_CUDA(c, cudaMemsetAsync(M.K.as<double>() + (size_t) v_begin * d.n_upper * ne, 0,
-                                   (size_t) (v_end - v_begin) * d.n_upper * ne * sizeof(double), c->stream));
+  int n_rows = 0;
+  for (auto &r : ranges) {
+    n_rows += r.second - r.first;
+    if (r.second > r.first)
+      B200RT_CUDA(c, cudaMemsetAsync(M.K.as<double>() + (size_t) r.first * d.n_upper * ne, 0,
+                                     (size_t) (r.second - r.first) * d.n_upper * ne * sizeof(double), c->stream));
+  }
+  const bool mapped = ranges.size() > 1;
+  if (mapped) {
+    std::vector<int> vox_of;
+    vox_of.reserve(n_rows);
+    for (auto &r : ranges) for (int v = r.first; v < r.second; v++) vox_of.push_back(v);
+    B200RT_CUDA(c, c->vox_map.ensure((size_t) n_rows * sizeof(int)));
+    B200RT_CUDA(c, cudaMemcpyAsync(c->vox_map.p, vox_of.data(), (size_t) n_rows * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    B200RT_CUDA(c, cudaStreamSynchronize(c->stream));   // (vox_of is pageable and goes out of scope)
+  }
+  const int first_voxel = ranges.empty() ? 0 : ranges[0].first;
   const long long cap_rays = batch_capacity(c, sizeof(Real));
-  const int vox_per_batch = (int) std::max<long long>(1, std::min<long long>(cap_rays / g.n_rays, v_end - v_begin));
+  const int vox_per_batch = (int) std::max<long long>(1, std::min<long long>(cap_rays / g.n_rays, n_rows));
   ListView<Real> lv;
   const long long need = std::max<long long>((long long) vox_per_batch * g.n_rays, n_vox);
   if (int rc = ensure_lists<Real>(c, need, &lv)) return rc;
   int *overflow = c->work_counter.as<int>() + 1;
   MultView<Real> mv = mult_view<Real>(c);
-  for (int vb = v_begin; vb < v_end; vb += vox_per_batch) {
-    const int ve = std::min(v_end, vb + vox_per_batch);
+  for (int lb = 0; lb < n_rows; lb += vox_per_batch) {
+    const int le = std::min(n_rows, lb + vox_per_batch);
+    GridView<Real> gb = g;
+    int vb = first_voxel + lb, ve = first_voxel + le;      // unmapped: the voxel range itself
+    if (mapped) { gb.vox_map = c->vox_map.as<int>() + lb; vb = 0; ve = le - lb; }
     {
       PhaseTimer t(c, PH_TRAVERSE);
-      B200RT_CUDA(c, launch_traverse_voxel_rays<Real>(g, vb, ve, lv, overflow, c->stream));
+      B200RT_CUDA(c, launch_traverse_voxel_rays<Real>(gb, vb, ve, lv, overflow, c->stream));
       t.stop(1);
     }
     {
       PhaseTimer t(c, PH_INFLUENCE);
-      B200RT_CUDA(c, launch_mult_influence<Real>(d, g, mv, vb, ve, lv, M.K.as<double>(), c->work_counter.as<int>(),
+      B200RT_CUDA(c, launch_mult_influence<Real>(d, gb, mv, vb, ve, lv, M.K.as<double>(), c->work_counter.as<int>(),
                                                  c->step_counter.as<unsigned long long>(), c->stream));
       t.stop(1);
       DBG(c, "multiplet influence march");
@@ -126,14 +145,23 @@ int mult_influence_impl(b200rt_ctx *c, int v_begin, int v_end) {
   PhaseTimer::collect(c);
   c->last_steps = (long long) steps;
   M.have_K = true; M.have_S = false;
+  c->built_ranges = ranges;
   return B200RT_OK;
 }
 
 int mult_solve_impl(b200rt_ctx *c, bool reset_timer) {
   Multiplet &M = c->mult;
   const int ne = c->hg.n_vox * M.d.n_upper;
-  if (reset_timer) PhaseTimer::reset(c);
   if (!M.have_K) return fail(c, B200RT_ERR_STATE, "b200rt_solve: influence matrix not built");
+  // the singlet's rule (api_source_function.cu, solve_impl): grids of B200RT_KRYLOV_MIN_N voxels and more whose rows were
+  // all built here take the GMRES over the n_el elements, the LU decides when it does not converge
+  if (use_gmres(c) && ne <= B200RT_KRYLOV_MAX_N) {
+    void *block = nullptr;
+    if (int rc = exchange_block(c, &block)) return rc;
+    const int rc = solve_distributed(c, 0, 1, &block, reset_timer);
+    if (rc != B200RT_ERR_NOT_DOMINANT) return rc;
+  }
+  if (reset_timer) PhaseTimer::reset(c);
   PhaseTimer t(c, PH_SOLVE);
   SolveResult r = {0, 0, 0};
   // multiplet_CFR_emission::pre_solve is empty: kernel = I - K (multiplet_CFR_emission.hpp:408; emission_voxels.hpp:170-176)
@@ -243,8 +271,8 @@ int mult_los_download_impl(b200rt_ctx *c, double *const dst[4], long long stride
 int set_multiplet(b200rt_ctx *c, const double *const arr[6]) {
   return is64(c) ? set_multiplet_impl<double>(c, arr) : set_multiplet_impl<float>(c, arr);
 }
-int mult_influence(b200rt_ctx *c, int v_begin, int v_end) {
-  return is64(c) ? mult_influence_impl<double>(c, v_begin, v_end) : mult_influence_impl<float>(c, v_begin, v_end);
+int mult_influence(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges) {
+  return is64(c) ? mult_influence_impl<double>(c, ranges) : mult_influence_impl<float>(c, ranges);
 }
 int mult_solve(b200rt_ctx *c, bool reset_timer) { return mult_solve_impl(c, reset_timer); }
 int mult_brightness(b200rt_ctx *c, int n_subsamples) {

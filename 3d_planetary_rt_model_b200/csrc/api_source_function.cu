@@ -142,15 +142,9 @@ int solve_impl(b200rt_ctx *c, bool reset_timer, int only_e = -1) {
   // systems (a 741-unknown LU is 0.4 ms, shorter than the iteration's set-up), of matrices assembled from peers' row
   // pushes, and the fallback when the iteration does not converge.  B200RT_SOLVER = lu | gmres overrides the size rule.
   if (only_e < 0) {
-    long long min_n = 2048;
-    if (const char *env = getenv("B200RT_KRYLOV_MIN_N")) min_n = atoll(env);
-    bool iterate = n >= min_n;
-    if (const char *env = getenv("B200RT_SOLVER")) iterate = std::strcmp(env, "gmres") == 0 || (iterate && std::strcmp(env, "lu") != 0);
-    long long own = 0;
-    for (auto &r : c->built_ranges) own += r.second - r.first;
-    bool have_all = own == n;
+    bool have_all = true;
     for (int e = 0; e < c->n_em; e++) have_all = have_all && c->em[e].have_K;
-    if (iterate && have_all && n <= B200RT_KRYLOV_MAX_N) {
+    if (have_all && use_gmres(c) && n <= B200RT_KRYLOV_MAX_N) {
       void *block = nullptr;
       if (int rc = exchange_block(c, &block)) return rc;
       const int rc = solve_distributed(c, 0, 1, &block, reset_timer);
@@ -217,6 +211,17 @@ int set_singlet_impl(b200rt_ctx *c, int e, const double *const arr[8]) {
 
 
 }  // namespace
+
+bool use_gmres(const b200rt_ctx *c) {
+  const long long n_vox = c->hg.n_vox;
+  long long min_n = 2048;
+  if (const char *env = getenv("B200RT_KRYLOV_MIN_N")) min_n = atoll(env);
+  bool iterate = n_vox >= min_n;
+  if (const char *env = getenv("B200RT_SOLVER")) iterate = std::strcmp(env, "gmres") == 0 || (iterate && std::strcmp(env, "lu") != 0);
+  long long own = 0;
+  for (auto &r : c->built_ranges) own += r.second - r.first;
+  return iterate && own == n_vox;
+}
 
 int influence(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges) {
   return is64(c) ? influence_impl<double>(c, ranges) : influence_impl<float>(c, ranges);

@@ -215,16 +215,15 @@ int b200rt_influence(b200rt_ctx *c, int v_begin, int v_end) {
   if (!c->have_grid || (c->n_em < 1 && !c->mult.defined)) return fail(c, B200RT_ERR_STATE, "grid / emissions not set");
   if (v_begin < 0 || v_end > c->hg.n_vox || v_begin > v_end) return fail(c, B200RT_ERR_ARG, "bad voxel range");
   cudaSetDevice(c->device);
-  if (c->mult.defined) return api::mult_influence(c, v_begin, v_end);
   const std::vector<std::pair<int, int>> one = {{v_begin, v_end}};
+  if (c->mult.defined) return api::mult_influence(c, one);
   return api::influence(c, one);
 }
 
 int b200rt_influence_ranges(b200rt_ctx *c, int n_ranges, const int *v_begin, const int *v_end) {
   if (!c || n_ranges < 0 || (n_ranges > 0 && (!v_begin || !v_end))) return B200RT_ERR_ARG;
   GROUP_DISPATCH(c, group_influence(c, n_ranges, v_begin, v_end));
-  if (!c->have_grid || c->n_em < 1) return fail(c, B200RT_ERR_STATE, "grid / singlet emissions not set");
-  if (c->mult.defined) return fail(c, B200RT_ERR_STATE, "b200rt_influence_ranges: singlet emissions only");
+  if (!c->have_grid || (c->n_em < 1 && !c->mult.defined)) return fail(c, B200RT_ERR_STATE, "grid / emissions not set");
   std::vector<std::pair<int, int>> r;
   int last_end = 0;
   for (int i = 0; i < n_ranges; i++) {
@@ -234,6 +233,7 @@ int b200rt_influence_ranges(b200rt_ctx *c, int n_ranges, const int *v_begin, con
     r.emplace_back(v_begin[i], v_end[i]);
   }
   cudaSetDevice(c->device);
+  if (c->mult.defined) return api::mult_influence(c, r);
   return api::influence(c, r);
 }
 
@@ -452,7 +452,7 @@ int b200rt_solve_exchange(b200rt_ctx *c, void **block_dev, void *ipc_handle64) {
 int b200rt_solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks) {
   if (!c) return B200RT_ERR_ARG;
   if (c->group) return fail(c, B200RT_ERR_STATE, "b200rt_solve_distributed: a device group does this behind b200rt_solve");
-  if (!c->have_grid || c->n_em < 1) return fail(c, B200RT_ERR_STATE, "grid / emissions not set");
+  if (!c->have_grid || (c->n_em < 1 && !c->mult.defined)) return fail(c, B200RT_ERR_STATE, "grid / emissions not set");
   cudaSetDevice(c->device);
   return api::solve_distributed(c, rank, world, blocks, true);
 }

@@ -172,21 +172,19 @@ int influence_rows(b200rt_ctx *g, int n_ranges, const int *vb, const int *ve) {
     n_rows += ve[i] - vb[i];
   }
   const int n_mem = (int) gr->m.size();
-  // the multiplet emissions have no row sink (b200rt.h: singlet emissions only), and small builds do not pay for the
-  // fan-out: both stay on the primary
-  const bool split = !p->mult.defined && n_rows * p->hg.n_rays >= gr->min_rays && n_rows >= 2 * n_mem;
+  // large grids, every row of the grid in this build: the rows stay on their members and the solve is distributed
+  const long long n_el = (long long) p->hg.n_vox * (p->mult.defined ? p->mult.d.n_upper : 1);
+  const bool distributed = p->hg.n_vox >= gr->kry_min_n && n_el <= B200RT_KRYLOV_MAX_N && n_mem <= B200RT_KRYLOV_MAX_WORLD &&
+                           n_rows == p->hg.n_vox;
+  // the multiplet emissions have no row sink (b200rt.h: singlet emissions only): they fan out only for the distributed
+  // solve; small builds do not pay for the fan-out.  Otherwise the build stays on the primary
+  const bool split = p->mult.defined ? distributed : n_rows * p->hg.n_rays >= gr->min_rays && n_rows >= 2 * n_mem;
   gr->distributed = false;
   gr->rows_gathered = true;
   if (!split) {
     for (int e = 0; e < MAX_EMISSIONS; e++) gr->owner[e] = 0;
     for (int e = 0; e < p->n_em && !p->mult.defined; e++) b200rt_set_row_sink(p, e, nullptr);
-    int rc;
-    if (p->mult.defined) {
-      if (n_ranges != 1) return fail(g, B200RT_ERR_STATE, "b200rt_influence_ranges: singlet emissions only");
-      rc = b200rt_influence(p, vb[0], ve[0]);
-    } else {
-      rc = b200rt_influence_ranges(p, n_ranges, vb, ve);
-    }
+    const int rc = b200rt_influence_ranges(p, n_ranges, vb, ve);
     if (rc != B200RT_OK) { g->err = p->err; return rc; }
     collect_phases(gr, 1);
     gr->last_steps = p->last_steps;
@@ -218,10 +216,8 @@ int influence_rows(b200rt_ctx *g, int n_ranges, const int *vb, const int *ve) {
     }
   }
   // emission e's rows are gathered on member e mod n_mem (one emission: the primary): every other member names that
-  // member's resident K as its sink for e
-  // large grids, every row of the grid in this build: the rows stay on their members and the solve is distributed
-  gr->distributed = p->hg.n_vox >= gr->kry_min_n && p->hg.n_vox <= B200RT_KRYLOV_MAX_N && n_mem <= B200RT_KRYLOV_MAX_WORLD &&
-                    n_rows == p->hg.n_vox;
+  // member's resident K as its sink for e -- unless the solve is distributed
+  gr->distributed = distributed;
   gr->rows_gathered = !gr->distributed;
   gr->shard_b = rb;
   gr->shard_e = re;
@@ -308,13 +304,16 @@ b200rt_ctx *group_owner_K(b200rt_ctx *g, int e) {
   Group *gr = G(g);
   if (gr->distributed && !gr->rows_gathered) {
     b200rt_ctx *p = gr->m[0];
-    const size_t n = (size_t) p->hg.n_vox;
+    const bool mm = p->mult.defined;
+    const size_t nu = mm ? p->mult.d.n_upper : 1, n = (size_t) p->hg.n_vox * nu;   // a voxel's rows: nu rows of n doubles
+    const int n_K = mm ? 1 : p->n_em;
+    auto K_of = [mm](b200rt_ctx *m, int em) { return mm ? m->mult.K.as<double>() : m->em[em].K.as<double>(); };
     for (size_t i = 1; i < gr->m.size(); i++)
-      for (int em = 0; em < p->n_em; em++)
+      for (int em = 0; em < n_K; em++)
         for (size_t k = 0; k < gr->shard_b[i].size(); k++) {
-          const size_t v0 = gr->shard_b[i][k], v1 = gr->shard_e[i][k];
-          cudaMemcpyPeer(p->em[em].K.as<double>() + v0 * n, p->device, gr->m[i]->em[em].K.as<double>() + v0 * n,
-                         gr->m[i]->device, (v1 - v0) * n * sizeof(double));
+          const size_t r0 = gr->shard_b[i][k] * nu, r1 = gr->shard_e[i][k] * nu;
+          cudaMemcpyPeer(K_of(p, em) + r0 * n, p->device, K_of(gr->m[i], em) + r0 * n, gr->m[i]->device,
+                         (r1 - r0) * n * sizeof(double));
         }
     cudaSetDevice(p->device);
     cudaDeviceSynchronize();

@@ -170,7 +170,11 @@ mult_march_kernel(GridView<Real> g, MultView<Real> mv, MultParams<Real> P_, int 
     int len = 0, v0 = 0, ir = 0;
     if (valid) {
       len = lists.len[ray];
-      if (MODE == 0) { v0 = v_begin + (int) (ray / g.n_rays); ir = (int) (ray % g.n_rays); }
+      if (MODE == 0) {
+        v0 = v_begin + (int) (ray / g.n_rays);
+        if (g.vox_map) v0 = g.vox_map[v0];       // interleaved shards: local slot -> source voxel
+        ir = (int) (ray % g.n_rays);
+      }
       else { v0 = (int) ray; if (shadow[v0]) len = -1; }
     }
     // origin factors: c0 (MODE 0) or weight*ls0 (MODE 1)

@@ -38,16 +38,16 @@ constexpr int KRY_SLICE = 96;                        // elements of the vector o
 constexpr int KRY_THREADS = 256;
 constexpr int KRY_WARPS = KRY_THREADS / 32;
 constexpr int KRY_VPT = 8;                            // basis vectors a warp has in flight per trip (L2 latency)
-constexpr int KRY_MAX_N = B200RT_KRYLOV_MAX_N;       // 16384 unknowns: the exchange block has a fixed layout
+constexpr int KRY_MAX_N = B200RT_KRYLOV_MAX_N;       // 24576 unknowns: the exchange block has a fixed layout
 constexpr int KRY_MAX_WORLD = B200RT_KRYLOV_MAX_WORLD;
 constexpr int KRY_MAX_B = (KRY_MAX_N + KRY_SLICE - 1) / KRY_SLICE;
 
-constexpr int KRY_MAX_NR = B200RT_KRYLOV_MAX_NR;     // radial voxels per SZA column the preconditioner handles (128)
+constexpr int KRY_MAX_NR = B200RT_KRYLOV_MAX_NR;     // unknowns of one diagonal block of the preconditioner (128)
 struct KryExchange {                                 // one per rank, written by every rank
   unsigned long long flag[KRY_MAX_WORLD][16];        // flag[q][0]: rounds rank q has completed into THIS block (own 128-byte line)
   double w[2][KRY_MAX_N];
-  double pre[(size_t) KRY_MAX_N * KRY_MAX_NR];       // pre[v][i']: A[v][(i', column of v)], the diagonal blocks of the
-                                                     // preconditioner, every row written by the rank that built it
+  double pre[(size_t) KRY_MAX_N * KRY_MAX_NR];       // pre[e][i']: A[e][unknown i' of the block of e], the diagonal blocks
+                                                     // of the preconditioner, every row written by the rank that built it
 };
 static_assert(sizeof(KryExchange) == B200RT_KRYLOV_BLOCK_BYTES, "include/b200rt.h states the size of the exchange block");
 
@@ -77,13 +77,35 @@ struct KryWork {                     // device pointers into one allocation
   double *R;                         // [KRY_MAX_IT + 1][KRY_MAX_IT], upper triangular after the rotations
   double *cs, *sn, *g, *y;           // [KRY_MAX_IT + 1]
   int ns;
-  // right preconditioner M = the diagonal blocks of A over the SZA columns of the grid (voxel = i_r * n_col + i_col):
-  double *Minv;                      // [n_col][nr][nr] the inverted blocks (every rank inverts all of them, identically)
-  double *Bp;                        // [own rows][n] rows of A M^-1, columns in column-major voxel order c' = i_col * nr + i_r
+  // right preconditioner M = diagonal blocks of A.  Unknown e = voxel * nu + state, voxel = i_r * n_col + i_col; the
+  // COLUMN ORDER p = i_col * cl + i_r * nu + state (cl = n_r * nu) lists every SZA column's unknowns radially outwards, and
+  // each column is cut into n_runs runs of `run` unknowns (whole voxels; the last run is shorter where run does not divide cl): block
+  // b = i_col * n_runs + k covers positions [i_col * cl + k * run, + min(run, cl - k * run)).  One state and n_r <= 128:
+  // one block per SZA column.
+  double *Minv;                      // [n_col * n_runs][run * run] the inverted blocks (every rank inverts all of them, identically)
+  double *Bp;                        // [own rows][n] rows of A M^-1, columns in the column order
   double *usol;                      // [ns] V y before M^-1 is applied
   double *wperm;                     // [ns] the current vector in the column order of Bp (what the product reads)
-  int nr, n_col;                     // 0: no preconditioner
+  int run, n_col, nu, cl, n_runs;    // run = 0: no preconditioner
 };
+
+__device__ __forceinline__ int pc_perm(const KryWork &wk, int e) {    // unknown -> position in the column order
+  const int v = e / wk.nu, s = e - v * wk.nu, ir = v / wk.n_col, ic = v - ir * wk.n_col;
+  return ic * wk.cl + ir * wk.nu + s;
+}
+__device__ __forceinline__ int pc_elem(const KryWork &wk, int p) {    // position in the column order -> unknown
+  const int ic = p / wk.cl, q = p - ic * wk.cl, ir = q / wk.nu, s = q - ir * wk.nu;
+  return (ir * wk.n_col + ic) * wk.nu + s;
+}
+__device__ __forceinline__ int pc_block_of(const KryWork &wk, int p) {
+  const int ic = p / wk.cl;
+  return ic * wk.n_runs + (p - ic * wk.cl) / wk.run;
+}
+__device__ __forceinline__ void pc_block(const KryWork &wk, int b, int *p0, int *len) {   // first position, unknowns
+  const int ic = b / wk.n_runs, k = b - ic * wk.n_runs;
+  *p0 = ic * wk.cl + k * wk.run;
+  *len = min(wk.run, wk.cl - k * wk.run);
+}
 
 __device__ __forceinline__ unsigned long long ld_flag(const unsigned long long *p) {
   unsigned long long v;
@@ -545,12 +567,15 @@ kry_pre_post(const double *__restrict__ K, int n, const int *__restrict__ rows, 
              KryPeers pe) {
   __shared__ int sh;
   KryState *st = wk.st;
-  const int tid = threadIdx.x, nr = wk.nr, n_col = wk.n_col;
+  const int tid = threadIdx.x;
   const unsigned long long round = st->round;
   for (int r = blockIdx.x; r < n_rows; r += gridDim.x) {
-    const int v = rows[r], iv = v / n_col, jv = v - iv * n_col;
-    if (tid < nr) {
-      const double val = (tid == iv ? 1.0 : 0.0) - branching * K[(size_t) v * n + (size_t) tid * n_col + jv];
+    const int v = rows[r];
+    int p0, len;
+    pc_block(wk, pc_block_of(wk, pc_perm(wk, v)), &p0, &len);
+    if (tid < len) {
+      const int e = pc_elem(wk, p0 + tid);
+      const double val = (e == v ? 1.0 : 0.0) - branching * K[(size_t) v * n + e];
       for (int q = 0; q < pe.world; q++) st_remote(&pe.p[q]->pre[(size_t) v * KRY_MAX_NR + tid], val);
     }
   }
@@ -564,12 +589,15 @@ kry_pre_invert(KryWork wk, KryPeers pe) {
   __shared__ int sh_flag;
   __shared__ double sh_inv;
   KryState *st = wk.st;
-  const int tid = threadIdx.x, nr = wk.nr, n_col = wk.n_col, ld = nr + 1, j = blockIdx.x;
+  const int tid = threadIdx.x, j = blockIdx.x;
+  int p0, nr;
+  pc_block(wk, j, &p0, &nr);
+  const int ld = nr + 1;
   if (!wait_round(st, pe, st->round, &sh_flag)) return;
   const KryExchange *mine = pe.p[pe.rank];
   for (int e = tid; e < nr * nr; e += KRY_THREADS) {
     const int i = e / nr, c = e - i * nr;
-    Mb[i * ld + c] = ld_remote(&mine->pre[(size_t) (i * n_col + j) * KRY_MAX_NR + c]);
+    Mb[i * ld + c] = ld_remote(&mine->pre[(size_t) pc_elem(wk, p0 + i) * KRY_MAX_NR + c]);
   }
   __syncthreads();
   const int tx = tid & 31, ty = tid >> 5;           // thread: columns tx, tx + 32, ...; rows ty, ty + 8, ...
@@ -599,27 +627,24 @@ kry_pre_invert(KryWork wk, KryPeers pe) {
       if (i != p) Mb[i * ld + p] = -Mb[i * ld + p] * inv;
     __syncthreads();
   }
-  double *out = wk.Minv + (size_t) j * nr * nr;
+  double *out = wk.Minv + (size_t) j * wk.run * wk.run;
   for (int e = tid; e < nr * nr; e += KRY_THREADS) out[e] = Mb[(e / nr) * ld + (e % nr)];
 }
 
-// own rows of A with the columns regrouped by SZA column: Bp[r][j * nr + i] = A[row r][i * n_col + j]  (a row is read
+// own rows of A with the columns in the column order: Bp[r][p] = A[row r][pc_elem(p)]  (a row is read
 // once, coalesced, and written once, coalesced; gathering the strided entries inside kry_pre_rows fetched every 64-byte
 // line of K eight times: 1.45 ms for the rows of one GPU)
 __global__ void __launch_bounds__(KRY_THREADS)
 kry_pre_permute(const double *__restrict__ K, int n, const int *__restrict__ rows, int n_rows, double branching, KryWork wk) {
   extern __shared__ double rowbuf[];               // [n]
-  const int tid = threadIdx.x, nr = wk.nr, n_col = wk.n_col;
+  const int tid = threadIdx.x;
   for (int r = blockIdx.x; r < n_rows; r += gridDim.x) {
     const int v = rows[r];
     const double *Kr = K + (size_t) v * n;
     for (int c = tid; c < n; c += KRY_THREADS) rowbuf[c] = (c == v ? 1.0 : 0.0) - branching * __ldcs(Kr + c);
     __syncthreads();
     double *out = wk.Bp + (size_t) r * n;
-    for (int c = tid; c < n; c += KRY_THREADS) {
-      const int j = c / nr, i = c - j * nr;
-      out[c] = rowbuf[i * n_col + j];
-    }
+    for (int c = tid; c < n; c += KRY_THREADS) out[c] = rowbuf[pc_elem(wk, c)];
     __syncthreads();
   }
 }
@@ -629,9 +654,11 @@ constexpr int KRY_PRE_RT = 32;                       // rows of a tile of kry_pr
 __global__ void __launch_bounds__(KRY_THREADS)
 kry_pre_rows(int n, int n_rows, KryWork wk) {
   extern __shared__ double sm[];                   // Minv_j [nr][nr] | At [RT][nr]
-  const int tid = threadIdx.x, nr = wk.nr, j = blockIdx.x;
+  const int tid = threadIdx.x, j = blockIdx.x;
+  int p0, nr;
+  pc_block(wk, j, &p0, &nr);
   double *Mj = sm, *At = sm + nr * nr;
-  const double *src = wk.Minv + (size_t) j * nr * nr;
+  const double *src = wk.Minv + (size_t) j * wk.run * wk.run;
   for (int e = tid; e < nr * nr; e += KRY_THREADS) Mj[e] = src[e];
   const int cg = tid & 31, rg = tid >> 5;
   // 4 x 4 register tiles: thread (rg, cg) = rows 4 rg .. 4 rg + 3 of the tile, outputs cg, cg + 32, cg + 64, cg + 96 (8 loads
@@ -642,7 +669,7 @@ kry_pre_rows(int n, int n_rows, KryWork wk) {
     const int rt = min(KRY_PRE_RT, n_rows - r0);
     __syncthreads();                               // (Minv_j in place; the previous tile's At no longer read)
     for (int r = tid >> 5; r < rt; r += KRY_WARPS) {
-      const double *in = wk.Bp + (size_t) (r0 + r) * n + (size_t) j * nr;
+      const double *in = wk.Bp + (size_t) (r0 + r) * n + p0;
       for (int i = tid & 31; i < nr; i += 32) At[r * nr + i] = in[i];
     }
     __syncthreads();
@@ -667,7 +694,7 @@ kry_pre_rows(int n, int n_rows, KryWork wk) {
     for (int u = 0; u < 4; u++) {
       const int r = 4 * rg + u;
       if (r >= rt) continue;
-      double *out = wk.Bp + (size_t) (r0 + r) * n + (size_t) j * nr;
+      double *out = wk.Bp + (size_t) (r0 + r) * n + p0;
 #pragma unroll
       for (int w = 0; w < 4; w++)
         if (cg + 32 * w < nr) out[cg + 32 * w] = acc[u][w];
@@ -694,6 +721,7 @@ struct KryLoopArgs {
   KryPeers pe;
   double branching, tol;
   int n, n_rows, max_it, orth_blocks;
+  bool stage_x;                      // x fits in shared memory beside a grid of at least orth_blocks CTAs
 };
 
 __device__ __forceinline__ unsigned int ld_vol_u32(const unsigned int *p) { return *reinterpret_cast<const volatile unsigned int *>(p); }
@@ -975,10 +1003,10 @@ kry_loop(KryLoopArgs a) {
   unsigned long long round = st->round;          // every CTA counts the rounds itself (st->round is for the host)
   unsigned int bar = 0, seq = 0;
   const KryExchange *mine = pe.p[pe.rank];
-  const bool stage = a.n_rows > 3 * (int) gridDim.x;   // rows per CTA and round
-  const bool pc = wk.nr > 0;                           // right-preconditioned: the iteration is on u, S = M^-1 u
+  const bool stage = a.stage_x && a.n_rows > 3 * (int) gridDim.x;   // rows per CTA and round
+  const bool pc = wk.run > 0;                          // right-preconditioned: the iteration is on u, S = M^-1 u
   int pos_perm = 0;                                    // where this thread's element of the slice sits in the column order of Bp
-  if (pc && tid < len) { const int v = lo + tid, iv = v / wk.n_col; pos_perm = (v - iv * wk.n_col) * wk.nr + iv; }
+  if (pc && tid < len) pos_perm = pc_perm(wk, lo + tid);
   const bool clock = cta == 0 && tid == 0;
   unsigned long long t_mark = 0, t_sub = 0, t_acc[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 
@@ -1166,15 +1194,16 @@ kry_loop(KryLoopArgs a) {
   ++seq;
   if (cta == 0) step_publish(st, seq);
   if (!step_wait(st, seq, bar * n_orth, &sh_flag)) return;
-  if (pc) {                                        // S = M^-1 u, block by block: element (i, j) = row i of Minv_j . u[(., j)]
-    ++bar;
+  if (pc) {                                        // S = M^-1 u, block by block: unknown at position p0 + i of block b =
+    ++bar;                                         // row i of Minv_b . u[unknowns of block b]
     if (orth) {
-      const int nr = wk.nr, n_col = wk.n_col;
       for (int e = warp; e < len; e += KRY_WARPS) {
-        const int v = lo + e, iv = v / n_col, jv = v - iv * n_col;
-        const double *mrow = wk.Minv + ((size_t) jv * nr + iv) * nr;
+        const int v = lo + e, p = pc_perm(wk, v), b = pc_block_of(wk, p);
+        int p0, nr;
+        pc_block(wk, b, &p0, &nr);
+        const double *mrow = wk.Minv + (size_t) b * wk.run * wk.run + (size_t) (p - p0) * nr;
         double sum = 0;
-        for (int i = lane; i < nr; i += 32) sum = fma(mrow[i], __ldcg(wk.usol + (size_t) i * n_col + jv), sum);
+        for (int i = lane; i < nr; i += 32) sum = fma(mrow[i], __ldcg(wk.usol + pc_elem(wk, p0 + i)), sum);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
         if (lane == 0) { wk.xsol[v] = sum; a.S[v] = sum; }
@@ -1232,11 +1261,36 @@ int exchange_block(b200rt_ctx *c, void **dev_ptr) {
 }
 
 int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, bool reset_timer, int cta_cap) {
-  const int n = c->hg.n_vox;
+  // the systems: every singlet emission's (I - w K) S = S0 over the voxels, or the multiplet's (I - K) S = S0 over the
+  // n_el = n_vox * n_upper elements (its branching is folded into K: multiplet_CFR_emission::pre_solve is empty)
+  const bool mm = c->mult.defined;
+  const int nu = mm ? c->mult.d.n_upper : 1;
+  const int n = c->hg.n_vox * nu;
   if (world < 1 || world > KRY_MAX_WORLD || rank < 0 || rank >= world || !blocks)
     return fail(c, B200RT_ERR_ARG, "b200rt_solve_distributed: bad rank / world / blocks");
-  if (n > KRY_MAX_N) return fail(c, B200RT_ERR_CAPACITY, "b200rt_solve_distributed: more than 16384 unknowns");
-  if (c->mult.defined) return fail(c, B200RT_ERR_STATE, "b200rt_solve_distributed: singlet emissions only");
+  if (n > KRY_MAX_N)
+    return fail(c, B200RT_ERR_CAPACITY, "b200rt_solve_distributed: more than " + std::to_string(KRY_MAX_N) + " unknowns");
+  struct System {
+    bool have_K;
+    const double *K, *S0;
+    double *S;
+    void *S_real;
+    double branching;
+    double *residual;
+    bool *have_S, *rec_dirty;
+  };
+  std::vector<System> sys;
+  if (mm) {
+    Multiplet &M = c->mult;
+    sys.push_back({M.have_K, M.K.as<double>(), M.S0.as<double>(), M.S.as<double>(), M.S_real.p, 1.0, &M.residual, &M.have_S,
+                   &M.rec_dirty});
+  } else {
+    for (int e = 0; e < c->n_em; e++) {
+      Emission &E = c->em[e];
+      sys.push_back({E.have_K, E.K.as<double>(), E.S0.as<double>(), E.S.as<double>(), E.S_real.p, E.branching, &E.residual,
+                     &E.have_S, &E.rec_dirty});
+    }
+  }
   if (int rc = exchange_block(c, nullptr)) return rc;
   if (blocks[rank] != c->kry_xchg.p)
     return fail(c, B200RT_ERR_ARG, "b200rt_solve_distributed: blocks[rank] is not this context's exchange block");
@@ -1244,10 +1298,11 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
   std::unique_lock<std::mutex> turn;
   if (world == 1) turn = std::unique_lock<std::mutex>(g_single_rank_solve[c->device & 63]);
 
-  // the rows this rank multiplies: what its last influence call built
+  // the rows this rank multiplies: what its last influence call built (every element of each voxel)
   std::vector<int> rows;
   for (auto &r : c->built_ranges)
-    for (int v = r.first; v < r.second; v++) rows.push_back(v);
+    for (int v = r.first; v < r.second; v++)
+      for (int s = 0; s < nu; s++) rows.push_back(v * nu + s);
   const int n_rows = (int) rows.size();
 
   // work area
@@ -1264,13 +1319,22 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
   const size_t o_cs = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)), o_sn = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)),
                o_g = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)), o_y = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double));
   const size_t o_rows = carve_bytes(off, (size_t) std::max(n, 1) * sizeof(int));
-  // right preconditioner over the SZA columns (spherical grids; B200RT_KRYLOV_PC=0 switches it off)
-  int pc_nr = c->hg.n_rb - 1, pc_nc = c->hg.n_sb - 1;
-  bool pc = !c->hg.pp && pc_nr >= 2 && pc_nr <= KRY_MAX_NR && pc_nc >= 2 && pc_nr * pc_nc == n;
+  // right preconditioner over the SZA columns (spherical grids; B200RT_KRYLOV_PC=0 switches it off): every column is cut,
+  // from the lowest voxel up, into runs of KRY_MAX_NR / nu radial voxels with all their states (KryWork); runs as equal
+  // as whole voxels allow took as many or more steps (tests/krylov_multiplet_model.py, pc_blocks)
+  const int pc_nr = c->hg.n_rb - 1, pc_nc = c->hg.n_sb - 1;
+  bool pc = !c->hg.pp && pc_nr >= 2 && pc_nc >= 2 && pc_nr * pc_nc == c->hg.n_vox && nu <= KRY_MAX_NR;
   if (const char *env = getenv("B200RT_KRYLOV_PC")) pc = pc && atoi(env) != 0;
   if (const char *env = getenv("B200RT_KRYLOV_FUSED")) pc = pc && atoi(env) != 0;     // the per-step launches iterate on A itself
+  int pc_runs = 1, pc_run = 0;
+  if (pc) {
+    const int run_vox = std::min(pc_nr, KRY_MAX_NR / nu);
+    pc_run = nu * run_vox;
+    pc_runs = (pc_nr + run_vox - 1) / run_vox;
+  }
+  const int pc_blocks = pc_nc * pc_runs;
   const size_t o_usol = carve_bytes(off, (size_t) ns * sizeof(double)), o_wperm = carve_bytes(off, (size_t) ns * sizeof(double));
-  const size_t o_minv = carve_bytes(off, pc ? (size_t) pc_nc * pc_nr * pc_nr * sizeof(double) : 16);
+  const size_t o_minv = carve_bytes(off, pc ? (size_t) pc_blocks * pc_run * pc_run * sizeof(double) : 16);
   const bool fresh = c->kry_work.bytes < off;
   B200RT_CUDA(c, c->kry_work.ensure(off));
   char *base = static_cast<char *>(c->kry_work.p);
@@ -1296,7 +1360,7 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
   wk.wperm = reinterpret_cast<double *>(base + o_wperm);
   wk.Minv = reinterpret_cast<double *>(base + o_minv);
   wk.Bp = nullptr;
-  wk.nr = 0; wk.n_col = 0;
+  wk.run = 0; wk.n_col = pc_nc; wk.nu = nu; wk.cl = pc_nr * nu; wk.n_runs = pc_runs;
   if (pc) {
     B200RT_CUDA(c, c->kry_bp.ensure((size_t) std::max(n_rows, 1) * n * sizeof(double)));
     wk.Bp = c->kry_bp.as<double>();
@@ -1322,12 +1386,11 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
   cudaStream_t s = c->stream;
   constexpr int CHUNK = 16;
 
-  for (int e = 0; e < c->n_em; e++) {
-    Emission &E = c->em[e];
+  for (System &E : sys) {
     if (!E.have_K) return fail(c, B200RT_ERR_STATE, "b200rt_solve_distributed: influence rows not built");
     PhaseTimer t(c, PH_SOLVE);
     int launches = 0;
-    const double *K = E.K.as<double>(), *S0 = E.S0.as<double>();
+    const double *K = E.K, *S0 = E.S0;
     // everything but the round counter starts from zero (no kernel of this context is in flight here)
     B200RT_CUDA(c, cudaMemsetAsync(reinterpret_cast<char *>(wk.st) + offsetof(KryState, iter), 0,
                                    sizeof(KryState) - offsetof(KryState, iter), s));
@@ -1339,46 +1402,54 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
     bool fused = true;
     if (const char *env = getenv("B200RT_KRYLOV_FUSED")) fused = atoi(env) != 0;
     if (fused && pc) {                             // the preconditioner: block entries to all ranks, inverses, rows of A M^-1
-      wk.nr = pc_nr; wk.n_col = pc_nc;
-      const size_t sm_inv = (size_t) pc_nr * (pc_nr + 1) * sizeof(double);
-      const size_t sm_rows = ((size_t) pc_nr * pc_nr + (size_t) KRY_PRE_RT * pc_nr) * sizeof(double);
+      wk.run = pc_run;
+      const size_t sm_inv = (size_t) pc_run * (pc_run + 1) * sizeof(double);
+      const size_t sm_rows = ((size_t) pc_run * pc_run + (size_t) KRY_PRE_RT * pc_run) * sizeof(double);
       B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_invert, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_inv));
       B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_rows));
       B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_permute, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) ((size_t) n * sizeof(double))));
       if (trace) mark();
       kry_pre_post<<<std::max(1, std::min(n_rows, 4 * NUM_SMS)), 128, 0, s>>>(K, n, d_rows, n_rows, E.branching, wk, pe);
       if (trace) mark();
-      kry_pre_invert<<<pc_nc, KRY_THREADS, sm_inv, s>>>(wk, pe);
+      kry_pre_invert<<<pc_blocks, KRY_THREADS, sm_inv, s>>>(wk, pe);
       if (trace) mark();
       if (n_rows > 0) {
         kry_pre_permute<<<std::min(n_rows, 4 * NUM_SMS), KRY_THREADS, (size_t) n * sizeof(double), s>>>(K, n, d_rows, n_rows, E.branching, wk);
-        kry_pre_rows<<<dim3(pc_nc, std::max(1, std::min((n_rows + KRY_PRE_RT - 1) / KRY_PRE_RT, 2 * NUM_SMS / pc_nc))), KRY_THREADS, sm_rows, s>>>(n, n_rows, wk);
+        kry_pre_rows<<<dim3(pc_blocks, std::max(1, std::min((n_rows + KRY_PRE_RT - 1) / KRY_PRE_RT, 2 * NUM_SMS / pc_blocks))), KRY_THREADS, sm_rows, s>>>(n, n_rows, wk);
       }
       if (trace) mark();
       launches += 4;
     }
     if (fused) {
-      const size_t smem = (size_t) n * sizeof(double);
-      int per_sm = 0;
-      cudaError_t e_occ = cudaFuncSetAttribute(kry_loop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-      if (e_occ == cudaSuccess) e_occ = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kry_loop, KRY_THREADS, smem);
+      // x staged in shared memory (n * 8 bytes per CTA) where that leaves room for a grid of orth_blocks CTAs; otherwise
+      // (above ~14k unknowns on a B200) the rows read x through L2 and the CTAs need no dynamic shared memory
       int cap = cta_cap > 0 ? cta_cap : 3 * NUM_SMS;
       if (const char *env = getenv("B200RT_KRYLOV_CTAS")) cap = std::max(1, atoi(env));
-      const int grid = std::min(cap, per_sm * NUM_SMS);
-      if (e_occ != cudaSuccess || grid < orth_blocks) {
-        cudaGetLastError();
-        fused = false;                             // (a vector too long for the shared-memory staging: the launches below)
+      int grid = 0;
+      size_t smem = 0;
+      for (const size_t try_smem : {(size_t) n * sizeof(double), (size_t) 0}) {
+        int per_sm = 0;
+        cudaError_t e_occ = cudaFuncSetAttribute(kry_loop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) try_smem);
+        if (e_occ == cudaSuccess) e_occ = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kry_loop, KRY_THREADS, try_smem);
+        if (e_occ != cudaSuccess) { cudaGetLastError(); continue; }
+        grid = std::min(cap, per_sm * NUM_SMS);
+        smem = try_smem;
+        if (grid >= orth_blocks) break;
+      }
+      if (grid < orth_blocks) {
+        fused = false;                             // (a grid too small to own every slice of the vector: the launches below)
       } else {
         KryLoopArgs a;
-        a.K = K; a.rows = d_rows; a.S0 = S0; a.S = E.S.as<double>(); a.wk = wk; a.pe = pe;
+        a.K = K; a.rows = d_rows; a.S0 = S0; a.S = E.S; a.wk = wk; a.pe = pe;
         a.branching = E.branching; a.tol = tol; a.n = n; a.n_rows = n_rows; a.max_it = max_it; a.orth_blocks = orth_blocks;
+        a.stage_x = smem > 0;
         void *kargs[] = {&a};
         const cudaError_t e_l = cudaLaunchCooperativeKernel((void *) kry_loop, dim3(grid), dim3(KRY_THREADS), kargs, smem, s);
         if (e_l == cudaSuccess) launches += 1;
         else { cudaGetLastError(); fused = false; }
       }
     }
-    if (!fused) wk.nr = wk.n_col = 0;               // (the launches below iterate on A itself)
+    if (!fused) wk.run = 0;                         // (the launches below iterate on A itself)
     if (!fused) {
     kry_post<0><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, E.branching, S0, wk, pe);
     kry_begin<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe, tol, max_it);
@@ -1414,16 +1485,16 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
     }
     (void) issued;
     kry_backsolve<<<1, 32, 0, s>>>(wk);
-    kry_solution<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, E.S.as<double>());
+    kry_solution<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, E.S);
     kry_post<2><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, E.branching, S0, wk, pe);
     kry_residual<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
     launches += 4;
     }   // !fused
     B200RT_CUDA(c, cudaGetLastError());
     if (c->precision == B200RT_F64)
-      B200RT_CUDA(c, launch_convert<double>(E.S.as<double>(), E.S_real.as<double>(), n, s));
+      B200RT_CUDA(c, launch_convert<double>(E.S, static_cast<double *>(E.S_real), n, s));
     else
-      B200RT_CUDA(c, launch_convert<float>(E.S.as<double>(), E.S_real.as<float>(), n, s));
+      B200RT_CUDA(c, launch_convert<float>(E.S, static_cast<float *>(E.S_real), n, s));
     t.stop(launches);
     B200RT_CUDA(c, cudaMemcpyAsync(h_st + 63, wk.st, sizeof(KryState), cudaMemcpyDeviceToHost, s));
     B200RT_CUDA(c, cudaStreamSynchronize(s));
@@ -1470,9 +1541,9 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
                                                   std::to_string(fin.iter) + " steps (rows missing on some rank, or a matrix the LU path should take)");
     if (!(fin.true_res <= 1e-8))
       return fail(c, B200RT_ERR_NOT_DOMINANT, "b200rt_solve_distributed: residual " + std::to_string(fin.true_res));
-    E.residual = fin.true_res;
-    E.have_S = true;
-    E.rec_dirty = true;
+    *E.residual = fin.true_res;
+    *E.have_S = true;
+    *E.rec_dirty = true;
   }
   PhaseTimer::collect(c);
   return B200RT_OK;

@@ -52,11 +52,14 @@ int b200rt_device_count(void);
  * each call out itself and every other entry point of this header takes it unchanged:
  *   geometry, emission tables, source function: replicated on every device;
  *   b200rt_generate_S / b200rt_influence*:      source-voxel rows split into interleaved shards.  Grids of
- *                                               B200RT_KRYLOV_MIN_N (2048) voxels and more: the rows STAY on the devices
- *                                               that built them.  Smaller grids: the devices write their finished row
- *                                               batches into the resident K of the device that solves that emission
- *                                               (emission e: device e mod n; one emission: the first device) over peer
- *                                               memory (copy engines, NVLink) while marching the next batch;
+ *                                               B200RT_KRYLOV_MIN_N (2048) voxels and more, every row in the call and
+ *                                               at most B200RT_KRYLOV_MAX_N unknowns: the rows STAY on the devices that
+ *                                               built them (singlet and multiplet emissions).  Smaller singlet grids: the
+ *                                               devices write their finished row batches into the resident K of the
+ *                                               device that solves that emission (emission e: device e mod n; one
+ *                                               emission: the first device) over peer memory (copy engines, NVLink)
+ *                                               while marching the next batch.  Smaller multiplet grids (no row sink
+ *                                               for them): the first device builds every row;
  *   b200rt_solve:                               large grids: all devices together, each multiplying its own rows
  *                                               ("distributed solve" below), S resident everywhere afterwards; small
  *                                               grids: each emission's LU on its device, side by side, S handed over;
@@ -167,15 +170,17 @@ int b200rt_set_multiplet(b200rt_ctx *ctx, const b200rt_multiplet_desc *desc,
  * separately so that rows can be sharded over GPUs (rows [v_begin, v_end) only). */
 int b200rt_generate_S(b200rt_ctx *ctx);
 int b200rt_influence(b200rt_ctx *ctx, int v_begin, int v_end);
-/* the same for several ascending, disjoint source-voxel ranges in one call (singlet emissions): the interleaved shards
- * that balance the cost of low-altitude (long rays through many voxels) and high-altitude rows across GPUs */
+/* the same for several ascending, disjoint source-voxel ranges in one call: the interleaved shards that balance the cost
+ * of low-altitude (long rays through many voxels) and high-altitude rows across GPUs.  A multiplet context builds all
+ * n_upper element rows of every voxel in the ranges. */
 int b200rt_influence_ranges(b200rt_ctx *ctx, int n_ranges, const int *v_begin, const int *v_end);
 /* RT_grid::solve_gpu, emission_voxels::solve_gpu: (I - w K) S = S0 per emission.  Two solvers behind it, both FP64 whatever
  * the context's Real: a block LU without row exchanges (FP64 tensor-core DMMA; the matrix is checked to be diagonally
  * dominant or an M-matrix first, B200RT_ERR_NOT_DOMINANT otherwise) and a right-preconditioned GMRES (see "distributed
  * solve" below; with one rank it is simply the faster solve of a large system: 4.0 ms against 5.8 ms at 5841 unknowns).
- * Systems of B200RT_KRYLOV_MIN_N (2048) unknowns and more whose rows were all built by this context take the GMRES and fall
- * back to the LU if it does not converge; everything else takes the LU.  B200RT_SOLVER = lu | gmres overrides the size rule.
+ * Grids of B200RT_KRYLOV_MIN_N (2048) voxels and more whose rows were all built by this context and whose system has at
+ * most B200RT_KRYLOV_MAX_N unknowns (n_vox, or n_el = n_vox * n_upper for a multiplet) take the GMRES and fall back to the
+ * LU if it does not converge; everything else takes the LU.  B200RT_SOLVER = lu | gmres overrides the size rule.
  * Either way b200rt_last_residual reports the true relative residual afterwards. */
 int b200rt_solve(b200rt_ctx *ctx);
 /* ray-voxel steps executed by the last b200rt_influence call (one step = one
@@ -211,7 +216,8 @@ int b200rt_sourcefn_dev(b200rt_ctx *ctx, int i_emission, void **S_dev);
  * (b200rt_ipc_open -> a device pointer valid in their process) and name it as their row sink; from then on
  * b200rt_influence(v_begin, v_end) marches its range in >= 4 batches and DMAs each finished batch into the sink with
  * the copy engines over NVLink WHILE the next batch is marched (no SMs, no collective kernel), and returns when the
- * rows have landed.  A host barrier across ranks then releases the solve.  Singlet emissions only.
+ * rows have landed.  A host barrier across ranks then releases the solve.  Singlet emissions only: a multiplet context
+ * refuses b200rt_ipc_export_influence and b200rt_set_row_sink (its rows stay where they were built: distributed solve).
  * (This is the form for a solve by factorisation on one GPU; the distributed solve below needs no row exchange at all.) */
 int b200rt_ipc_export_influence(b200rt_ctx *ctx, int i_emission, void *handle64);
 int b200rt_ipc_open(b200rt_ctx *ctx, const void *handle64, void **peer_ptr);
@@ -221,13 +227,15 @@ int b200rt_set_row_sink(b200rt_ctx *ctx, int i_emission, void *peer_K_dev);   /*
 /* ---- distributed solve: the rows stay where they were built ---------------------------
  * The N-GPU form of RT_grid::solve_gpu.  Instead of gathering K on one GPU and factorising it there, every rank keeps
  * the rows its b200rt_influence / b200rt_influence_ranges call built (no row sink) and all ranks solve
- * (I - w K) S = S0 together by GMRES: one step is one product with K, each rank multiplies its own rows and writes its
+ * (I - w K) S = S0 together by GMRES -- for a multiplet context (I - K) S = S0 over the n_el element rows, every rank
+ * multiplying the n_upper rows of each voxel it built: one step is one product with K, each rank multiplies its own rows and writes its
  * piece of the result into every rank's EXCHANGE BLOCK over peer memory (NVLink), then every rank orthogonalises the
  * assembled vector redundantly -- bit-identical on all ranks -- so S ends up resident on every rank with no row gather,
  * no broadcast and no host barrier.  K is the kernel of a second-kind integral equation: the step count does not grow
  * with the grid (csrc/solve_krylov.cu).  Right preconditioner on spherical grids: the inverted diagonal blocks of I - wK
- * over the SZA columns (all radial voxels of one SZA index), whose entries every rank contributes for its rows in one more
- * exchange round and which every rank inverts redundantly; 38 steps instead of 71 on the 100x60 grid at 1e-13.
+ * over runs of B200RT_KRYLOV_MAX_NR / n_upper radial voxels of one SZA column with all their states (one state and at
+ * most 128 radial voxels: the whole column), whose entries every rank contributes for its rows in one more exchange round
+ * and which every rank inverts redundantly; 38 steps instead of 71 on the 100x60 grid at 1e-13.
  *   b200rt_solve_exchange:    this context's exchange block (B200RT_KRYLOV_BLOCK_BYTES of device memory, allocated on
  *                             first use, alive until destroy): its device pointer (ranks of one process, peer access
  *                             enabled) and/or a CUDA IPC handle of it (64 bytes; other processes open it with
@@ -240,12 +248,14 @@ int b200rt_set_row_sink(b200rt_ctx *ctx, int i_emission, void *peer_K_dev);   /*
  *                             (B200RT_PHASE_SOLVE) counts the launches.  The union of the ranks' rows must be every
  *                             voxel; a rank that never arrives is reported (B200RT_ERR_CUDA) after 20 s, no convergence
  *                             within 160 steps as B200RT_ERR_NOT_DOMINANT.  world = 1 is allowed (one GPU, GMRES
- *                             instead of the LU).  Singlet emissions, n_vox <= B200RT_KRYLOV_MAX_N.
+ *                             instead of the LU).  Singlet emissions: n_vox <= B200RT_KRYLOV_MAX_N; a multiplet:
+ *                             n_el <= B200RT_KRYLOV_MAX_N (B200RT_ERR_CAPACITY beyond).
  * A device group (b200rt_create_multi) does this behind b200rt_solve / b200rt_generate_S for grids of
  * B200RT_KRYLOV_MIN_N (default 2048) voxels and more; smaller systems keep the LU on the owning device.
+ * B200RT_KRYLOV_MAX_N = 24576 covers the H Lyman multiplet on the 100x60 grid (5841 voxels x 4 states = 23364).
  * Knobs: B200RT_KRYLOV_TOL (relative residual of the Krylov recurrence, default 1e-13), B200RT_KRYLOV_MAXIT,
  * B200RT_KRYLOV_PC=0 (no preconditioner). */
-#define B200RT_KRYLOV_MAX_N 16384
+#define B200RT_KRYLOV_MAX_N 24576
 #define B200RT_KRYLOV_MAX_WORLD 16
 #define B200RT_KRYLOV_MAX_NR 128
 #define B200RT_KRYLOV_BLOCK_BYTES (B200RT_KRYLOV_MAX_WORLD * 128 + 2 * B200RT_KRYLOV_MAX_N * 8 + (unsigned long long) B200RT_KRYLOV_MAX_N * B200RT_KRYLOV_MAX_NR * 8)
