@@ -35,6 +35,7 @@ SIGNATURES = {
     "b200rt_make_grid_sph": (C.c_int, [C.c_int] * 5 + [_dp, C.c_int, C.c_int] + [_dp] * 6),
     "b200rt_set_grid_pp": (C.c_int, [_vp, C.c_int, C.c_int] + [_dp] * 4),
     "b200rt_make_grid_pp": (C.c_int, [C.c_int] * 3 + [_dp] * 4),
+    "b200rt_fold_rays": (C.c_int, [C.c_int, C.c_int] + [_dp] * 3 + [_ip, C.POINTER(C.c_int)]),
     "b200rt_set_singlet": (C.c_int, [_vp, C.c_int, C.c_int] + [C.c_double] * 4 + [_dp] * 8),
     "b200rt_set_g_factor": (C.c_int, [_vp, C.c_int, C.c_double]),
     "b200rt_influence_ranges": (C.c_int, [_vp, C.c_int, np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS"),
@@ -115,6 +116,19 @@ def load():
 
 class B200RTError(RuntimeError):
     pass
+
+
+def fold_rays(precision, ray_theta, ray_phi, ray_domega):
+    """b200rt_fold_rays (host only): (rep, n_marched) -- rep[k] is the ray whose march stands for ray k in an influence
+    build (k itself for a marched ray; the lower index of a mirror pair)"""
+    lib = load()
+    t, p, d = (np.ascontiguousarray(a, dtype=np.float64) for a in (ray_theta, ray_phi, ray_domega))
+    rep = np.zeros(len(t), dtype=np.int32)
+    n = C.c_int(0)
+    rc = lib.b200rt_fold_rays(precision, len(t), t, p, d, rep, C.byref(n))
+    if rc != 0:
+        raise B200RTError(f"b200rt_fold_rays: status {rc}")
+    return rep, n.value
 
 
 def _ptr(a):

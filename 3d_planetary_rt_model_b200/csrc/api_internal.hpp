@@ -19,8 +19,9 @@ namespace b200rt {
 namespace api {
 
 
-// Boundary-list scratch per batch: 8 GiB of the 180 GB, so that the bench workload (2.24e6 voxel rays, 1e6 lines of
-// sight on the 100x60 grid: 7.0 and 3.1 GB of lists) runs as ONE batch per phase.  Every batch boundary drains the
+// Boundary-list scratch per batch: 8 GiB of the 180 GB, so that the bench workload (1e6 lines of sight and 2.24e6 voxel
+// rays on the 100x60 grid, 1.12e6 of them marched once mirror pairs are folded: 3.1 and 3.5 GB of lists) runs as ONE
+// batch per phase.  Every batch boundary drains the
 // persistent brightness kernel (a single line of sight takes ~0.5 ms): measured 1.45 ms per boundary (r01n launch
 // list: 686k LOS in 29.63 ms, 314k in 14.35 ms).  B200RT_SCRATCH_BYTES overrides it (tests force several batches).
 constexpr size_t SCRATCH_BUDGET_BYTES = size_t(1) << 33;
@@ -75,6 +76,9 @@ inline int dbg_sync(b200rt_ctx *c, const char *what) {
 
 template <class Real>
 GridView<Real> &gv(b200rt_ctx *c) { return *static_cast<GridView<Real> *>(c->grid_view); }
+// the influence builds march this one: mirror pairs of voxel-origin rays folded (grid_host.cpp, fold_pairs)
+template <class Real>
+GridView<Real> &march_gv(b200rt_ctx *c) { return *static_cast<GridView<Real> *>(c->march_view); }
 
 template <class Real>
 EmissionView<Real> em_view(b200rt_ctx *c, int e) {

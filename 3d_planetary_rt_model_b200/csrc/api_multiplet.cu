@@ -66,6 +66,7 @@ int set_multiplet_impl(b200rt_ctx *c, const double *const arr[6]) {
 template <class Real>
 int mult_influence_impl(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges) {
   GridView<Real> &g = gv<Real>(c);
+  const GridView<Real> &gm = march_gv<Real>(c);   // voxel-origin rays: mirror pairs folded
   Multiplet &M = c->mult;
   const b200rt_multiplet_desc &d = M.d;
   const int n_vox = g.n_vox;
@@ -91,15 +92,15 @@ int mult_influence_impl(b200rt_ctx *c, const std::vector<std::pair<int, int>> &r
   }
   const int first_voxel = ranges.empty() ? 0 : ranges[0].first;
   const long long cap_rays = batch_capacity(c, sizeof(Real));
-  const int vox_per_batch = (int) std::max<long long>(1, std::min<long long>(cap_rays / g.n_rays, n_rows));
+  const int vox_per_batch = (int) std::max<long long>(1, std::min<long long>(cap_rays / gm.n_rays, n_rows));
   ListView<Real> lv;
-  const long long need = std::max<long long>((long long) vox_per_batch * g.n_rays, n_vox);
+  const long long need = std::max<long long>((long long) vox_per_batch * gm.n_rays, n_vox);
   if (int rc = ensure_lists<Real>(c, need, &lv)) return rc;
   int *overflow = c->work_counter.as<int>() + 1;
   MultView<Real> mv = mult_view<Real>(c);
   for (int lb = 0; lb < n_rows; lb += vox_per_batch) {
     const int le = std::min(n_rows, lb + vox_per_batch);
-    GridView<Real> gb = g;
+    GridView<Real> gb = gm;
     int vb = first_voxel + lb, ve = first_voxel + le;      // unmapped: the voxel range itself
     if (mapped) { gb.vox_map = c->vox_map.as<int>() + lb; vb = 0; ve = le - lb; }
     {

@@ -12,6 +12,7 @@ namespace {
 template <class Real>
 int influence_impl(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges) {
   GridView<Real> &g = gv<Real>(c);
+  const GridView<Real> &gm = march_gv<Real>(c);   // voxel-origin rays: mirror pairs folded
   const int n_vox = g.n_vox;
   PhaseTimer::reset(c);
   SideStreamDrain drain(c);        // row pushes into a peer's K never outlive the call
@@ -40,7 +41,7 @@ int influence_impl(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges
   }
   const int first_voxel = ranges.empty() ? 0 : ranges[0].first;
   const long long cap_rays = batch_capacity(c, sizeof(Real));
-  int vox_per_batch = (int) std::max<long long>(1, std::min<long long>(cap_rays / g.n_rays, std::max(n_rows, 1)));
+  int vox_per_batch = (int) std::max<long long>(1, std::min<long long>(cap_rays / gm.n_rays, std::max(n_rows, 1)));
   bool pushing = false;
   for (int e = 0; e < c->n_em; e++) {
     if (c->row_sink[e] && c->row_sink_n_vox[e] != n_vox)
@@ -54,13 +55,13 @@ int influence_impl(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges
     if (!c->ev_rows) B200RT_CUDA(c, cudaEventCreateWithFlags(&c->ev_rows, cudaEventDisableTiming));
   }
   ListView<Real> lv;
-  const long long need = std::max<long long>((long long) vox_per_batch * g.n_rays, n_vox);
+  const long long need = std::max<long long>((long long) vox_per_batch * gm.n_rays, n_vox);
   if (int rc = ensure_lists<Real>(c, need, &lv)) return rc;
   int *overflow = c->work_counter.as<int>() + 1;
 
   for (int lb = 0; lb < n_rows; lb += vox_per_batch) {
     const int le = std::min(n_rows, lb + vox_per_batch);
-    GridView<Real> gb = g;
+    GridView<Real> gb = gm;
     int vb = first_voxel + lb, ve = first_voxel + le;      // unmapped: the voxel range itself
     if (mapped) { gb.vox_map = c->vox_map.as<int>() + lb; vb = 0; ve = le - lb; }
     {

@@ -63,6 +63,7 @@ int b200rt_destroy(b200rt_ctx *c) {
     for (DevBuf *b : mb) b->release();
   }
   if (c->grid_view) ::operator delete(c->grid_view);
+  if (c->march_view) ::operator delete(c->march_view);
   for (cudaEvent_t ev : c->lu_events) cudaEventDestroy(ev);
   for (cudaEvent_t ev : c->timer_events) cudaEventDestroy(ev);
   if (c->lu_graph) cudaGraphExecDestroy(c->lu_graph);
@@ -91,6 +92,14 @@ int b200rt_make_grid_sph(int precision, int n_rb, int n_sb, int n_theta, int n_p
   if (n_rb < 2 || n_sb < 3 || n_theta < 2 || n_phi < 1 || !rb) return B200RT_ERR_ARG;
   if (precision == B200RT_F64) make_grid_sph<double>(n_rb, n_sb, n_theta, n_phi, rb, szamethod, raymethod, sb, pts_r, pts_s, ray_t, ray_p, ray_domega);
   else make_grid_sph<float>(n_rb, n_sb, n_theta, n_phi, rb, szamethod, raymethod, sb, pts_r, pts_s, ray_t, ray_p, ray_domega);
+  return B200RT_OK;
+}
+
+int b200rt_fold_rays(int precision, int n_rays, const double *ray_t, const double *ray_p, const double *ray_domega,
+                     int *rep, int *n_marched) {
+  if (n_rays < 1 || !ray_t || !ray_p || !ray_domega || !rep || !n_marched) return B200RT_ERR_ARG;
+  *n_marched = precision == B200RT_F64 ? fold_rays<double>(n_rays, ray_t, ray_p, ray_domega, rep)
+                                       : fold_rays<float>(n_rays, ray_t, ray_p, ray_domega, rep);
   return B200RT_OK;
 }
 

@@ -75,6 +75,8 @@ struct GridView {
   const Real *ray_sint;    // [n_rays]
   const double *ray_cp;    // [n_rays] cos(ray.p) (double call in ptray)
   const Real *ray_domega;  // [n_rays]
+  const int *ray_mult;     // [n_rays] rays of the full set this one stands for (march view: 2 for a folded mirror pair,
+                           // and ray_domega is already multiplied by it); nullptr: 1 (full view)
   // voxel-origin rays: the sphere crossings of a ray depend on (radial shell of its voxel, cos of its polar angle) only,
   // so their ordered, trimmed list is built once per (shell, polar-angle class) and shared by every voxel of the shell
   // and every azimuth (traverse.cu, sphere_table_kernel).  nullptr: every ray builds its own.
@@ -203,7 +205,9 @@ struct b200rt_ctx {
   bool have_grid = false;
   b200rt::HostGrid hg;
   b200rt::DevBuf grid_tables;       // one slab holding every GridView array
-  void *grid_view = nullptr;        // heap GridView<Real> (host struct of device pointers)
+  void *grid_view = nullptr;        // heap GridView<Real> (host struct of device pointers): every ray
+  void *march_view = nullptr;       // heap GridView<Real>: the same grid with mirror pairs of rays folded (influence builds)
+  int n_rays_marched = 0;           // rays of the march view (a device group sizes its fan-out by them)
   b200rt::DevBuf sph_table;         // ordered sphere-crossing lists per (radial shell, polar-angle class), traverse.cu
   b200rt::DevBuf sun_rays;          // RayList arrays for the n_vox sun-ward rays + shadow flags
   std::vector<int> shadow;          // host copy of the shadow test per voxel
@@ -292,6 +296,10 @@ void make_grid_sph(int n_rb, int n_sb, int n_theta, int n_phi, const double *rb,
                    double *ray_p, double *ray_domega);
 template <class Real>
 void make_grid_pp(int n_rb, int n_theta, const double *rb, double *pts_r, double *ray_t, double *ray_domega);
+// mirror-pair fold of a ray set in Real (b200rt_fold_rays): rep[k] = the ray whose march stands for ray k; returns the
+// number of rays marched
+template <class Real>
+int fold_rays(int n_rays, const double *ray_t, const double *ray_p, const double *ray_domega, int *rep);
 template <class Real>
 void los_from_MSO(int n, const double *loc, const double *dir, double *x, double *y, double *z,
                   double *r, double *t, double *lx, double *ly, double *lz, double *cost);

@@ -178,7 +178,8 @@ int influence_rows(b200rt_ctx *g, int n_ranges, const int *vb, const int *ve) {
                            n_rows == p->hg.n_vox;
   // the multiplet emissions have no row sink (b200rt.h: singlet emissions only): they fan out only for the distributed
   // solve; small builds do not pay for the fan-out.  Otherwise the build stays on the primary
-  const bool split = p->mult.defined ? distributed : n_rows * p->hg.n_rays >= gr->min_rays && n_rows >= 2 * n_mem;
+  // (the work counted is the rays the build marches: mirror pairs folded, grid_host.cpp fold_pairs)
+  const bool split = p->mult.defined ? distributed : (long long) n_rows * p->n_rays_marched >= gr->min_rays && n_rows >= 2 * n_mem;
   gr->distributed = false;
   gr->rows_gathered = true;
   if (!split) {

@@ -28,7 +28,70 @@ size_t carve(size_t &off, size_t n) {
   off += n * sizeof(T);
   return at;
 }
+
+// the per-ray tables the traversal and the march read (atmo_ray::tp, atmo_vector::ptray), in Real
+template <class Real>
+struct RayTables {
+  std::vector<Real> cost, sint, dom;
+  std::vector<double> cp;
+  std::vector<char> lower;   // sin(ray.p) < 0: the ray is the mirror image of one with sin(ray.p) > 0
+  RayTables(int n, const double *ray_t, const double *ray_p, const double *ray_domega)
+      : cost(n), sint(n), dom(n), cp(n), lower(n) {
+    for (int k = 0; k < n; k++) {
+      const Real t = (Real) ray_t[k], p = (Real) ray_p[k];
+      cost[k] = std::cos(t);
+      sint[k] = std::sin(t);
+      cp[k] = ::cos((double) p);
+      dom[k] = (Real) ray_domega[k];
+      lower[k] = ::sin((double) p) < 0;
+    }
+  }
+};
+
+template <class T>
+bool same_bits(const T &a, const T &b) { return std::memcmp(&a, &b, sizeof(T)) == 0; }
+
+// cos(phi) of a mirror pair: phi and 2 pi - phi are each rounded once (ulp(2 pi) = 8.9e-16) before libm takes the
+// cosine, so the two values differ by up to ~1e-15 (measured: 6 x 2^-53 at n_phi = 32, 8 x 2^-53 at n_phi = 12)
+constexpr double MIRROR_COS_TOL = 0x1p-49;   // 1.8e-15
+// Mirror pairs of voxel-origin rays.  Every voxel point lies in the phi = 0 half-plane of an azimuthally symmetric grid,
+// so the rays at phi and 2 pi - phi of one voxel cross the same voxels over the same lengths: the traversal reads a ray
+// only through cos(theta), sin(theta) and cos(phi) (traverse.cu ray_scalars), and the march adds domega * G.  A pair is
+// marched once with multiplicity 2.  Rays pair when
+//   - all four tables are bit-equal (both precisions: the two lists are then identical by construction), or
+//   - in double only, cos(theta), sin(theta) and domega are bit-equal, cos(phi) agrees to MIRROR_COS_TOL and sin(phi)
+//     has the opposite sign.  The lists of such a pair agree to ~1e-13 relative in distance, and K moves by at most
+//     ~4e-8 relative per contribution on the 100x60 grid.  In float, line_z rounds differently often enough that the
+//     lists of a near pair drift apart (segment lengths up to 100 % on that grid), so float folds bit-equal pairs only.
+// The lower index represents the pair; every other ray, and every ray of a set without mirror symmetry, stays single.
+template <class Real>
+int fold_pairs(const RayTables<Real> &rt, int *rep) {
+  const int n = (int) rt.cost.size();
+  for (int k = 0; k < n; k++) rep[k] = k;
+  int marched = 0;
+  for (int k = 0; k < n; k++) {
+    if (rep[k] != k) continue;
+    marched++;
+    for (int q = k + 1; q < n; q++) {
+      if (rep[q] != q || !same_bits(rt.cost[k], rt.cost[q]) || !same_bits(rt.sint[k], rt.sint[q]) ||
+          !same_bits(rt.dom[k], rt.dom[q]))
+        continue;
+      const bool exact = same_bits(rt.cp[k], rt.cp[q]);
+      const bool mirror = sizeof(Real) == sizeof(double) && rt.lower[k] != rt.lower[q] &&
+                          std::fabs(rt.cp[k] - rt.cp[q]) <= MIRROR_COS_TOL;
+      if (exact || mirror) { rep[q] = k; break; }
+    }
+  }
+  return marched;
+}
 } // namespace
+
+template <class Real>
+int fold_rays(int n_rays, const double *ray_t, const double *ray_p, const double *ray_domega, int *rep) {
+  return fold_pairs<Real>(RayTables<Real>(n_rays, ray_t, ray_p, ray_domega), rep);
+}
+template int fold_rays<double>(int, const double *, const double *, const double *, int *);
+template int fold_rays<float>(int, const double *, const double *, const double *, int *);
 
 // Derived tables + upload.  Mirrors (reference src/):
 //   sphere::set_radius      grid/intersections.cpp:53-56   R = rb/1e9, R2 = R*R
@@ -44,8 +107,8 @@ int upload_grid(b200rt_ctx *c) {
   const int n_rb = h.n_rb, n_sb = h.n_sb, n_vox = h.n_vox, n_rays = h.n_rays;
 
   std::vector<Real> rb(n_rb), R2(n_rb), sb(n_sb), ccos(std::max(n_sb - 2, 1)), ccos2(std::max(n_sb - 2, 1)),
-      pr(n_rb - 1), lpr(n_rb - 1), ps(n_sb - 1), vz(n_vox), vzn(n_vox), rcost(n_rays), rsint(n_rays), rdom(n_rays);
-  std::vector<double> ct(n_sb - 1), st(n_sb - 1), rcp(n_rays);
+      pr(n_rb - 1), lpr(n_rb - 1), ps(n_sb - 1), vz(n_vox), vzn(n_vox);
+  std::vector<double> ct(n_sb - 1), st(n_sb - 1);
   // sun-ward rays
   std::vector<Real> sr(n_vox), sz(n_vox), stt(n_vox), scost(n_vox), slz(n_vox);
   std::vector<int> sidx(n_vox);
@@ -91,13 +154,9 @@ int upload_grid(b200rt_ctx *c) {
       scost[v] = costx + costy + costz;
       slz[v] = lz;
     }
-  for (int k = 0; k < n_rays; k++) {
-    const Real t = (Real) h.ray_t[k], p = (Real) h.ray_p[k];
-    rcost[k] = std::cos(t);
-    rsint[k] = std::sin(t);
-    rcp[k] = ::cos((double) p);
-    rdom[k] = (Real) h.ray_domega[k];
-  }
+  const RayTables<Real> rt(n_rays, h.ray_t.data(), h.ray_p.data(), h.ray_domega.data());
+  const std::vector<Real> &rcost = rt.cost, &rsint = rt.sint, &rdom = rt.dom;
+  const std::vector<double> &rcp = rt.cp;
 
   // polar-angle classes of the rays: rays with bitwise equal cos(theta) cross every sphere at the same distances
   std::vector<int> rcls(n_rays), cls_ray;
@@ -113,6 +172,24 @@ int upload_grid(b200rt_ctx *c) {
   const bool use_table = !h.pp && n_rb <= 128 && 2 * n_cls <= n_rays;
   const size_t n_pairs = (size_t) (n_rb - 1) * n_cls;
 
+  // march view: the representative rays of the mirror-pair fold (fold_pairs) in ascending order, domega * multiplicity
+  // (doubling is exact).  The first ray of a polar-angle class is always a representative, so every class keeps one.
+  std::vector<int> rep(n_rays);
+  const int n_fold = fold_pairs<Real>(rt, rep.data());
+  std::vector<Real> fcost, fsint, fdom;
+  std::vector<double> fcp;
+  std::vector<int> fcls, fmult, fpos(n_rays, -1), fcls_ray(n_cls);
+  for (int k = 0; k < n_rays; k++)
+    if (rep[k] == k) {
+      fpos[k] = (int) fcost.size();
+      fcost.push_back(rcost[k]); fsint.push_back(rsint[k]); fcp.push_back(rcp[k]); fcls.push_back(rcls[k]);
+      fdom.push_back(rdom[k]); fmult.push_back(1);
+    } else {
+      fdom[fpos[rep[k]]] += rdom[k];   // bit-equal to the representative's: exactly 2 domega
+      fmult[fpos[rep[k]]] += 1;
+    }
+  for (int q = 0; q < n_cls; q++) fcls_ray[q] = fpos[cls_ray[q]];
+
   // one slab
   size_t off = 0;
   const size_t o_rb = carve<Real>(off, n_rb), o_R2 = carve<Real>(off, n_rb), o_sb = carve<Real>(off, n_sb),
@@ -121,7 +198,10 @@ int upload_grid(b200rt_ctx *c) {
                o_ct = carve<double>(off, n_sb), o_st = carve<double>(off, n_sb),
                o_rc = carve<Real>(off, n_rays), o_rs = carve<Real>(off, n_rays),
                o_rcp = carve<double>(off, n_rays), o_rd = carve<Real>(off, n_rays),
-               o_cls = carve<int>(off, n_rays), o_clr = carve<int>(off, n_cls), o_vzn = carve<Real>(off, n_vox);
+               o_cls = carve<int>(off, n_rays), o_clr = carve<int>(off, n_cls), o_vzn = carve<Real>(off, n_vox),
+               o_fc = carve<Real>(off, n_fold), o_fs = carve<Real>(off, n_fold), o_fcp = carve<double>(off, n_fold),
+               o_fd = carve<Real>(off, n_fold), o_fcls = carve<int>(off, n_fold), o_fclr = carve<int>(off, n_cls),
+               o_fm = carve<int>(off, n_fold);
   std::vector<char> slab(off + 16, 0);
   auto put = [&](size_t at, const void *src, size_t bytes) { std::memcpy(slab.data() + at, src, bytes); };
   put(o_rb, rb.data(), n_rb * sizeof(Real));       put(o_R2, R2.data(), n_rb * sizeof(Real));
@@ -134,6 +214,10 @@ int upload_grid(b200rt_ctx *c) {
   put(o_rcp, rcp.data(), n_rays * sizeof(double)); put(o_rd, rdom.data(), n_rays * sizeof(Real));
   put(o_vzn, vzn.data(), n_vox * sizeof(Real));
   put(o_cls, rcls.data(), n_rays * sizeof(int));   put(o_clr, cls_ray.data(), n_cls * sizeof(int));
+  put(o_fc, fcost.data(), n_fold * sizeof(Real));  put(o_fs, fsint.data(), n_fold * sizeof(Real));
+  put(o_fcp, fcp.data(), n_fold * sizeof(double)); put(o_fd, fdom.data(), n_fold * sizeof(Real));
+  put(o_fcls, fcls.data(), n_fold * sizeof(int));  put(o_fclr, fcls_ray.data(), n_cls * sizeof(int));
+  put(o_fm, fmult.data(), n_fold * sizeof(int));
 
   // the slab and, below, the sun-ward ray block each travel as one asynchronous copy out of page-locked staging (see
   // set_singlet_impl: copies out of pageable memory are staged by the runtime under a process-wide lock)
@@ -145,6 +229,7 @@ int upload_grid(b200rt_ctx *c) {
   B200RT_CUDA(c, cudaMemcpyAsync(c->grid_tables.p, c->host_stage.p, slab.size(), cudaMemcpyHostToDevice, c->stream));
 
   if (c->grid_view) { ::operator delete(c->grid_view); c->grid_view = nullptr; }
+  if (c->march_view) { ::operator delete(c->march_view); c->march_view = nullptr; }
   GridView<Real> *g = new GridView<Real>;
   char *base = static_cast<char *>(c->grid_tables.p);
   g->n_rb = n_rb; g->n_sb = n_sb; g->n_vox = n_vox; g->n_rays = n_rays; g->cap = h.cap; g->pp = h.pp ? 1 : 0;
@@ -156,7 +241,7 @@ int upload_grid(b200rt_ctx *c) {
   g->vox_z = (const Real *) (base + o_vz);       g->col_ct = (const double *) (base + o_ct);
   g->col_st = (const double *) (base + o_st);    g->ray_cost = (const Real *) (base + o_rc);
   g->ray_sint = (const Real *) (base + o_rs);    g->ray_cp = (const double *) (base + o_rcp);
-  g->ray_domega = (const Real *) (base + o_rd);
+  g->ray_domega = (const Real *) (base + o_rd);  g->ray_mult = nullptr;
   g->n_cls = n_cls;
   g->vox_zn = (const Real *) (base + o_vzn);
   g->ray_cls = (const int *) (base + o_cls);     g->cls_ray = (const int *) (base + o_clr);
@@ -172,6 +257,14 @@ int upload_grid(b200rt_ctx *c) {
     B200RT_CUDA(c, launch_sphere_table<Real>(*g, c->stream));   // (same stream as the slab copy; the sync below covers it)
   }
   c->grid_view = g;
+  GridView<Real> *f = new GridView<Real>(*g);   // shares everything but the rays (the sphere table included)
+  f->n_rays = n_fold;
+  f->ray_cost = (const Real *) (base + o_fc);    f->ray_sint = (const Real *) (base + o_fs);
+  f->ray_cp = (const double *) (base + o_fcp);   f->ray_domega = (const Real *) (base + o_fd);
+  f->ray_cls = (const int *) (base + o_fcls);    f->cls_ray = (const int *) (base + o_fclr);
+  f->ray_mult = (const int *) (base + o_fm);
+  c->march_view = f;
+  c->n_rays_marched = n_fold;
 
   // sun-ward ray descriptors + shadow flags: [r | z | t | cost | lz](Real) [i_voxel | shadow](int)
   B200RT_CUDA(c, c->sun_rays.ensure(sun_bytes));

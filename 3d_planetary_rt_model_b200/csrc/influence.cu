@@ -130,13 +130,14 @@ march_kernel(GridView<Real> g, EmissionView<Real> em, int v_begin, long long n_r
 
     const long long ray = task * RAYS_PER_WARP + grp;
     const bool valid = ray < n_rays_total;
-    int len = 0, v0 = 0, ir = 0;
+    int len = 0, v0 = 0, ir = 0, mult = 1;
     if (valid) {
       len = lists.len[ray];
       if (MODE == 0) {
         v0 = v_begin + (int) (ray / g.n_rays);
         if (g.vox_map) v0 = g.vox_map[v0];
         ir = (int) (ray % g.n_rays);
+        if (g.ray_mult) mult = g.ray_mult[ir];
       }
       else { v0 = (int) ray; if (shadow[v0]) len = -1; }
     }
@@ -147,7 +148,7 @@ march_kernel(GridView<Real> g, EmissionView<Real> em, int v_begin, long long n_r
     Real P[LAMBDA_PER_LANE];
 #pragma unroll
     for (int m = 0; m < LAMBDA_PER_LANE; m++) P[m] = renorm * rexp<Real>(-l2[m] * Tr0);
-    const Real domega = (MODE == 0 && valid) ? g.ray_domega[ir] : Real(1);
+    const Real domega = (MODE == 0 && valid) ? g.ray_domega[ir] : Real(1);   // march view: x the ray's multiplicity
     Real tau_sp = 0, tau_abs = 0;
 
     int maxlen = len;
@@ -219,7 +220,7 @@ march_kernel(GridView<Real> g, EmissionView<Real> em, int v_begin, long long n_r
       for (int m = 0; m < LAMBDA_PER_LANE; m++) rec[m] = rec_next[m];
     }
     if (MODE == 0) {
-      if (sub == 0 && len > 1) my_steps += (unsigned long long) (len - 1);
+      if (sub == 0 && len > 1) my_steps += (unsigned long long) (len - 1) * mult;   // the reference's count
     } else {
       // holstein_T_final = sum_i w_i * norm(T0) * phi0_i * P_i   (singlet_CFR.hpp:183-186)
       Real T = 0;

@@ -167,13 +167,14 @@ mult_march_kernel(GridView<Real> g, MultView<Real> mv, MultParams<Real> P_, int 
 
     const long long ray = task * RPW + grp;
     const bool valid = ray < n_rays_total;
-    int len = 0, v0 = 0, ir = 0;
+    int len = 0, v0 = 0, ir = 0, mult = 1;
     if (valid) {
       len = lists.len[ray];
       if (MODE == 0) {
         v0 = v_begin + (int) (ray / g.n_rays);
         if (g.vox_map) v0 = g.vox_map[v0];       // interleaved shards: local slot -> source voxel
         ir = (int) (ray % g.n_rays);
+        if (g.ray_mult) mult = g.ray_mult[ir];
       }
       else { v0 = (int) ray; if (shadow[v0]) len = -1; }
     }
@@ -191,7 +192,7 @@ mult_march_kernel(GridView<Real> g, MultView<Real> mv, MultParams<Real> P_, int 
     for (int m = 0; m < NM; m++)
 #pragma unroll
       for (int j = 0; j < NLP; j++) P[m][j] = Real(1);
-    const Real domega = (MODE == 0 && valid) ? g.ray_domega[ir] : Real(1);
+    const Real domega = (MODE == 0 && valid) ? g.ray_domega[ir] : Real(1);   // march view: x the ray's multiplicity
     Real tsp[NL], tab[NL];
 #pragma unroll
     for (int l = 0; l < NL; l++) { tsp[l] = 0; tab[l] = 0; }
@@ -253,7 +254,7 @@ mult_march_kernel(GridView<Real> g, MultView<Real> mv, MultParams<Real> P_, int 
       }
     }
     if (MODE == 0) {
-      if (sub == 0 && len > 1) my_steps += (unsigned long long) (len - 1);
+      if (sub == 0 && len > 1) my_steps += (unsigned long long) (len - 1) * mult;   // the reference's count
     } else {
       // holstein_T_final[line] = sum_i weight ls0 P_final   (multiplet_CFR_emission.hpp:222-228)
 #pragma unroll

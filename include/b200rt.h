@@ -67,7 +67,8 @@ int b200rt_device_count(void);
  *   b200rt_brightness*, b200rt_iph_*:           lines of sight split by index, results at their offsets in the
  *                                               caller's arrays; counters add up, b200rt_last_kernel_ms is the
  *                                               slowest device's time.
- * Work too small to pay for the fan-out stays on the first device (B200RT_GROUP_MIN_RAYS voxel rays, default 262144;
+ * Work too small to pay for the fan-out stays on the first device (B200RT_GROUP_MIN_RAYS voxel rays marched -- a mirror
+ * pair of rays folded by b200rt_fold_rays counts once --, default 262144;
  * B200RT_GROUP_MIN_LOS lines of sight, default 65536).  n_dev <= 0: every visible device; dev_ids NULL: 0..n_dev-1;
  * one device: a plain context, exactly b200rt_create; an id may repeat (several members on one device, as the sweep's
  * contexts per GPU).  b200rt_group_size: devices behind a handle (1 for a plain one). */
@@ -108,6 +109,15 @@ int b200rt_set_grid_pp(b200rt_ctx *ctx, int n_rb, int n_rays, const double *radi
                        const double *pts_radii, const double *ray_theta, const double *ray_domega);
 int b200rt_make_grid_pp(int precision, int n_rb, int n_theta, const double *radial_boundaries,
                         double *pts_radii, double *ray_theta, double *ray_domega);
+
+/* host helper, no device needed: the mirror-pair fold b200rt_set_grid_sph / _pp apply to the influence build.  On an
+ * azimuthally symmetric grid the voxel-origin rays at phi and 2 pi - phi cross the same voxels over the same lengths, so
+ * b200rt_influence* marches such a pair once and adds its contribution with twice the ray's domega.  Rays pair when
+ * their uploaded cos/sin(theta), cos(phi) and domega are bit-equal, or (F64 only) when cos/sin(theta) and domega are
+ * bit-equal, cos(phi) agrees to 1.8e-15 and sin(phi) has the opposite sign.  rep[n_rays]: the ray whose march stands for
+ * ray k (k itself for a marched ray; a pair is represented by its lower index); n_marched: rays marched per voxel. */
+int b200rt_fold_rays(int precision, int n_rays, const double *ray_theta, const double *ray_phi,
+                     const double *ray_domega, int *rep, int *n_marched);
 
 /* ---- emissions ------------------------------------------------------------------
  * replaces singlet_CFR::copy_to_device_influence / copy_to_device_brightness
@@ -183,8 +193,9 @@ int b200rt_influence_ranges(b200rt_ctx *ctx, int n_ranges, const int *v_begin, c
  * LU if it does not converge; everything else takes the LU.  B200RT_SOLVER = lu | gmres overrides the size rule.
  * Either way b200rt_last_residual reports the true relative residual afterwards. */
 int b200rt_solve(b200rt_ctx *ctx);
-/* ray-voxel steps executed by the last b200rt_influence call (one step = one
- * RT_grid::influence_update, RT_grid.hpp:90-105, covering all emissions) */
+/* ray-voxel steps of the last b200rt_influence call as the reference counts them (one step = one
+ * RT_grid::influence_update, RT_grid.hpp:90-105, covering all emissions).  A folded mirror pair (b200rt_fold_rays) is
+ * marched once and counted for both of its rays. */
 int b200rt_last_step_count(b200rt_ctx *ctx, long long *n_steps);
 /* line-of-sight sub-steps integrated by the last singlet b200rt_brightness* call: sum over lines of sight of
  * (segments inside the grid) x (n_subsamples - 1), one sub-step = one update_tracker_brightness_interp of every
