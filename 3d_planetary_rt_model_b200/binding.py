@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(HERE, "libb200rt.so")
 F64, F32 = 0, 1
 ROW_MAJOR, COL_MAJOR = 0, 1
 PH_TRAVERSE, PH_INFLUENCE, PH_SOLVE, PH_BRIGHTNESS, PH_IPH, PH_ORDER = 0, 1, 2, 3, 4, 5
+PH_LW_STRUCTURE, PH_LW_VALUES, PH_LW_APPLY = 6, 7, 8
 
 _dp = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")
 _ip = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
@@ -65,6 +66,9 @@ SIGNATURES = {
     "b200rt_los_upload": (C.c_int, [_vp, C.c_int] + [_dp] * 9),
     "b200rt_brightness_resident": (C.c_int, [_vp, C.c_int]),
     "b200rt_los_download": (C.c_int, [_vp] + [_vp] * 4),
+    "b200rt_los_weights": (C.c_int, [_vp, C.c_int, C.POINTER(C.c_longlong)]),
+    "b200rt_los_weights_download": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "b200rt_los_weights_apply": (C.c_int, [_vp, C.c_int, C.c_int, _dp, _dp]),
     "b200rt_iph_load_table": (C.c_int, [_vp, C.c_char_p]),
     "b200rt_iph_set_table": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_float] + [_fp] * 7),
     "b200rt_iph_background": (C.c_int, [_vp] + [C.c_float] * 4 + [C.c_int, _fp, _fp, _fp, _fp, _vp]),
@@ -157,6 +161,7 @@ class Context:
         self.n_vox = 0
         self.n_em = 0
         self.n_los = 0
+        self.lw_nnz = 0
 
     def close(self):
         if getattr(self, "h", None):
@@ -370,6 +375,31 @@ class Context:
         self._ck(self.lib.b200rt_los_download(self.h, *[_ptr(o) for o in out]))
         return dict(brightness=out[0], tau_species_final=out[1], tau_absorber_final=out[2], species_col_dens=out[3])
 
+    # ---- line-of-sight weighting functions: brightness_e = W_e S_e on the resident lines of sight
+    def los_weights(self, n_subsamples=10):
+        """b200rt_los_weights: builds W for every emission; returns nnz"""
+        nnz = C.c_longlong(0)
+        self._ck(self.lib.b200rt_los_weights(self.h, n_subsamples, C.byref(nnz)))
+        self.lw_nnz = nnz.value
+        return nnz.value
+
+    def los_weights_download(self):
+        """-> (indptr int64 [n_los + 1], indices int32 [nnz], data float64 [n_em][nnz]):
+        scipy.sparse.csr_matrix((data[e], indices, indptr), shape=(n_los, n_vox)) is W_e"""
+        nnz = self.lw_nnz
+        indptr = np.zeros(self.n_los + 1, np.int64)
+        indices = np.zeros(max(nnz, 1), np.int32)
+        data = np.zeros((self.n_em, max(nnz, 1)))
+        self._ck(self.lib.b200rt_los_weights_download(self.h, _ptr(indptr), _ptr(indices), _ptr(data)))
+        return indptr, indices[:nnz], data[:, :nnz]
+
+    def los_weights_apply(self, e, x, transpose=False):
+        """W_e x (x of length n_vox), or W_e^T x (x of length n_los) with transpose=True"""
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        y = np.zeros(self.n_vox if transpose else self.n_los)
+        self._ck(self.lib.b200rt_los_weights_apply(self.h, e, int(bool(transpose)), x, y))
+        return y
+
     # ---- interplanetary hydrogen background
     def iph_load_table(self, fname):
         self._ck(self.lib.b200rt_iph_load_table(self.h, os.fsencode(fname)))
@@ -513,6 +543,12 @@ class GpuModel:
         r = self.ctx.brightness(los, n_subsamples)
         out = np.stack([r["brightness"], r["tau_species_final"], r["tau_absorber_final"], r["species_col_dens"]], axis=1)
         return self.ctx.kernel_ms(PH_BRIGHTNESS)[0] * 1e-3, out
+
+    def los_weights(self, locs, dirs, n_subsamples=10):
+        """line-of-sight weighting functions of these lines of sight: (indptr, indices, data[n_em]) of W_e"""
+        self.ctx.los_upload(self.ctx.los_from_MSO(locs, dirs))
+        self.ctx.los_weights(n_subsamples)
+        return self.ctx.los_weights_download()
 
 
 def define_multiplet_tables(scn, precision=F64):

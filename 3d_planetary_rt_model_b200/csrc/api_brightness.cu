@@ -29,6 +29,7 @@ int brightness_impl(b200rt_ctx *c, int n_subsamples, const HostLos *io = nullptr
     B200RT_CUDA(c, c->los_in.ensure((size_t) 9 * io->n * sizeof(Real)));
     c->n_los = io->n;
     c->los_done = false;
+    c->lw.valid = false;
     if (!c->copy_stream) B200RT_CUDA(c, cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     if (!c->out_stream) B200RT_CUDA(c, cudaStreamCreateWithFlags(&c->out_stream, cudaStreamNonBlocking));
   }
@@ -189,6 +190,7 @@ int los_upload_impl(b200rt_ctx *c, int n, const double *const src[9]) {
   stage.release();
   c->n_los = n;
   c->los_done = false;
+  c->lw.valid = false;
   return rc;
 }
 

@@ -5,6 +5,7 @@
 //   api_brightness.cu        line-of-sight upload / brightness (resident and pipelined host-buffer forms) / download
 //   api_traverse.cu          the traversal parity surface (boundary lists back to the host)
 //   api_multiplet.cu         the same four steps for the multiplet CFR emissions
+//   api_weights.cu           line-of-sight weighting functions: build, download, products
 #pragma once
 #include <algorithm>
 #include <cmath>
@@ -190,6 +191,12 @@ int mult_influence(b200rt_ctx *c, const std::vector<std::pair<int, int>> &ranges
 int mult_solve(b200rt_ctx *c, bool reset_timer);
 int mult_brightness(b200rt_ctx *c, int n_subsamples);
 int mult_los_download(b200rt_ctx *c, double *const dst[4], long long stride, long long offset);
+// ---- api_weights.cu
+int los_weights(b200rt_ctx *c, int n_subsamples, long long *nnz);
+int los_weights_nnz(b200rt_ctx *c, long long *nnz);   // B200RT_ERR_STATE unless built for the current inputs
+// row_ptr[0..n_los] (+ ptr_offset), col[nnz], val[e * val_stride + p]; any may be null
+int los_weights_download(b200rt_ctx *c, long long *row_ptr, long long ptr_offset, int *col, double *val, long long val_stride);
+int los_weights_apply(b200rt_ctx *c, int e, int transpose, const double *x, double *y);
 
 }  // namespace api
 }  // namespace b200rt

@@ -44,7 +44,8 @@ int b200rt_destroy(b200rt_ctx *c) {
   cudaStreamSynchronize(c->stream);
   DevBuf *bufs[] = {&c->grid_tables, &c->sun_rays, &c->list_dist, &c->list_ent, &c->list_len, &c->list_flag,
                     &c->work_counter, &c->step_counter, &c->los_in, &c->los_out, &c->los_order, &c->lu, &c->lu_dinv, &c->lu_flag,
-                    &c->iph.dev, &c->iph.io, &c->vox_map, &c->sph_table, &c->kry_xchg, &c->kry_work, &c->kry_bp};
+                    &c->iph.dev, &c->iph.io, &c->vox_map, &c->sph_table, &c->kry_xchg, &c->kry_work, &c->kry_bp,
+                    &c->lw.row_ptr, &c->lw.row_cnt, &c->lw.col, &c->lw.val, &c->lw.rec, &c->lw.scratch, &c->lw.xy};
   for (DevBuf *b : bufs) b->release();
   c->host_scratch.release();
   c->host_words.release();
@@ -125,6 +126,7 @@ int b200rt_set_grid_sph(b200rt_ctx *c, int n_rb, int n_sb, int n_rays, const dou
   for (int e = 0; e < 2; e++) { c->row_sink[e] = nullptr; c->row_sink_n_vox[e] = 0; }   // named for the old geometry
   for (int e = 0; e < MAX_EMISSIONS; e++) { c->em[e].defined = c->em[e].have_K = c->em[e].have_S = false; }
   c->mult.defined = c->mult.have_K = c->mult.have_S = false;
+  c->lw.valid = false;
   return B200RT_OK;
 }
 
@@ -159,6 +161,7 @@ int b200rt_set_grid_pp(b200rt_ctx *c, int n_rb, int n_rays, const double *rb, co
   for (int e = 0; e < 2; e++) { c->row_sink[e] = nullptr; c->row_sink_n_vox[e] = 0; }   // named for the old geometry
   for (int e = 0; e < MAX_EMISSIONS; e++) { c->em[e].defined = c->em[e].have_K = c->em[e].have_S = false; }
   c->mult.defined = c->mult.have_K = c->mult.have_S = false;
+  c->lw.valid = false;
   return B200RT_OK;
 }
 
@@ -175,6 +178,7 @@ int b200rt_set_singlet(b200rt_ctx *c, int e, int n_em, double branching, double 
   cudaSetDevice(c->device);
   c->n_em = n_em;
   c->mult.defined = false;
+  c->lw.valid = false;
   Emission &E = c->em[e];
   E.branching = branching; E.T_ref = T_ref; E.sigma_ref = sigma_ref; E.g_factor = g;
   int rc = api::set_singlet(c, e, arr);
@@ -200,6 +204,7 @@ int b200rt_set_multiplet(b200rt_ctx *c, const b200rt_multiplet_desc *d, const do
     return fail(c, B200RT_ERR_ARG, "multiplet descriptor does not match the line / level tables of its kind");
   cudaSetDevice(c->device);
   c->n_em = 0;
+  c->lw.valid = false;
   for (int e = 0; e < 2; e++) { c->row_sink[e] = nullptr; c->row_sink_n_vox[e] = 0; }
   for (int e = 0; e < MAX_EMISSIONS; e++) { c->em[e].defined = c->em[e].have_K = c->em[e].have_S = false; }
   Multiplet &M = c->mult;
@@ -215,6 +220,7 @@ int b200rt_set_g_factor(b200rt_ctx *c, int e, double g) {
   if (!c || e < 0 || e >= MAX_EMISSIONS) return B200RT_ERR_ARG;
   GROUP_DISPATCH(c, group_set_g_factor(c, e, g));
   c->em[e].g_factor = g;
+  c->lw.valid = false;
   return B200RT_OK;
 }
 
@@ -522,6 +528,27 @@ int b200rt_brightness(b200rt_ctx *c, int n, const double *x, const double *y, co
   double *dst[4] = {B, tsp, tab, col};
   GROUP_DISPATCH(c, group_brightness(c, n, src, n_subsamples, dst));
   return brightness_slice(c, n, src, n_subsamples, dst, n, 0);
+}
+
+int b200rt_los_weights(b200rt_ctx *c, int n_subsamples, long long *nnz) {
+  if (!c) return B200RT_ERR_ARG;
+  GROUP_DISPATCH(c, group_los_weights(c, n_subsamples, nnz));
+  cudaSetDevice(c->device);
+  return api::los_weights(c, n_subsamples, nnz);
+}
+
+int b200rt_los_weights_download(b200rt_ctx *c, long long *row_ptr, int *col, double *val) {
+  if (!c) return B200RT_ERR_ARG;
+  GROUP_DISPATCH(c, group_los_weights_download(c, row_ptr, col, val));
+  cudaSetDevice(c->device);
+  return api::los_weights_download(c, row_ptr, 0, col, val, c->lw.nnz);
+}
+
+int b200rt_los_weights_apply(b200rt_ctx *c, int i_emission, int transpose, const double *x, double *y) {
+  if (!c || !x || !y || (transpose != 0 && transpose != 1)) return B200RT_ERR_ARG;
+  GROUP_DISPATCH(c, group_los_weights_apply(c, i_emission, transpose, x, y));
+  cudaSetDevice(c->device);
+  return api::los_weights_apply(c, i_emission, transpose, x, y);
 }
 
 int b200rt_traverse_voxel_rays(b200rt_ctx *c, int v_begin, int v_end, long long capacity, int *len, int *eb,

@@ -178,7 +178,22 @@ struct Multiplet {
   DevBuf S_real, rec_pt, rec_avg;
 };
 
-enum Phase { PH_TRAVERSE = 0, PH_INFLUENCE = 1, PH_SOLVE = 2, PH_BRIGHTNESS = 3, PH_IPH = 4, PH_ORDER = 5, PH_COUNT = 6 };
+enum Phase { PH_TRAVERSE = 0, PH_INFLUENCE = 1, PH_SOLVE = 2, PH_BRIGHTNESS = 3, PH_IPH = 4, PH_ORDER = 5,
+             PH_LW_STRUCTURE = 6, PH_LW_VALUES = 7, PH_LW_APPLY = 8, PH_COUNT = 9 };
+
+// line-of-sight weighting functions of the resident lines of sight (los_weights.cu, api_weights.cu): CSR shared by
+// the emissions, values [n_em][nnz] in Real
+struct LosWeights {
+  bool valid = false;      // cleared by a re-grid, new emission tables or g-factors, new lines of sight
+  long long nnz = 0;
+  DevBuf row_ptr;          // [n_los + 1] long long
+  DevBuf row_cnt;          // [n_los] int: row lengths of the count pass
+  DevBuf col;              // [nnz] int
+  DevBuf val;              // [n_em][nnz] Real
+  DevBuf rec;              // [n_em][2][n_vox][8] Real: the brightness records of the tables with S = 0
+  DevBuf scratch;          // scan tile sums, bitmaps of large grids
+  DevBuf xy;               // operand and result of b200rt_los_weights_apply (double)
+};
 
 // Quemerais IPH model: tables and the constants of BACKGROUND (ipbackgroundCFR_fun.f:176-235), iph.cu
 struct IphTable {
@@ -266,10 +281,11 @@ struct b200rt_ctx {
 
   // timing
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  float phase_ms[b200rt::PH_COUNT] = {0, 0, 0, 0, 0, 0};
-  int phase_launches[b200rt::PH_COUNT] = {0, 0, 0, 0, 0, 0};
+  float phase_ms[b200rt::PH_COUNT] = {};
+  int phase_launches[b200rt::PH_COUNT] = {};
 
   b200rt::IphTable iph;
+  b200rt::LosWeights lw;
 };
 
 namespace b200rt {
@@ -342,8 +358,31 @@ bool brightness_splits_emissions(int n_em, long long count);
 long long brightness_resident_groups();   // 4-lane groups the machine holds at once
 cudaError_t launch_los_order(const int *len, long long count, int cap, int *bins, int *order, cudaStream_t s);
 constexpr int LOS_ORDER_MAX_CAP = 8000;
+// em.sourcefn may be null: the records then carry S = 0
 template <class Real>
 cudaError_t launch_pack_records(const EmissionView<Real> &em, int n_vox, Real *rec_pt, Real *rec_avg, cudaStream_t s);
+
+// ---- los_weights.cu  (compiled with -fmad=false: the structure and value passes must agree on every stencil)
+// structure pass: col == nullptr counts the rows into row_cnt[first + t]; otherwise fills the columns at row_ptr[first + t].
+// bitmap_scratch: lw_bitmap_scratch_bytes(n_vox, count) bytes (0: none needed)
+size_t lw_bitmap_scratch_bytes(int n_vox, long long count);
+template <class Real>
+cudaError_t launch_lw_structure(const GridView<Real> &g, const Real *los_in, long long los_stride, long long first,
+                                long long count, ListView<Real> lists, int n_subsamples, unsigned *bitmap_scratch,
+                                int *row_cnt, const long long *row_ptr, int *col, cudaStream_t s);
+// row_ptr[0..n] = exclusive scan of row_cnt[0..n); scratch: lw_scan_scratch_bytes(n) bytes
+size_t lw_scan_scratch_bytes(long long n);
+cudaError_t launch_lw_scan(const int *row_cnt, long long n, long long *row_ptr, long long *scratch, cudaStream_t s);
+// value pass: val must be zero; *missing is set if a stencil voxel was not found in its row (an internal error)
+template <class Real>
+cudaError_t launch_lw_values(const GridView<Real> &g, const EmissionView<Real> *em, int n_em, const Real *los_in,
+                             long long los_stride, long long first, long long count, ListView<Real> lists, int n_subsamples,
+                             const long long *row_ptr, const int *col, Real *val, long long nnz, int *queue,
+                             unsigned long long *substep_counter, const int *order, int *missing, cudaStream_t s);
+// transpose 0: y[n_rows] = W x[n_vox]; 1: y[n_vox] = W^T x[n_rows]
+template <class Real>
+cudaError_t launch_lw_apply(const long long *row_ptr, const int *col, const Real *val, long long n_rows, int n_vox,
+                            int transpose, const double *x, double *y, cudaStream_t s);
 
 // ---- multiplet.cu
 template <class Real>
@@ -411,6 +450,9 @@ int group_los_upload(b200rt_ctx *g, int n, const double *x, const double *y, con
 int group_brightness_resident(b200rt_ctx *g, int n_subsamples);
 int group_los_download(b200rt_ctx *g, double *B, double *tsp, double *tab, double *col);
 int group_brightness(b200rt_ctx *g, int n, const double *const src[9], int n_subsamples, double *const dst[4]);
+int group_los_weights(b200rt_ctx *g, int n_subsamples, long long *nnz);
+int group_los_weights_download(b200rt_ctx *g, long long *row_ptr, int *col, double *val);
+int group_los_weights_apply(b200rt_ctx *g, int e, int transpose, const double *x, double *y);
 int group_traverse_los(b200rt_ctx *g, long long capacity, int *len, int *eb, int *entering, double *distance,
                        long long *n_entries);
 int group_kernel_ms(b200rt_ctx *g, int phase, float *ms, int *n_launches);

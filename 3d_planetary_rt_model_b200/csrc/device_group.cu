@@ -97,6 +97,7 @@ struct Group {
   int los_members = 0;
   long long n_los = 0;
   std::vector<long long> los_lo;
+  std::vector<long long> lw_nnz;     // line-of-sight weights: nonzeros of each member's rows (b200rt_los_weights)
   // bookkeeping of the last call(s), as b200rt_last_kernel_ms / *_count report them
   float phase_ms[PH_COUNT] = {0, 0, 0, 0, 0, 0};
   int phase_launches[PH_COUNT] = {0, 0, 0, 0, 0, 0};
@@ -471,6 +472,89 @@ int group_brightness(b200rt_ctx *g, int n, const double *const src[9], int n_sub
   collect_phases(gr, gr->los_members);
   gr->last_substeps = 0;
   for (int i = 0; i < gr->los_members; i++) gr->last_substeps += gr->m[i]->last_substeps;
+  return B200RT_OK;
+}
+
+// ---- line-of-sight weights: every member builds the rows of its slice; the matrix is their rows one after the other
+int group_los_weights(b200rt_ctx *g, int n_subsamples, long long *nnz) {
+  Group *gr = G(g);
+  if (n_subsamples == 1 || n_subsamples < 0) return fail(g, B200RT_ERR_ARG, "n_subsamples must be 0 or > 1 (RT_grid.hpp:237)");
+  if (gr->los_members <= 0) return fail(g, B200RT_ERR_STATE, "no lines of sight uploaded");
+  reset_phases(gr);
+  gr->lw_nnz.assign(gr->los_members, 0);
+  const int rc = run_members(g, gr->los_members, [&](int i) { return b200rt_los_weights(gr->m[i], n_subsamples, &gr->lw_nnz[i]); });
+  if (rc != B200RT_OK) { gr->lw_nnz.clear(); return rc; }
+  collect_phases(gr, gr->los_members);
+  gr->last_substeps = 0;
+  long long total = 0;
+  for (int i = 0; i < gr->los_members; i++) { gr->last_substeps += gr->m[i]->last_substeps; total += gr->lw_nnz[i]; }
+  if (nnz) *nnz = total;
+  return B200RT_OK;
+}
+
+namespace {
+// the members' matrices are current (not invalidated since the group's build); offsets of their first nonzero
+int lw_members_ready(b200rt_ctx *g, std::vector<long long> *offset) {
+  Group *gr = G(g);
+  if (gr->los_members <= 0 || (int) gr->lw_nnz.size() != gr->los_members)
+    return fail(g, B200RT_ERR_STATE, "line-of-sight weights not built for the current lines of sight and tables");
+  offset->assign(gr->los_members + 1, 0);
+  for (int i = 0; i < gr->los_members; i++) {
+    long long k = 0;
+    if (api::los_weights_nnz(gr->m[i], &k) != B200RT_OK || k != gr->lw_nnz[i]) {
+      g->err = "device " + std::to_string(gr->m[i]->device) + ": " + gr->m[i]->err;
+      return B200RT_ERR_STATE;
+    }
+    (*offset)[i + 1] = (*offset)[i] + k;
+  }
+  return B200RT_OK;
+}
+}  // namespace
+
+int group_los_weights_download(b200rt_ctx *g, long long *row_ptr, int *col, double *val) {
+  Group *gr = G(g);
+  std::vector<long long> off;
+  if (int rc = lw_members_ready(g, &off)) return rc;
+  const long long total = off[gr->los_members];
+  // row_ptr: each member's n_i + 1 entries into its own buffer first (neighbours share the boundary entry)
+  std::vector<std::vector<long long>> rp(gr->los_members);
+  const int rc = run_members(g, gr->los_members, [&](int i) {
+    if (row_ptr) rp[i].resize(gr->los_lo[i + 1] - gr->los_lo[i] + 1);
+    cudaSetDevice(gr->m[i]->device);
+    return api::los_weights_download(gr->m[i], row_ptr ? rp[i].data() : nullptr, off[i], col ? col + off[i] : nullptr,
+                                     val ? val + off[i] : nullptr, total);
+  });
+  if (rc != B200RT_OK) return rc;
+  if (row_ptr) {
+    for (int i = 0; i < gr->los_members; i++)
+      std::copy(rp[i].begin(), rp[i].end() - 1, row_ptr + gr->los_lo[i]);
+    row_ptr[gr->n_los] = total;
+  }
+  return B200RT_OK;
+}
+
+int group_los_weights_apply(b200rt_ctx *g, int e, int transpose, const double *x, double *y) {
+  Group *gr = G(g);
+  std::vector<long long> off;
+  if (int rc = lw_members_ready(g, &off)) return rc;
+  reset_phases(gr);
+  int rc;
+  if (!transpose) {
+    rc = run_members(g, gr->los_members, [&](int i) { return b200rt_los_weights_apply(gr->m[i], e, 0, x, y + gr->los_lo[i]); });
+  } else {
+    // each member's n_vox partial sums over its rows, added on the host in member order
+    const int n_vox = gr->m[0]->hg.n_vox;
+    std::vector<std::vector<double>> part(gr->los_members);
+    rc = run_members(g, gr->los_members, [&](int i) {
+      if (i > 0) part[i].resize(n_vox);
+      return b200rt_los_weights_apply(gr->m[i], e, 1, x + gr->los_lo[i], i == 0 ? y : part[i].data());
+    });
+    if (rc == B200RT_OK)
+      for (int i = 1; i < gr->los_members; i++)
+        for (int v = 0; v < n_vox; v++) y[v] += part[i][v];
+  }
+  if (rc != B200RT_OK) return rc;
+  collect_phases(gr, gr->los_members);
   return B200RT_OK;
 }
 

@@ -1,6 +1,8 @@
 // capi.cpp -- flat C handles over the observation_fit facade, for ctypes-driven tests and for bindings
 // that cannot consume C++ (the reference's own binding is Cython on the C++ class, python/py_corona_sim.pyx).
 #include <fstream>
+#include <map>
+#include <mutex>
 #include <csignal>
 #include <cstdlib>
 #include <cstring>
@@ -42,6 +44,12 @@ struct install_handler {
 } g_install_handler;
 }
 
+// obsfit_brightness_weights keeps the matrix here until obsfit_brightness_weights_get copies it out
+namespace {
+std::mutex g_weights_mu;
+std::map<void *, observation_fit::csr_matrix> g_weights;
+}
+
 extern "C" {
 const char *obsfit_last_error() { return g_err.c_str(); }
 void *obsfit_create_ex(const char *iph_fname, int device, int single_precision) {
@@ -54,7 +62,13 @@ void *obsfit_create(const char *iph_fname, int device) {
   if (guard([&] { o = new observation_fit(iph_fname ? iph_fname : "", device); })) return nullptr;
   return o;
 }
-void obsfit_destroy(void *h) { delete static_cast<observation_fit *>(h); }
+void obsfit_destroy(void *h) {
+  {
+    std::lock_guard<std::mutex> lock(g_weights_mu);
+    g_weights.erase(h);
+  }
+  delete static_cast<observation_fit *>(h);
+}
 int obsfit_add_observation(void *h, int n, const double *loc, const double *dir) {
   return guard([&] { static_cast<observation_fit *>(h)->add_observation(rows3(n, loc), rows3(n, dir)); });
 }
@@ -209,6 +223,31 @@ int obsfit_source_function(void *h, int e, double *out) {
 }
 int obsfit_radial_boundaries(void *h, double *out) {
   return guard([&] { auto s = static_cast<observation_fit *>(h)->radial_boundaries(); std::memcpy(out, s.data(), s.size() * sizeof(double)); });
+}
+// line-of-sight weighting functions (observation_fit::brightness_weights): the CSR of emission e of model `which` is
+// built and kept in the handle; *nnz, *n_rows, *n_cols tell the caller what to allocate for obsfit_brightness_weights_get
+int obsfit_brightness_weights(void *h, int e, int which, long long *nnz, int *n_rows, int *n_cols) {
+  return guard([&] {
+    observation_fit::csr_matrix m = static_cast<observation_fit *>(h)->brightness_weights(e, which);
+    std::lock_guard<std::mutex> lock(g_weights_mu);
+    auto &w = g_weights[h];
+    w = std::move(m);
+    *nnz = (long long) w.indices.size();
+    *n_rows = w.n_rows;
+    *n_cols = w.n_cols;
+  });
+}
+int obsfit_brightness_weights_get(void *h, long long *indptr, int *indices, double *data) {
+  return guard([&] {
+    std::lock_guard<std::mutex> lock(g_weights_mu);
+    auto it = g_weights.find(h);
+    if (it == g_weights.end()) throw std::runtime_error("obsfit_brightness_weights_get: call obsfit_brightness_weights first");
+    const auto &w = it->second;
+    std::memcpy(indptr, w.indptr.data(), w.indptr.size() * sizeof(long long));
+    std::memcpy(indices, w.indices.data(), w.indices.size() * sizeof(int));
+    std::memcpy(data, w.data.data(), w.data.size() * sizeof(double));
+    g_weights.erase(it);
+  });
 }
 // out[n_sets][2][n_obs]
 int obsfit_brightness_batch(void *h, int n_sets, const double *nH, const double *T, int contexts_per_gpu, int n_gpus,

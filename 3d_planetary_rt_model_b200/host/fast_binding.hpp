@@ -51,4 +51,18 @@ inline int fetch(observation_fit *o, int which, double *out) {
 }
 inline int fetch_cols(observation_fit *o, int) { return o->n_obs(); }   // length of one row of fetch(which)
 
+// observation_fit::brightness_weights into a matrix the caller keeps (new) and frees (weights_free) after copying it out
+inline observation_fit::csr_matrix *weights(observation_fit *o, int e, int which) {
+  return new observation_fit::csr_matrix(o->brightness_weights(e, which));
+}
+inline long long weights_nnz(const observation_fit::csr_matrix *w) { return (long long) w->indices.size(); }
+inline int weights_rows(const observation_fit::csr_matrix *w) { return w->n_rows; }
+inline int weights_cols(const observation_fit::csr_matrix *w) { return w->n_cols; }
+inline void weights_copy(const observation_fit::csr_matrix *w, long long *indptr, int *indices, double *data) {
+  std::memcpy(indptr, w->indptr.data(), w->indptr.size() * sizeof(long long));
+  std::memcpy(indices, w->indices.data(), w->indices.size() * sizeof(int));
+  std::memcpy(data, w->data.data(), w->data.size() * sizeof(double));
+}
+inline void weights_free(observation_fit::csr_matrix *w) { delete w; }
+
 }  // namespace b200_fast

@@ -414,6 +414,33 @@ vector<vector<observation_fit::Real>> observation_fit::iph_brightness_unextincte
   return r;
 }
 
+observation_fit::csr_matrix observation_fit::brightness_weights(int e, int which) {
+  if (which == 2 || which == 3)
+    throw std::invalid_argument("brightness_weights: the plane-parallel grid has no brightness (grid_plane_parallel.hpp:304-311)");
+  if (which != 0 && which != 1) throw std::invalid_argument("brightness_weights: model must be 0 (H) or 1 (D)");
+  if (e < 0 || e >= n_hydrogen_emissions) throw std::invalid_argument("brightness_weights: bad emission index");
+  singlet_model &m = singlet(which);
+  if (!m.have_S) throw std::runtime_error("observation_fit: generate a source function before asking for brightness weights");
+  if (n_obs() == 0) throw std::runtime_error("there must be at least one observation to simulate");
+  b200rt_ctx *c = m.ctx;
+  if (!m.los_uploaded) {
+    check(b200rt_los_upload(c, n_obs(), los[0].data(), los[1].data(), los[2].data(), los[3].data(), los[4].data(),
+                            los[5].data(), los[6].data(), los[7].data(), los[8].data()), c);
+    m.los_uploaded = true;
+  }
+  long long nnz = 0;
+  check(b200rt_los_weights(c, 10, &nnz), c);
+  csr_matrix r;
+  r.n_rows = n_obs();
+  r.n_cols = m.in.n_vox;
+  r.indptr.resize((size_t) r.n_rows + 1);
+  r.indices.resize((size_t) nnz);
+  vector<double> val((size_t) n_hydrogen_emissions * nnz);
+  check(b200rt_los_weights_download(c, r.indptr.data(), r.indices.data(), val.data()), c);
+  r.data.assign(val.begin() + (size_t) e * nnz, val.begin() + (size_t) (e + 1) * nnz);
+  return r;
+}
+
 // deuterium_RT / deuterium_obs (observation_fit.cpp:591-637)
 vector<vector<observation_fit::Real>> observation_fit::D_brightness() {
   singlet_model &m = singlet(1);

@@ -147,6 +147,17 @@ public:
   std::vector<Real> multiplet_source_function(int model);
   int n_obs() const { return (int) los[0].size(); }
 
+  // ---- line-of-sight weighting functions of the H (which = 0) or D (1) model for the current observations, with
+  // n_subsamples = 10 like brightness(): W (n_obs x n_vox, CSR) with W * source_function(e, which) = brightness()[e]
+  // without the IPH term.  The plane-parallel models (2, 3) have no brightness and throw.
+  struct csr_matrix {
+    int n_rows = 0, n_cols = 0;
+    std::vector<long long> indptr;   // [n_rows + 1]
+    std::vector<int> indices;        // [nnz] voxel ids, ascending within a row
+    std::vector<Real> data;          // [nnz]
+  };
+  csr_matrix brightness_weights(int i_emission, int which = 0);
+
 private:
   struct set_inputs;       // grid + the eight tables of each emission for one parameter set
   struct singlet_model;    // one RT_grid<singlet_CFR, 2, grid> of the reference + its observation outputs

@@ -21,6 +21,14 @@ cdef extern from "fast_binding.hpp" namespace "b200_fast" nogil:
     int b200_n_obs "b200_fast::n_obs"(const observation_fit *o)
     int b200_fetch "b200_fast::fetch"(observation_fit *o, int which, double *out) except +
     int b200_fetch_cols "b200_fast::fetch_cols"(observation_fit *o, int which)
+    cppclass b200_csr "observation_fit::csr_matrix":
+        pass
+    b200_csr *b200_weights "b200_fast::weights"(observation_fit *o, int e, int which) except +
+    long long b200_weights_nnz "b200_fast::weights_nnz"(const b200_csr *w)
+    int b200_weights_rows "b200_fast::weights_rows"(const b200_csr *w)
+    int b200_weights_cols "b200_fast::weights_cols"(const b200_csr *w)
+    void b200_weights_copy "b200_fast::weights_copy"(const b200_csr *w, long long *indptr, int *indices, double *data)
+    void b200_weights_free "b200_fast::weights_free"(b200_csr *w)
 
 
 cdef class Pyobservation_fit_b200(Pyobservation_fit):
@@ -103,3 +111,21 @@ cdef class Pyobservation_fit_b200(Pyobservation_fit):
 
     def tau_D_final(self):
         return self._fetch(8)
+
+    def brightness_weights(self, int i_emission, int which=0):
+        """line-of-sight weighting functions of the H (which = 0) or D (1) model for the current observations:
+        (indptr, indices, data) with scipy.sparse.csr_matrix((data, indices, indptr), shape=(n_obs, n_voxels)) times
+        the source function = the brightness without the IPH term"""
+        cdef b200_csr *w
+        with nogil:
+            w = b200_weights(self.thisptr, i_emission, which)
+        cdef long long nnz = b200_weights_nnz(w)
+        indptr = np.empty(b200_weights_rows(w) + 1, dtype=np.int64)
+        indices = np.empty(max(nnz, 1), dtype=np.int32)
+        data = np.empty(max(nnz, 1), dtype=np.float64)
+        cdef long long[::1] P = indptr
+        cdef int[::1] I = indices
+        cdef double[::1] D = data
+        b200_weights_copy(w, &P[0], &I[0], &D[0])
+        b200_weights_free(w)
+        return indptr, indices[:nnz], data[:nnz]

@@ -53,6 +53,9 @@ SIGNATURES = {
     "obsfit_write_S_file": (C.c_int, [C.c_char_p, C.c_int, C.c_int, _dp, _dp, _dp, _dp, C.c_int, C.POINTER(C.c_char_p), _dp]),
     "obsfit_write_influence_file": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_char_p), _dp, C.c_int]),
     "obsfit_multiplet_source_function": (C.c_int, [_vp, C.c_int, _dp, C.c_int, C.POINTER(C.c_int)]),
+    "obsfit_brightness_weights": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(C.c_longlong), C.POINTER(C.c_int),
+                                            C.POINTER(C.c_int)]),
+    "obsfit_brightness_weights_get": (C.c_int, [_vp, _vp, _vp, _vp]),
 }
 MODEL_H, MODEL_D, MODEL_H_PP, MODEL_D_PP = 0, 1, 2, 3
 _lib = None
@@ -270,6 +273,19 @@ class Pyobservation_fit:
         out = np.zeros(self.n_vox if which < 2 else self.n_rb - 1)
         self._ck(self.lib.obsfit_source_function_ex(self.h, e, which, out))
         return out
+
+    def brightness_weights(self, e, which=MODEL_H):
+        """line-of-sight weighting functions of emission e of model `which` for the current observations:
+        (indptr, indices, data, shape); scipy.sparse.csr_matrix((data, indices, indptr), shape=shape) times
+        source_function(e, which) is brightness()[e] without the IPH term"""
+        nnz, nr, nc = C.c_longlong(0), C.c_int(0), C.c_int(0)
+        self._ck(self.lib.obsfit_brightness_weights(self.h, e, which, C.byref(nnz), C.byref(nr), C.byref(nc)))
+        indptr = np.zeros(nr.value + 1, np.int64)
+        indices = np.zeros(max(nnz.value, 1), np.int32)
+        data = np.zeros(max(nnz.value, 1))
+        self._ck(self.lib.obsfit_brightness_weights_get(self.h, indptr.ctypes.data_as(_vp), indices.ctypes.data_as(_vp),
+                                                        data.ctypes.data_as(_vp)))
+        return indptr, indices[:nnz.value], data[:nnz.value], (nr.value, nc.value)
 
     def radial_boundaries(self, which=MODEL_H):
         out = np.zeros(self.n_rb)

@@ -301,6 +301,42 @@ int b200rt_brightness_resident(b200rt_ctx *ctx, int n_subsamples);
 int b200rt_los_download(b200rt_ctx *ctx, double *brightness, double *tau_species_final,
                         double *tau_absorber_final, double *species_col_dens);
 
+/* ---- line-of-sight weighting functions -------------------------------------------------
+ * The brightness of a singlet emission is linear in its source function: in RT_grid::brightness (RT_grid.hpp:233-299)
+ * every sub-step adds S_interp * g * w / sigma_ref / sqrt(pi) / 1e9 * T_int, where S_interp = sum_k w_k S[idx_k] is the
+ * 4-corner interpolation of S and T_int (clamped at tau_species_voxel) depends on the emission tables and the geometry
+ * only.  So brightness_e = W_e S_e, with W_e a sparse n_los x n_vox matrix: contribution functions (where along each
+ * line of sight the emission originates), the exact derivative d brightness / d S, and a cheap re-evaluation when only S
+ * changes.  The IPH background is not part of W (it does not depend on S).
+ *   b200rt_los_weights: builds W_e for every singlet emission on the lines of sight resident in the context
+ *     (b200rt_los_upload), with b200rt_brightness's n_subsamples rule: 0 = one step per segment with the voxel-average
+ *     tables (brightness_nointerp), 1 = illegal (B200RT_ERR_ARG), otherwise interpolated sub-steps.  It needs the grid
+ *     and the emission tables, not a source function (it works before any solve).  *nnz (may be NULL) = stored entries.
+ *     W[l, v] = sum over l's sub-steps, in march order, of w_k * gfac * T_int for every stencil corner k with idx_k == v
+ *     (without interpolation: the current voxel with weight 1); gfac = g_factor * branching / sigma_ref / sqrt(pi) / 1e9,
+ *     so W_e S_e is in kR.  Column v is stored in row l iff some sub-step of l reads v with a nonzero interpolation
+ *     weight; columns of a row are ascending and unique; a stored value may be exactly 0 (e.g. zero density); a line of
+ *     sight that misses the grid has an empty row.  The structure is shared by the emissions.  The values are a
+ *     deterministic function of the inputs (two builds, and a device group against a plain context, give the same
+ *     bytes).  In a float context they are accumulated in float and widened on download.
+ *     b200rt_last_substep_count reports the sub-steps of the build; b200rt_last_kernel_ms: phase 6 = structure passes,
+ *     7 = value pass (and 0 / 5 the traversal and ordering kernels it runs).
+ *     Refused with B200RT_ERR_STATE: a multiplet context, a plane-parallel grid (no brightness there either), no lines
+ *     of sight; with B200RT_ERR_NOMEM: device memory too small for the matrix.
+ *   The matrix stays on the device until the next build; a re-grid, new emission tables or g-factors, or new lines of
+ *   sight (b200rt_los_upload, b200rt_brightness) make it stale, and download / apply then return B200RT_ERR_STATE.
+ *   b200rt_los_weights_download: CSR of the matrix: row_ptr[n_los + 1] (int64, row_ptr[0] = 0, row_ptr[n_los] = nnz),
+ *     col[nnz] (voxel ids), val[n_emissions][nnz].  Any pointer may be NULL.
+ *   b200rt_los_weights_apply: transpose 0: y[n_los] = W_e x[n_vox]; 1: y[n_vox] = W_e^T x[n_los], in double.  W x sums
+ *     each row in a fixed order (the same bits every run; not those of a sequential sum).  W^T x adds with atomics: its
+ *     last bits may vary between runs.  b200rt_last_kernel_ms phase 8 = the product kernel.
+ * A device group splits the lines of sight by index, as for the brightness: every member builds the rows of its slice;
+ * download stitches the rows in order, W x fills each member's slice of y, W^T x adds the members' n_vox partial
+ * vectors on the host in member order. */
+int b200rt_los_weights(b200rt_ctx *ctx, int n_subsamples, long long *nnz);
+int b200rt_los_weights_download(b200rt_ctx *ctx, long long *row_ptr, int *col, double *val);
+int b200rt_los_weights_apply(b200rt_ctx *ctx, int i_emission, int transpose, const double *x, double *y);
+
 /* ---- interplanetary hydrogen background ---------------------------------------------
  * replaces quemerais_iph_model -> Fortran BACKGROUND (quemerais_IPH_model/iph_model_interface.cpp:19-82,
  * ipbackgroundCFR_fun.f:1-741).  The table file (fsm99td12v20t80 layout, :107-164) is parsed ONCE per
@@ -341,7 +377,8 @@ int b200rt_traverse_los(b200rt_ctx *ctx, long long capacity,
 /* ---- timing ---------------------------------------------------------------------
  * device time (CUDA events on the ctx stream) of the kernels of the last call:
  * phase 0 = traversal, 1 = influence march, 2 = solve, 3 = brightness march (the march launches alone),
- * 4 = IPH, 5 = the longest-first ordering kernels of the lines of sight (3 launches per batch) */
+ * 4 = IPH, 5 = the longest-first ordering kernels of the lines of sight (3 launches per batch),
+ * 6 / 7 / 8 = line-of-sight weights: structure passes (count, scan, fill), value pass, products (b200rt_los_weights*) */
 int b200rt_last_kernel_ms(b200rt_ctx *ctx, int phase, float *ms, int *n_launches);
 int b200rt_synchronize(b200rt_ctx *ctx);
 /* measured FP64 peaks of this device (TFLOP/s): plain DFMA and DMMA.8x8x4 (mma.sync m8n8k4.f64).
