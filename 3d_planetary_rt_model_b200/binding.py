@@ -18,6 +18,7 @@ F64, F32 = 0, 1
 ROW_MAJOR, COL_MAJOR = 0, 1
 PH_TRAVERSE, PH_INFLUENCE, PH_SOLVE, PH_BRIGHTNESS, PH_IPH, PH_ORDER = 0, 1, 2, 3, 4, 5
 PH_LW_STRUCTURE, PH_LW_VALUES, PH_LW_APPLY = 6, 7, 8
+PH_TRANSPOSE = 9
 
 _dp = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")
 _ip = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
@@ -48,6 +49,7 @@ SIGNATURES = {
     "b200rt_solve_exchange": (C.c_int, [_vp, C.POINTER(C.c_void_p), C.c_char_p]),
     "b200rt_solve_distributed": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "b200rt_last_solve_steps": (C.c_int, [_vp, C.POINTER(C.c_int)]),
+    "b200rt_solve_adjoint": (C.c_int, [_vp, C.c_int, C.c_int, _vp, _vp, _vp, _vp]),
     "b200rt_multiplet_desc_init": (C.c_int, [C.c_int, C.c_int, _vp]),
     "b200rt_set_multiplet": (C.c_int, [_vp, _vp] + [_dp] * 6),
     "b200rt_generate_S": (C.c_int, [_vp]),
@@ -375,6 +377,18 @@ class Context:
         self._ck(self.lib.b200rt_los_download(self.h, *[_ptr(o) for o in out]))
         return dict(brightness=out[0], tau_species_final=out[1], tau_absorber_final=out[2], species_col_dens=out[3])
 
+    def solve_adjoint(self, e, rhs):
+        """b200rt_solve_adjoint: lam = (I - w K)^-T rhs for a 1-D rhs (n unknowns) or each row of a 2-D one ->
+        (lam, steps, residuals), lam shaped like rhs; r . S = lam . S0 for the solved S"""
+        rhs = np.ascontiguousarray(rhs, dtype=np.float64)
+        r2 = np.atleast_2d(rhs)
+        n_rhs = r2.shape[0]
+        lam = np.zeros_like(r2)
+        steps = np.zeros(n_rhs, np.int32)
+        res = np.zeros(n_rhs)
+        self._ck(self.lib.b200rt_solve_adjoint(self.h, e, n_rhs, _ptr(r2), _ptr(lam), _ptr(steps), _ptr(res)))
+        return (lam.reshape(rhs.shape), steps, res)
+
     # ---- line-of-sight weighting functions: brightness_e = W_e S_e on the resident lines of sight
     def los_weights(self, n_subsamples=10):
         """b200rt_los_weights: builds W for every emission; returns nnz"""
@@ -550,6 +564,18 @@ class GpuModel:
         self.ctx.los_weights(n_subsamples)
         return self.ctx.los_weights_download()
 
+    def solve_adjoint(self, e, rhs):
+        """(lam, steps, residuals): lam = (I - w K)^-T rhs on the resident K of emission e"""
+        return self.ctx.solve_adjoint(e, rhs)
+
+    def brightness_source_sensitivity(self, locs, dirs, w, e, n_subsamples=10):
+        """d(sum_l w_l brightness_e,l) / dS0_e over the voxels: W_e of these lines of sight, r = W_e^T w, then the
+        adjoint solve (r . S = lam . S0).  Needs the influence matrix (build_rows)."""
+        self.ctx.los_upload(self.ctx.los_from_MSO(locs, dirs))
+        self.ctx.los_weights(n_subsamples)
+        r = self.ctx.los_weights_apply(e, np.asarray(w, dtype=np.float64), transpose=True)
+        return self.ctx.solve_adjoint(e, r)[0]
+
 
 def define_multiplet_tables(scn, precision=F64):
     """Host restatement of O_1026_emission::define (reference emission/O_1026.hpp:134-217: Boltzmann populations of
@@ -641,3 +667,7 @@ class GpuMultiplet:
 
     def brightness(self, locs, dirs, n_subsamples=10):
         return self.ctx.brightness(self.ctx.los_from_MSO(locs, dirs), n_subsamples)
+
+    def solve_adjoint(self, rhs):
+        """(lam, steps, residuals): lam = (I - K)^-T rhs over the n_el element unknowns (voxel * n_upper + state)"""
+        return self.ctx.solve_adjoint(0, rhs)

@@ -45,6 +45,7 @@ int b200rt_destroy(b200rt_ctx *c) {
   DevBuf *bufs[] = {&c->grid_tables, &c->sun_rays, &c->list_dist, &c->list_ent, &c->list_len, &c->list_flag,
                     &c->work_counter, &c->step_counter, &c->los_in, &c->los_out, &c->los_order, &c->lu, &c->lu_dinv, &c->lu_flag,
                     &c->iph.dev, &c->iph.io, &c->vox_map, &c->sph_table, &c->kry_xchg, &c->kry_work, &c->kry_bp,
+                    &c->kry_adj_xchg, &c->kry_adj_work, &c->kry_kt, &c->kry_adj_io,
                     &c->lw.row_ptr, &c->lw.row_cnt, &c->lw.col, &c->lw.val, &c->lw.rec, &c->lw.scratch, &c->lw.xy};
   for (DevBuf *b : bufs) b->release();
   c->host_scratch.release();
@@ -470,6 +471,15 @@ int b200rt_solve_distributed(b200rt_ctx *c, int rank, int world, void *const *bl
   if (!c->have_grid || (c->n_em < 1 && !c->mult.defined)) return fail(c, B200RT_ERR_STATE, "grid / emissions not set");
   cudaSetDevice(c->device);
   return api::solve_distributed(c, rank, world, blocks, true);
+}
+int b200rt_solve_adjoint(b200rt_ctx *c, int i_emission, int n_rhs, const double *rhs, double *lambda, int *n_steps,
+                         double *residual) {
+  if (!c) return B200RT_ERR_ARG;
+  if (n_rhs < 1 || !rhs || !lambda) return fail(c, B200RT_ERR_ARG, "b200rt_solve_adjoint: n_rhs < 1, or rhs / lambda NULL");
+  GROUP_DISPATCH(c, group_solve_adjoint(c, i_emission, n_rhs, rhs, lambda, n_steps, residual));
+  if (!c->have_grid || (c->n_em < 1 && !c->mult.defined)) return fail(c, B200RT_ERR_STATE, "grid / emissions not set");
+  cudaSetDevice(c->device);
+  return api::solve_adjoint(c, i_emission, n_rhs, rhs, lambda, n_steps, residual, false);
 }
 int b200rt_last_solve_steps(b200rt_ctx *c, int *n_steps) {
   if (!c || !n_steps) return B200RT_ERR_ARG;

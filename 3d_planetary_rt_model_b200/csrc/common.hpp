@@ -179,7 +179,7 @@ struct Multiplet {
 };
 
 enum Phase { PH_TRAVERSE = 0, PH_INFLUENCE = 1, PH_SOLVE = 2, PH_BRIGHTNESS = 3, PH_IPH = 4, PH_ORDER = 5,
-             PH_LW_STRUCTURE = 6, PH_LW_VALUES = 7, PH_LW_APPLY = 8, PH_COUNT = 9 };
+             PH_LW_STRUCTURE = 6, PH_LW_VALUES = 7, PH_LW_APPLY = 8, PH_TRANSPOSE = 9, PH_COUNT = 10 };
 
 // line-of-sight weighting functions of the resident lines of sight (los_weights.cu, api_weights.cu): CSR shared by
 // the emissions, values [n_em][nnz] in Real
@@ -264,6 +264,10 @@ struct b200rt_ctx {
   std::vector<std::pair<int, int>> built_ranges;
   unsigned long long kry_round_base = 0;
   int kry_last_iters = 0;
+  // the adjoint solve (b200rt_solve_adjoint): its own exchange block, work area and round counter (its rounds must not
+  // advance the forward solve's), K^T (n^2 doubles, rebuilt on every call) and the right-hand sides / solutions
+  b200rt::DevBuf kry_adj_xchg, kry_adj_work, kry_kt, kry_adj_io;
+  unsigned long long kry_adj_round_base = 0;
   bool solve_attrs_set = false;              // the LU kernels' dynamic shared memory limits were raised on this device
   cudaGraphExec_t lu_graph = nullptr;        // the factorisation + back substitution of one (np, workspace), replayed
   int lu_graph_np = 0, lu_graph_launches = 0;
@@ -453,6 +457,7 @@ int group_brightness(b200rt_ctx *g, int n, const double *const src[9], int n_sub
 int group_los_weights(b200rt_ctx *g, int n_subsamples, long long *nnz);
 int group_los_weights_download(b200rt_ctx *g, long long *row_ptr, int *col, double *val);
 int group_los_weights_apply(b200rt_ctx *g, int e, int transpose, const double *x, double *y);
+int group_solve_adjoint(b200rt_ctx *g, int e, int n_rhs, const double *rhs, double *lambda, int *n_steps, double *residual);
 int group_traverse_los(b200rt_ctx *g, long long capacity, int *len, int *eb, int *entering, double *distance,
                        long long *n_entries);
 int group_kernel_ms(b200rt_ctx *g, int phase, float *ms, int *n_launches);
@@ -471,6 +476,10 @@ int measure_fp64_peaks(b200rt_ctx *c, double *dfma_tflops, double *dmma_tflops);
 namespace api {
 int exchange_block(b200rt_ctx *c, void **dev_ptr);
 int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, bool reset_timer, int cta_cap = 0);
+// lambda[k] = (I - w K)^-T rhs[k] on this context's K (world = 1); rows_complete: K holds every row although the last
+// influence call built only some of them here (a device group after gathering distributed rows)
+int solve_adjoint(b200rt_ctx *c, int e, int n_rhs, const double *rhs, double *lambda, int *n_steps, double *residual,
+                  bool rows_complete);
 }
 // ---- solve.cu
 struct SolveResult { double residual; double min_margin; int launches; };

@@ -113,6 +113,7 @@ struct Group {
   // the assembled matrix afterwards: rows_gathered)
   int kry_min_n = 2048;
   bool distributed = false, rows_gathered = true;
+  bool all_rows = false;             // the last build covered every voxel (the adjoint solve needs all of K)
   std::vector<std::vector<int>> shard_b, shard_e;
 };
 
@@ -173,6 +174,7 @@ int influence_rows(b200rt_ctx *g, int n_ranges, const int *vb, const int *ve) {
     n_rows += ve[i] - vb[i];
   }
   const int n_mem = (int) gr->m.size();
+  gr->all_rows = n_rows == p->hg.n_vox;
   // large grids, every row of the grid in this build: the rows stay on their members and the solve is distributed
   const long long n_el = (long long) p->hg.n_vox * (p->mult.defined ? p->mult.d.n_upper : 1);
   const bool distributed = p->hg.n_vox >= gr->kry_min_n && n_el <= B200RT_KRYLOV_MAX_N && n_mem <= B200RT_KRYLOV_MAX_WORLD &&
@@ -555,6 +557,24 @@ int group_los_weights_apply(b200rt_ctx *g, int e, int transpose, const double *x
   }
   if (rc != B200RT_OK) return rc;
   collect_phases(gr, gr->los_members);
+  return B200RT_OK;
+}
+
+// the adjoint runs on the member that holds every row of K (gathered there first after a distributed build: the
+// primary's own record of what it built then still names only its shard)
+int group_solve_adjoint(b200rt_ctx *g, int e, int n_rhs, const double *rhs, double *lambda, int *n_steps, double *residual) {
+  Group *gr = G(g);
+  b200rt_ctx *p = gr->m[0];
+  if (!p->have_grid || (p->n_em < 1 && !p->mult.defined)) return fail(g, B200RT_ERR_STATE, "grid / emissions not set");
+  if (p->mult.defined ? e != 0 : (e < 0 || e >= p->n_em)) return fail(g, B200RT_ERR_ARG, "b200rt_solve_adjoint: bad emission index");
+  if (!gr->all_rows)
+    return fail(g, B200RT_ERR_STATE, "b200rt_solve_adjoint: the last influence build did not cover every voxel");
+  reset_phases(gr);
+  b200rt_ctx *o = group_owner_K(g, e);
+  cudaSetDevice(o->device);
+  const int rc = api::solve_adjoint(o, e, n_rhs, rhs, lambda, n_steps, residual, true);
+  if (rc != B200RT_OK) { g->err = o->err; return rc; }
+  for (int q = 0; q < PH_COUNT; q++) { gr->phase_ms[q] = o->phase_ms[q]; gr->phase_launches[q] = o->phase_launches[q]; }
   return B200RT_OK;
 }
 

@@ -1234,11 +1234,324 @@ kry_loop(KryLoopArgs a) {
   }
 }
 
+// =====================================================================================================================
+// The adjoint system (I - w K)^T lambda = r runs through the machinery above unchanged, on K^T: the preconditioner's
+// set-up then builds the diagonal blocks of A^T (= M^T), their inverses and the rows of A^T M^-T, kry_loop iterates with
+// the tuned row product, and its true-residual pass checks the adjoint system itself.  (A column-wise product inside
+// kry_loop would have to reduce full-length partial vectors in every step.)  Kt = K^T, n x n row major, through padded
+// 32 x 32 tiles in shared memory: reads and writes are rows of 256 bytes, K streams through L2 with evict-first loads
+// (273 MB on the 100x60 grid, more than L2 holds).  The padding keeps both tile accesses free of bank conflicts (a double
+// spans two banks; a warp's 256 bytes go out as two half-warp phases).
+constexpr int KT_TILE = 32, KT_ROWS = 8;
+__global__ void __launch_bounds__(KT_TILE * KT_ROWS)
+kry_transpose(const double *__restrict__ K, int n, double *__restrict__ Kt) {
+  __shared__ double tile[KT_TILE][KT_TILE + 1];
+  const int tx = threadIdx.x, ty = threadIdx.y;
+  const int c0 = blockIdx.x * KT_TILE, r0 = blockIdx.y * KT_TILE;
+  double v[KT_TILE / KT_ROWS];
+#pragma unroll
+  for (int k = 0; k < KT_TILE / KT_ROWS; k++) {
+    const int r = r0 + ty + k * KT_ROWS, col = c0 + tx;
+    v[k] = (r < n && col < n) ? __ldcs(K + (size_t) r * n + col) : 0.0;
+  }
+#pragma unroll
+  for (int k = 0; k < KT_TILE / KT_ROWS; k++) tile[ty + k * KT_ROWS][tx] = v[k];
+  __syncthreads();
+#pragma unroll
+  for (int k = 0; k < KT_TILE / KT_ROWS; k++) {
+    const int r = c0 + ty + k * KT_ROWS, col = r0 + tx;     // row r of Kt = column r of K
+    if (r < n && col < n) Kt[(size_t) r * n + col] = tile[tx][ty + k * KT_ROWS];
+  }
+}
+
 size_t carve_bytes(size_t &off, size_t bytes) {
   off = (off + 255) & ~size_t(255);
   const size_t at = off;
   off += bytes;
   return at;
+}
+
+// One rank's GMRES over a fixed set of rows, for one system after another (the forward solve: every emission; the
+// adjoint: every right-hand side).  kry_open carves the work area and uploads the rows; kry_setup builds the
+// preconditioner of one matrix (K, branching); kry_iterate launches the iteration for one right-hand side into one
+// solution vector.  No iteration launch writes what kry_setup wrote (Minv and Bp of the work area, pre[] of the exchange
+// blocks): one set-up serves any number of right-hand sides.
+struct KrySolver {
+  KryWork wk;
+  KryPeers pe;
+  int *d_rows;
+  int n, n_rows, cta_cap;
+  bool pc, fused;                    // fused: the one-launch form (B200RT_KRYLOV_FUSED=0: the per-step launches)
+  int pc_run, pc_blocks;
+  double tol;
+  int max_it, post_blocks, orth_blocks;
+  KryState *h_st;                    // page-locked: [0, 63) the per-step form's chunk read-backs, [63 + k] final state k
+  bool trace;                        // B200RT_KRYLOV_TRACE=1: event marks around the set-up and the first 48 steps
+  std::vector<cudaEvent_t> marks;
+};
+
+// work: this solver's work area; round_base: the round counter its exchange blocks have reached (restored when the work
+// area is new); n_final: final states the caller reads back
+int kry_open(b200rt_ctx *c, const std::vector<int> &rows, int n, int nu, DevBuf &work, unsigned long long round_base,
+             void *const *blocks, int rank, int world, int cta_cap, int n_final, KrySolver &ks) {
+  const int n_rows = (int) rows.size();
+  const int ns = (n + 31) & ~31;
+  size_t off = 0;
+  const size_t o_st = carve_bytes(off, sizeof(KryState));
+  const size_t o_V = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * ns * sizeof(double));
+  const size_t o_w = carve_bytes(off, (size_t) ns * sizeof(double)), o_b = carve_bytes(off, (size_t) ns * sizeof(double)),
+               o_x = carve_bytes(off, (size_t) ns * sizeof(double));
+  const size_t o_p1 = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * KRY_MAX_B * sizeof(double)),
+               o_p2 = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * KRY_MAX_B * sizeof(double));
+  const size_t o_np = carve_bytes(off, KRY_MAX_B * sizeof(double));
+  const size_t o_R = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * KRY_MAX_IT * sizeof(double));
+  const size_t o_cs = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)), o_sn = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)),
+               o_g = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)), o_y = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double));
+  const size_t o_rows = carve_bytes(off, (size_t) std::max(n, 1) * sizeof(int));
+  // right preconditioner over the SZA columns (spherical grids; B200RT_KRYLOV_PC=0 switches it off): every column is cut,
+  // from the lowest voxel up, into runs of KRY_MAX_NR / nu radial voxels with all their states (KryWork); runs as equal
+  // as whole voxels allow took as many or more steps (tests/krylov_multiplet_model.py, pc_blocks)
+  const int pc_nr = c->hg.n_rb - 1, pc_nc = c->hg.n_sb - 1;
+  bool pc = !c->hg.pp && pc_nr >= 2 && pc_nc >= 2 && pc_nr * pc_nc == c->hg.n_vox && nu <= KRY_MAX_NR;
+  if (const char *env = getenv("B200RT_KRYLOV_PC")) pc = pc && atoi(env) != 0;
+  if (const char *env = getenv("B200RT_KRYLOV_FUSED")) pc = pc && atoi(env) != 0;     // the per-step launches iterate on A itself
+  int pc_runs = 1, pc_run = 0;
+  if (pc) {
+    const int run_vox = std::min(pc_nr, KRY_MAX_NR / nu);
+    pc_run = nu * run_vox;
+    pc_runs = (pc_nr + run_vox - 1) / run_vox;
+  }
+  const int pc_blocks = pc_nc * pc_runs;
+  const size_t o_usol = carve_bytes(off, (size_t) ns * sizeof(double)), o_wperm = carve_bytes(off, (size_t) ns * sizeof(double));
+  const size_t o_minv = carve_bytes(off, pc ? (size_t) pc_blocks * pc_run * pc_run * sizeof(double) : 16);
+  const bool fresh = work.bytes < off;
+  B200RT_CUDA(c, work.ensure(off));
+  char *base = static_cast<char *>(work.p);
+  if (fresh) {    // the round counter lives with the exchange block's life: it restarts only together with it
+    B200RT_CUDA(c, cudaMemsetAsync(base + o_st, 0, sizeof(KryState), c->stream));
+    if (round_base) {
+      B200RT_CUDA(c, cudaMemcpyAsync(base + o_st, &round_base, sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
+      B200RT_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+  }
+  KryWork &wk = ks.wk;
+  wk.st = reinterpret_cast<KryState *>(base + o_st);
+  wk.V = reinterpret_cast<double *>(base + o_V);
+  wk.wloc = reinterpret_cast<double *>(base + o_w); wk.bvec = reinterpret_cast<double *>(base + o_b);
+  wk.xsol = reinterpret_cast<double *>(base + o_x);
+  wk.part1 = reinterpret_cast<double *>(base + o_p1); wk.part2 = reinterpret_cast<double *>(base + o_p2);
+  wk.npart = reinterpret_cast<double *>(base + o_np);
+  wk.R = reinterpret_cast<double *>(base + o_R);
+  wk.cs = reinterpret_cast<double *>(base + o_cs); wk.sn = reinterpret_cast<double *>(base + o_sn);
+  wk.g = reinterpret_cast<double *>(base + o_g); wk.y = reinterpret_cast<double *>(base + o_y);
+  wk.ns = ns;
+  wk.usol = reinterpret_cast<double *>(base + o_usol);
+  wk.wperm = reinterpret_cast<double *>(base + o_wperm);
+  wk.Minv = reinterpret_cast<double *>(base + o_minv);
+  wk.Bp = nullptr;
+  wk.run = 0; wk.n_col = pc_nc; wk.nu = nu; wk.cl = pc_nr * nu; wk.n_runs = pc_runs;
+  if (pc) {       // (shared by the forward and the adjoint solver: every set-up rewrites each row an iteration reads)
+    B200RT_CUDA(c, c->kry_bp.ensure((size_t) std::max(n_rows, 1) * n * sizeof(double)));
+    wk.Bp = c->kry_bp.as<double>();
+  }
+  ks.d_rows = reinterpret_cast<int *>(base + o_rows);
+  B200RT_CUDA(c, c->host_stage.ensure((size_t) std::max(n, 1) * sizeof(int)));
+  std::memcpy(c->host_stage.p, rows.data(), (size_t) n_rows * sizeof(int));
+  B200RT_CUDA(c, cudaMemcpyAsync(ks.d_rows, c->host_stage.p, (size_t) n_rows * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+  B200RT_CUDA(c, cudaStreamSynchronize(c->stream));
+  for (int q = 0; q < KRY_MAX_WORLD; q++) ks.pe.p[q] = q < world ? static_cast<KryExchange *>(blocks[q]) : nullptr;
+  ks.pe.rank = rank; ks.pe.world = world;
+
+  ks.tol = 1e-13;
+  if (const char *env = getenv("B200RT_KRYLOV_TOL")) ks.tol = atof(env);
+  ks.max_it = KRY_MAX_IT;
+  if (const char *env = getenv("B200RT_KRYLOV_MAXIT")) ks.max_it = std::max(1, std::min(KRY_MAX_IT, atoi(env)));
+  ks.fused = true;
+  if (const char *env = getenv("B200RT_KRYLOV_FUSED")) ks.fused = atoi(env) != 0;
+
+  ks.n = n; ks.n_rows = n_rows; ks.cta_cap = cta_cap;
+  ks.pc = pc; ks.pc_run = pc_run; ks.pc_blocks = pc_blocks;
+  ks.post_blocks = std::max(1, std::min(n_rows, NUM_SMS * 8));   // CTAs pull rows from a queue
+  ks.orth_blocks = (n + KRY_SLICE - 1) / KRY_SLICE;
+  B200RT_CUDA(c, c->host_scratch.ensure((63 + (size_t) std::max(n_final, 1)) * sizeof(KryState)));
+  ks.h_st = c->host_scratch.as<KryState>();
+  static const bool trace = getenv("B200RT_KRYLOV_TRACE") != nullptr;
+  ks.trace = trace;
+  ks.marks.clear();
+  return B200RT_OK;
+}
+
+// everything but the round counter starts from zero (no kernel of this solver is in flight here)
+cudaError_t kry_reset(const KrySolver &ks, cudaStream_t s) {
+  return cudaMemsetAsync(reinterpret_cast<char *>(ks.wk.st) + offsetof(KryState, iter), 0,
+                         sizeof(KryState) - offsetof(KryState, iter), s);
+}
+
+void kry_mark(KrySolver &ks, cudaStream_t s) {
+  cudaEvent_t ev;
+  cudaEventCreate(&ev);
+  cudaEventRecord(ev, s);
+  ks.marks.push_back(ev);
+}
+
+// the preconditioner of the one-launch form: block entries to all ranks, inverses, rows of A M^-1
+int kry_setup(b200rt_ctx *c, KrySolver &ks, const double *K, double branching, int *launches) {
+  if (!(ks.fused && ks.pc)) return B200RT_OK;
+  KryWork &wk = ks.wk;
+  const int n = ks.n, n_rows = ks.n_rows, pc_run = ks.pc_run, pc_blocks = ks.pc_blocks;
+  cudaStream_t s = c->stream;
+  wk.run = pc_run;
+  const size_t sm_inv = (size_t) pc_run * (pc_run + 1) * sizeof(double);
+  const size_t sm_rows = ((size_t) pc_run * pc_run + (size_t) KRY_PRE_RT * pc_run) * sizeof(double);
+  B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_invert, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_inv));
+  B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_rows));
+  B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_permute, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) ((size_t) n * sizeof(double))));
+  if (ks.trace) kry_mark(ks, s);
+  kry_pre_post<<<std::max(1, std::min(n_rows, 4 * NUM_SMS)), 128, 0, s>>>(K, n, ks.d_rows, n_rows, branching, wk, ks.pe);
+  if (ks.trace) kry_mark(ks, s);
+  kry_pre_invert<<<pc_blocks, KRY_THREADS, sm_inv, s>>>(wk, ks.pe);
+  if (ks.trace) kry_mark(ks, s);
+  if (n_rows > 0) {
+    kry_pre_permute<<<std::min(n_rows, 4 * NUM_SMS), KRY_THREADS, (size_t) n * sizeof(double), s>>>(K, n, ks.d_rows, n_rows, branching, wk);
+    kry_pre_rows<<<dim3(pc_blocks, std::max(1, std::min((n_rows + KRY_PRE_RT - 1) / KRY_PRE_RT, 2 * NUM_SMS / pc_blocks))), KRY_THREADS, sm_rows, s>>>(n, n_rows, wk);
+  }
+  if (ks.trace) kry_mark(ks, s);
+  *launches += 4;
+  return B200RT_OK;
+}
+
+// one iteration for the right-hand side S0 into S: the one-launch form, or the per-step launches when the cooperative
+// grid does not fit (or B200RT_KRYLOV_FUSED=0); *fused says which ran
+int kry_iterate(b200rt_ctx *c, KrySolver &ks, const double *K, double branching, const double *S0, double *S,
+                int *launches, bool *fused_out) {
+  KryWork wk = ks.wk;
+  const KryPeers &pe = ks.pe;
+  const int n = ks.n, n_rows = ks.n_rows, orth_blocks = ks.orth_blocks, post_blocks = ks.post_blocks, max_it = ks.max_it;
+  const int *d_rows = ks.d_rows;
+  KryState *h_st = ks.h_st;
+  cudaStream_t s = c->stream;
+  constexpr int CHUNK = 16;
+  bool fused = ks.fused;
+  if (fused) {
+    // x staged in shared memory (n * 8 bytes per CTA) where that leaves room for a grid of orth_blocks CTAs; otherwise
+    // (above ~14k unknowns on a B200) the rows read x through L2 and the CTAs need no dynamic shared memory
+    int cap = ks.cta_cap > 0 ? ks.cta_cap : 3 * NUM_SMS;
+    if (const char *env = getenv("B200RT_KRYLOV_CTAS")) cap = std::max(1, atoi(env));
+    int grid = 0;
+    size_t smem = 0;
+    for (const size_t try_smem : {(size_t) n * sizeof(double), (size_t) 0}) {
+      int per_sm = 0;
+      cudaError_t e_occ = cudaFuncSetAttribute(kry_loop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) try_smem);
+      if (e_occ == cudaSuccess) e_occ = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kry_loop, KRY_THREADS, try_smem);
+      if (e_occ != cudaSuccess) { cudaGetLastError(); continue; }
+      grid = std::min(cap, per_sm * NUM_SMS);
+      smem = try_smem;
+      if (grid >= orth_blocks) break;
+    }
+    if (grid < orth_blocks) {
+      fused = false;                             // (a grid too small to own every slice of the vector: the launches below)
+    } else {
+      KryLoopArgs a;
+      a.K = K; a.rows = d_rows; a.S0 = S0; a.S = S; a.wk = wk; a.pe = pe;
+      a.branching = branching; a.tol = ks.tol; a.n = n; a.n_rows = n_rows; a.max_it = max_it; a.orth_blocks = orth_blocks;
+      a.stage_x = smem > 0;
+      void *kargs[] = {&a};
+      const cudaError_t e_l = cudaLaunchCooperativeKernel((void *) kry_loop, dim3(grid), dim3(KRY_THREADS), kargs, smem, s);
+      if (e_l == cudaSuccess) *launches += 1;
+      else { cudaGetLastError(); fused = false; }
+    }
+  }
+  *fused_out = fused;
+  if (fused) return B200RT_OK;
+  wk.run = 0;                                      // (the launches below iterate on A itself)
+  kry_post<0><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, branching, S0, wk, pe);
+  kry_begin<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe, ks.tol, max_it);
+  *launches += 2;
+  // Arnoldi steps in chunks; the state after chunk k is read back while chunk k + 1 runs, so at most two chunks of
+  // (empty: every kernel returns at once after `done`) launches follow the step that converged
+  const int n_chunks = (max_it + CHUNK - 1) / CHUNK;
+  std::vector<cudaEvent_t> read(n_chunks);
+  bool stop = false;
+  for (int k = 0; k < n_chunks && !stop; k++) {
+    for (int it = 0; it < CHUNK && k * CHUNK + it < max_it; it++) {
+      const bool tr = ks.trace && k * CHUNK + it < 48;
+      if (tr) kry_mark(ks, s);
+      kry_post<1><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, branching, S0, wk, pe);
+      if (tr) kry_mark(ks, s);
+      kry_orth<0><<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
+      if (tr) kry_mark(ks, s);
+      kry_orth<1><<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
+      if (tr) kry_mark(ks, s);
+      kry_orth<2><<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
+      if (tr) kry_mark(ks, s);
+      *launches += 4;
+    }
+    B200RT_CUDA(c, cudaMemcpyAsync(h_st + k, wk.st, sizeof(KryState), cudaMemcpyDeviceToHost, s));
+    read[k] = api::PhaseTimer::take(c);
+    B200RT_CUDA(c, cudaEventRecord(read[k], s));
+    if (k >= 1) {
+      B200RT_CUDA(c, cudaEventSynchronize(read[k - 1]));
+      stop = h_st[k - 1].done != 0;
+    }
+  }
+  kry_backsolve<<<1, 32, 0, s>>>(wk);
+  kry_solution<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, S);
+  kry_post<2><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, branching, S0, wk, pe);
+  kry_residual<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
+  *launches += 4;
+  return B200RT_OK;
+}
+
+// B200RT_KRYLOV_TRACE: what the marks of the last set-up and iteration measured (after the stream has been synchronised)
+void kry_trace_report(KrySolver &ks, bool fused, const KryState &fin) {
+  if (!ks.trace) return;
+  auto &marks = ks.marks;
+  if (fused && marks.size() == 4) {
+    float ms[3];
+    for (int q = 0; q < 3; q++) cudaEventElapsedTime(&ms[q], marks[q], marks[q + 1]);
+    fprintf(stderr, "krylov trace: preconditioner set-up [us]: block entries to all ranks %.1f  inverses %.1f  rows of A M^-1 %.1f\n",
+            ms[0] * 1e3, ms[1] * 1e3, ms[2] * 1e3);
+    for (auto ev : marks) cudaEventDestroy(ev);
+    marks.clear();
+  }
+  if (!marks.empty()) {
+    double sum[4] = {0, 0, 0, 0};
+    const int steps_traced = (int) marks.size() / 5;
+    for (int st_ = 0; st_ < steps_traced; st_++)
+      for (int q = 0; q < 4; q++) {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, marks[st_ * 5 + q], marks[st_ * 5 + q + 1]);
+        sum[q] += ms;
+      }
+    fprintf(stderr, "krylov trace (%d steps, us per step): post %.2f  orth0 %.2f  orth1 %.2f  orth2 %.2f\n", steps_traced,
+            sum[0] / steps_traced * 1e3, sum[1] / steps_traced * 1e3, sum[2] / steps_traced * 1e3, sum[3] / steps_traced * 1e3);
+    for (auto ev : marks) cudaEventDestroy(ev);
+    marks.clear();
+  }
+  if (fused && fin.iter > 0)
+    fprintf(stderr, "krylov trace (one launch, %d steps, CTA 0's clock, us per step): product %.2f  wait for peers %.2f  "
+            "orthogonalisation %.2f (pass / barrier: %.2f / %.2f, %.2f / %.2f, %.2f / %.2f)  closing %.2f\n", fin.iter,
+            fin.t_phase[0] * 1e-3 / fin.iter, fin.t_phase[1] * 1e-3 / fin.iter, fin.t_phase[2] * 1e-3 / fin.iter,
+            fin.t_phase[4] * 1e-3 / fin.iter, fin.t_phase[5] * 1e-3 / fin.iter, fin.t_phase[6] * 1e-3 / fin.iter,
+            fin.t_phase[7] * 1e-3 / fin.iter, fin.t_phase[8] * 1e-3 / fin.iter, fin.t_phase[9] * 1e-3 / fin.iter,
+            fin.t_phase[3] * 1e-3 / fin.iter);
+}
+
+// the outcome of one iteration; `who` names the entry point, `hint` follows a residual that did not converge
+int kry_status(b200rt_ctx *c, const KryState &fin, const std::string &who, const char *hint) {
+  if (fin.error == 3)
+    return fail(c, B200RT_ERR_CUDA, who + ": the resident grid of the solve never became complete (30 s): another resident "
+                                          "grid on this device holds its SMs (B200RT_KRYLOV_CTAS limits the grid; B200RT_KRYLOV_FUSED=0 avoids it)");
+  if (fin.error == 2)
+    return fail(c, B200RT_ERR_STATE, who + ": the rows the ranks built do not add up to the grid (every voxel must be in exactly one rank's influence call)");
+  if (fin.error)
+    return fail(c, B200RT_ERR_CUDA, who + ": a peer never posted its rows (20 s): all ranks must call it, with the same grid");
+  if (!fin.converged)
+    return fail(c, B200RT_ERR_NOT_DOMINANT, who + ": GMRES residual " + std::to_string(fin.res) + " after " +
+                                                std::to_string(fin.iter) + " steps" + hint);
+  if (!(fin.true_res <= 1e-8))
+    return fail(c, B200RT_ERR_NOT_DOMINANT, who + ": residual " + std::to_string(fin.true_res));
+  return B200RT_OK;
 }
 
 }  // namespace
@@ -1303,248 +1616,140 @@ int solve_distributed(b200rt_ctx *c, int rank, int world, void *const *blocks, b
   for (auto &r : c->built_ranges)
     for (int v = r.first; v < r.second; v++)
       for (int s = 0; s < nu; s++) rows.push_back(v * nu + s);
-  const int n_rows = (int) rows.size();
-
-  // work area
-  const int ns = (n + 31) & ~31;
-  size_t off = 0;
-  const size_t o_st = carve_bytes(off, sizeof(KryState));
-  const size_t o_V = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * ns * sizeof(double));
-  const size_t o_w = carve_bytes(off, (size_t) ns * sizeof(double)), o_b = carve_bytes(off, (size_t) ns * sizeof(double)),
-               o_x = carve_bytes(off, (size_t) ns * sizeof(double));
-  const size_t o_p1 = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * KRY_MAX_B * sizeof(double)),
-               o_p2 = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * KRY_MAX_B * sizeof(double));
-  const size_t o_np = carve_bytes(off, KRY_MAX_B * sizeof(double));
-  const size_t o_R = carve_bytes(off, (size_t) (KRY_MAX_IT + 1) * KRY_MAX_IT * sizeof(double));
-  const size_t o_cs = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)), o_sn = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)),
-               o_g = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double)), o_y = carve_bytes(off, (KRY_MAX_IT + 1) * sizeof(double));
-  const size_t o_rows = carve_bytes(off, (size_t) std::max(n, 1) * sizeof(int));
-  // right preconditioner over the SZA columns (spherical grids; B200RT_KRYLOV_PC=0 switches it off): every column is cut,
-  // from the lowest voxel up, into runs of KRY_MAX_NR / nu radial voxels with all their states (KryWork); runs as equal
-  // as whole voxels allow took as many or more steps (tests/krylov_multiplet_model.py, pc_blocks)
-  const int pc_nr = c->hg.n_rb - 1, pc_nc = c->hg.n_sb - 1;
-  bool pc = !c->hg.pp && pc_nr >= 2 && pc_nc >= 2 && pc_nr * pc_nc == c->hg.n_vox && nu <= KRY_MAX_NR;
-  if (const char *env = getenv("B200RT_KRYLOV_PC")) pc = pc && atoi(env) != 0;
-  if (const char *env = getenv("B200RT_KRYLOV_FUSED")) pc = pc && atoi(env) != 0;     // the per-step launches iterate on A itself
-  int pc_runs = 1, pc_run = 0;
-  if (pc) {
-    const int run_vox = std::min(pc_nr, KRY_MAX_NR / nu);
-    pc_run = nu * run_vox;
-    pc_runs = (pc_nr + run_vox - 1) / run_vox;
-  }
-  const int pc_blocks = pc_nc * pc_runs;
-  const size_t o_usol = carve_bytes(off, (size_t) ns * sizeof(double)), o_wperm = carve_bytes(off, (size_t) ns * sizeof(double));
-  const size_t o_minv = carve_bytes(off, pc ? (size_t) pc_blocks * pc_run * pc_run * sizeof(double) : 16);
-  const bool fresh = c->kry_work.bytes < off;
-  B200RT_CUDA(c, c->kry_work.ensure(off));
-  char *base = static_cast<char *>(c->kry_work.p);
-  if (fresh) {    // the round counter lives with the exchange block's life: it restarts only together with it
-    B200RT_CUDA(c, cudaMemsetAsync(base + o_st, 0, sizeof(KryState), c->stream));
-    if (c->kry_round_base) {
-      B200RT_CUDA(c, cudaMemcpyAsync(base + o_st, &c->kry_round_base, sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
-      B200RT_CUDA(c, cudaStreamSynchronize(c->stream));
-    }
-  }
-  KryWork wk;
-  wk.st = reinterpret_cast<KryState *>(base + o_st);
-  wk.V = reinterpret_cast<double *>(base + o_V);
-  wk.wloc = reinterpret_cast<double *>(base + o_w); wk.bvec = reinterpret_cast<double *>(base + o_b);
-  wk.xsol = reinterpret_cast<double *>(base + o_x);
-  wk.part1 = reinterpret_cast<double *>(base + o_p1); wk.part2 = reinterpret_cast<double *>(base + o_p2);
-  wk.npart = reinterpret_cast<double *>(base + o_np);
-  wk.R = reinterpret_cast<double *>(base + o_R);
-  wk.cs = reinterpret_cast<double *>(base + o_cs); wk.sn = reinterpret_cast<double *>(base + o_sn);
-  wk.g = reinterpret_cast<double *>(base + o_g); wk.y = reinterpret_cast<double *>(base + o_y);
-  wk.ns = ns;
-  wk.usol = reinterpret_cast<double *>(base + o_usol);
-  wk.wperm = reinterpret_cast<double *>(base + o_wperm);
-  wk.Minv = reinterpret_cast<double *>(base + o_minv);
-  wk.Bp = nullptr;
-  wk.run = 0; wk.n_col = pc_nc; wk.nu = nu; wk.cl = pc_nr * nu; wk.n_runs = pc_runs;
-  if (pc) {
-    B200RT_CUDA(c, c->kry_bp.ensure((size_t) std::max(n_rows, 1) * n * sizeof(double)));
-    wk.Bp = c->kry_bp.as<double>();
-  }
-  int *d_rows = reinterpret_cast<int *>(base + o_rows);
-  B200RT_CUDA(c, c->host_stage.ensure((size_t) std::max(n, 1) * sizeof(int)));
-  std::memcpy(c->host_stage.p, rows.data(), (size_t) n_rows * sizeof(int));
-  B200RT_CUDA(c, cudaMemcpyAsync(d_rows, c->host_stage.p, (size_t) n_rows * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-  B200RT_CUDA(c, cudaStreamSynchronize(c->stream));
-  KryPeers pe;
-  for (int q = 0; q < KRY_MAX_WORLD; q++) pe.p[q] = q < world ? static_cast<KryExchange *>(blocks[q]) : nullptr;
-  pe.rank = rank; pe.world = world;
-
-  double tol = 1e-13;
-  if (const char *env = getenv("B200RT_KRYLOV_TOL")) tol = atof(env);
-  int max_it = KRY_MAX_IT;
-  if (const char *env = getenv("B200RT_KRYLOV_MAXIT")) max_it = std::max(1, std::min(KRY_MAX_IT, atoi(env)));
-
-  const int post_blocks = std::max(1, std::min(n_rows, NUM_SMS * 8));   // CTAs pull rows from a queue
-  const int orth_blocks = (n + KRY_SLICE - 1) / KRY_SLICE;
-  B200RT_CUDA(c, c->host_scratch.ensure(64 * sizeof(KryState)));
-  KryState *h_st = c->host_scratch.as<KryState>();
+  KrySolver ks;
+  if (int rc = kry_open(c, rows, n, nu, c->kry_work, c->kry_round_base, blocks, rank, world, cta_cap, 1, ks)) return rc;
   cudaStream_t s = c->stream;
-  constexpr int CHUNK = 16;
 
   for (System &E : sys) {
     if (!E.have_K) return fail(c, B200RT_ERR_STATE, "b200rt_solve_distributed: influence rows not built");
     PhaseTimer t(c, PH_SOLVE);
     int launches = 0;
-    const double *K = E.K, *S0 = E.S0;
-    // everything but the round counter starts from zero (no kernel of this context is in flight here)
-    B200RT_CUDA(c, cudaMemsetAsync(reinterpret_cast<char *>(wk.st) + offsetof(KryState, iter), 0,
-                                   sizeof(KryState) - offsetof(KryState, iter), s));
-    // B200RT_KRYLOV_TRACE=1: time the four kernels of the first 48 steps (development aid)
-    static const bool trace = getenv("B200RT_KRYLOV_TRACE") != nullptr;
-    std::vector<cudaEvent_t> marks;
-    auto mark = [&] { cudaEvent_t ev; cudaEventCreate(&ev); cudaEventRecord(ev, s); marks.push_back(ev); };
-    // ---- the one-launch form: the grid stays resident for the whole iteration (cooperative launch, so that it is)
-    bool fused = true;
-    if (const char *env = getenv("B200RT_KRYLOV_FUSED")) fused = atoi(env) != 0;
-    if (fused && pc) {                             // the preconditioner: block entries to all ranks, inverses, rows of A M^-1
-      wk.run = pc_run;
-      const size_t sm_inv = (size_t) pc_run * (pc_run + 1) * sizeof(double);
-      const size_t sm_rows = ((size_t) pc_run * pc_run + (size_t) KRY_PRE_RT * pc_run) * sizeof(double);
-      B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_invert, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_inv));
-      B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) sm_rows));
-      B200RT_CUDA(c, cudaFuncSetAttribute(kry_pre_permute, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) ((size_t) n * sizeof(double))));
-      if (trace) mark();
-      kry_pre_post<<<std::max(1, std::min(n_rows, 4 * NUM_SMS)), 128, 0, s>>>(K, n, d_rows, n_rows, E.branching, wk, pe);
-      if (trace) mark();
-      kry_pre_invert<<<pc_blocks, KRY_THREADS, sm_inv, s>>>(wk, pe);
-      if (trace) mark();
-      if (n_rows > 0) {
-        kry_pre_permute<<<std::min(n_rows, 4 * NUM_SMS), KRY_THREADS, (size_t) n * sizeof(double), s>>>(K, n, d_rows, n_rows, E.branching, wk);
-        kry_pre_rows<<<dim3(pc_blocks, std::max(1, std::min((n_rows + KRY_PRE_RT - 1) / KRY_PRE_RT, 2 * NUM_SMS / pc_blocks))), KRY_THREADS, sm_rows, s>>>(n, n_rows, wk);
-      }
-      if (trace) mark();
-      launches += 4;
-    }
-    if (fused) {
-      // x staged in shared memory (n * 8 bytes per CTA) where that leaves room for a grid of orth_blocks CTAs; otherwise
-      // (above ~14k unknowns on a B200) the rows read x through L2 and the CTAs need no dynamic shared memory
-      int cap = cta_cap > 0 ? cta_cap : 3 * NUM_SMS;
-      if (const char *env = getenv("B200RT_KRYLOV_CTAS")) cap = std::max(1, atoi(env));
-      int grid = 0;
-      size_t smem = 0;
-      for (const size_t try_smem : {(size_t) n * sizeof(double), (size_t) 0}) {
-        int per_sm = 0;
-        cudaError_t e_occ = cudaFuncSetAttribute(kry_loop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) try_smem);
-        if (e_occ == cudaSuccess) e_occ = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kry_loop, KRY_THREADS, try_smem);
-        if (e_occ != cudaSuccess) { cudaGetLastError(); continue; }
-        grid = std::min(cap, per_sm * NUM_SMS);
-        smem = try_smem;
-        if (grid >= orth_blocks) break;
-      }
-      if (grid < orth_blocks) {
-        fused = false;                             // (a grid too small to own every slice of the vector: the launches below)
-      } else {
-        KryLoopArgs a;
-        a.K = K; a.rows = d_rows; a.S0 = S0; a.S = E.S; a.wk = wk; a.pe = pe;
-        a.branching = E.branching; a.tol = tol; a.n = n; a.n_rows = n_rows; a.max_it = max_it; a.orth_blocks = orth_blocks;
-        a.stage_x = smem > 0;
-        void *kargs[] = {&a};
-        const cudaError_t e_l = cudaLaunchCooperativeKernel((void *) kry_loop, dim3(grid), dim3(KRY_THREADS), kargs, smem, s);
-        if (e_l == cudaSuccess) launches += 1;
-        else { cudaGetLastError(); fused = false; }
-      }
-    }
-    if (!fused) wk.run = 0;                         // (the launches below iterate on A itself)
-    if (!fused) {
-    kry_post<0><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, E.branching, S0, wk, pe);
-    kry_begin<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe, tol, max_it);
-    launches += 2;
-    // Arnoldi steps in chunks; the state after chunk k is read back while chunk k + 1 runs, so at most two chunks of
-    // (empty: every kernel returns at once after `done`) launches follow the step that converged
-    const int n_chunks = (max_it + CHUNK - 1) / CHUNK;
-    std::vector<cudaEvent_t> read(n_chunks);
-    int issued = 0;
-    bool stop = false;
-    for (int k = 0; k < n_chunks && !stop; k++) {
-      for (int it = 0; it < CHUNK && k * CHUNK + it < max_it; it++) {
-        const bool tr = trace && k * CHUNK + it < 48;
-        if (tr) mark();
-        kry_post<1><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, E.branching, S0, wk, pe);
-        if (tr) mark();
-        kry_orth<0><<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
-        if (tr) mark();
-        kry_orth<1><<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
-        if (tr) mark();
-        kry_orth<2><<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
-        if (tr) mark();
-        launches += 4;
-      }
-      B200RT_CUDA(c, cudaMemcpyAsync(h_st + k, wk.st, sizeof(KryState), cudaMemcpyDeviceToHost, s));
-      read[k] = PhaseTimer::take(c);
-      B200RT_CUDA(c, cudaEventRecord(read[k], s));
-      issued = k + 1;
-      if (k >= 1) {
-        B200RT_CUDA(c, cudaEventSynchronize(read[k - 1]));
-        stop = h_st[k - 1].done != 0;
-      }
-    }
-    (void) issued;
-    kry_backsolve<<<1, 32, 0, s>>>(wk);
-    kry_solution<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, E.S);
-    kry_post<2><<<post_blocks, KRY_THREADS, 0, s>>>(K, n, d_rows, n_rows, E.branching, S0, wk, pe);
-    kry_residual<<<orth_blocks, KRY_THREADS, 0, s>>>(n, wk, pe);
-    launches += 4;
-    }   // !fused
+    B200RT_CUDA(c, kry_reset(ks, s));
+    if (int rc = kry_setup(c, ks, E.K, E.branching, &launches)) return rc;
+    bool fused = false;
+    if (int rc = kry_iterate(c, ks, E.K, E.branching, E.S0, E.S, &launches, &fused)) return rc;
     B200RT_CUDA(c, cudaGetLastError());
     if (c->precision == B200RT_F64)
       B200RT_CUDA(c, launch_convert<double>(E.S, static_cast<double *>(E.S_real), n, s));
     else
       B200RT_CUDA(c, launch_convert<float>(E.S, static_cast<float *>(E.S_real), n, s));
     t.stop(launches);
-    B200RT_CUDA(c, cudaMemcpyAsync(h_st + 63, wk.st, sizeof(KryState), cudaMemcpyDeviceToHost, s));
+    B200RT_CUDA(c, cudaMemcpyAsync(ks.h_st + 63, ks.wk.st, sizeof(KryState), cudaMemcpyDeviceToHost, s));
     B200RT_CUDA(c, cudaStreamSynchronize(s));
-    if (trace && fused && marks.size() == 4) {
-      float ms[3];
-      for (int q = 0; q < 3; q++) cudaEventElapsedTime(&ms[q], marks[q], marks[q + 1]);
-      fprintf(stderr, "krylov trace: preconditioner set-up [us]: block entries to all ranks %.1f  inverses %.1f  rows of A M^-1 %.1f\n",
-              ms[0] * 1e3, ms[1] * 1e3, ms[2] * 1e3);
-      for (auto ev : marks) cudaEventDestroy(ev);
-      marks.clear();
-    }
-    if (trace && !marks.empty()) {
-      double sum[4] = {0, 0, 0, 0};
-      const int steps_traced = (int) marks.size() / 5;
-      for (int st_ = 0; st_ < steps_traced; st_++)
-        for (int q = 0; q < 4; q++) {
-          float ms = 0;
-          cudaEventElapsedTime(&ms, marks[st_ * 5 + q], marks[st_ * 5 + q + 1]);
-          sum[q] += ms;
-        }
-      fprintf(stderr, "krylov trace (%d steps, us per step): post %.2f  orth0 %.2f  orth1 %.2f  orth2 %.2f\n", steps_traced,
-              sum[0] / steps_traced * 1e3, sum[1] / steps_traced * 1e3, sum[2] / steps_traced * 1e3, sum[3] / steps_traced * 1e3);
-      for (auto ev : marks) cudaEventDestroy(ev);
-    }
-    const KryState fin = h_st[63];
-    if (trace && fused && fin.iter > 0)
-      fprintf(stderr, "krylov trace (one launch, %d steps, CTA 0's clock, us per step): product %.2f  wait for peers %.2f  "
-              "orthogonalisation %.2f (pass / barrier: %.2f / %.2f, %.2f / %.2f, %.2f / %.2f)  closing %.2f\n", fin.iter,
-              fin.t_phase[0] * 1e-3 / fin.iter, fin.t_phase[1] * 1e-3 / fin.iter, fin.t_phase[2] * 1e-3 / fin.iter,
-              fin.t_phase[4] * 1e-3 / fin.iter, fin.t_phase[5] * 1e-3 / fin.iter, fin.t_phase[6] * 1e-3 / fin.iter,
-              fin.t_phase[7] * 1e-3 / fin.iter, fin.t_phase[8] * 1e-3 / fin.iter, fin.t_phase[9] * 1e-3 / fin.iter,
-              fin.t_phase[3] * 1e-3 / fin.iter);
+    const KryState fin = ks.h_st[63];
+    kry_trace_report(ks, fused, fin);
     c->kry_round_base = fin.round;
     c->kry_last_iters = fin.iter;
-    if (fin.error == 3)
-      return fail(c, B200RT_ERR_CUDA, "b200rt_solve_distributed: the resident grid of the solve never became complete (30 s): another resident "
-                                      "grid on this device holds its SMs (B200RT_KRYLOV_CTAS limits the grid; B200RT_KRYLOV_FUSED=0 avoids it)");
-    if (fin.error == 2)
-      return fail(c, B200RT_ERR_STATE, "b200rt_solve_distributed: the rows the ranks built do not add up to the grid (every voxel must be in exactly one rank's influence call)");
-    if (fin.error)
-      return fail(c, B200RT_ERR_CUDA, "b200rt_solve_distributed: a peer never posted its rows (20 s): all ranks must call it, with the same grid");
-    if (!fin.converged)
-      return fail(c, B200RT_ERR_NOT_DOMINANT, "b200rt_solve_distributed: GMRES residual " + std::to_string(fin.res) + " after " +
-                                                  std::to_string(fin.iter) + " steps (rows missing on some rank, or a matrix the LU path should take)");
-    if (!(fin.true_res <= 1e-8))
-      return fail(c, B200RT_ERR_NOT_DOMINANT, "b200rt_solve_distributed: residual " + std::to_string(fin.true_res));
+    if (int rc = kry_status(c, fin, "b200rt_solve_distributed", " (rows missing on some rank, or a matrix the LU path should take)"))
+      return rc;
     *E.residual = fin.true_res;
     *E.have_S = true;
     *E.rec_dirty = true;
   }
+  PhaseTimer::collect(c);
+  return B200RT_OK;
+}
+
+int solve_adjoint(b200rt_ctx *c, int e, int n_rhs, const double *rhs, double *lambda, int *n_steps, double *residual,
+                  bool rows_complete) {
+  const bool mm = c->mult.defined;
+  if (mm ? e != 0 : (e < 0 || e >= c->n_em)) return fail(c, B200RT_ERR_ARG, "b200rt_solve_adjoint: bad emission index");
+  if (n_rhs < 1 || !rhs || !lambda) return fail(c, B200RT_ERR_ARG, "b200rt_solve_adjoint: n_rhs < 1, or rhs / lambda NULL");
+  const int nu = mm ? c->mult.d.n_upper : 1;
+  const int n = c->hg.n_vox * nu;
+  if (n > KRY_MAX_N)
+    return fail(c, B200RT_ERR_CAPACITY, "b200rt_solve_adjoint: more than " + std::to_string(KRY_MAX_N) + " unknowns");
+  if (!(mm ? c->mult.have_K : c->em[e].have_K)) return fail(c, B200RT_ERR_STATE, "b200rt_solve_adjoint: influence matrix not built");
+  if (!rows_complete) {
+    long long own = 0;
+    for (auto &r : c->built_ranges) own += r.second - r.first;
+    if (own != c->hg.n_vox)
+      return fail(c, B200RT_ERR_STATE, "b200rt_solve_adjoint: this context did not build every row of K (a rank of a "
+                                       "distributed job, or the solving rank of row sinks)");
+  }
+  const double *K = mm ? c->mult.K.as<double>() : c->em[e].K.as<double>();
+  const double branching = mm ? 1.0 : c->em[e].branching;
+  PhaseTimer::reset(c);
+  // W^T w is zero when every weighted line of sight misses the grid: lambda = 0 without iterating
+  std::vector<char> zero(n_rhs, 1);
+  bool any = false;
+  for (int k = 0; k < n_rhs; k++) {
+    const double *r = rhs + (size_t) k * n;
+    for (int i = 0; i < n && zero[k]; i++) zero[k] = r[i] == 0.0;
+    any = any || !zero[k];
+  }
+  if (!any) {
+    std::memset(lambda, 0, (size_t) n_rhs * n * sizeof(double));
+    for (int k = 0; k < n_rhs; k++) {
+      if (n_steps) n_steps[k] = 0;
+      if (residual) residual[k] = 0.0;
+    }
+    return B200RT_OK;
+  }
+
+  std::unique_lock<std::mutex> turn(g_single_rank_solve[c->device & 63]);
+  // its own exchange block and work area: the forward solve's round counters, which every rank of a distributed solve
+  // must agree on, never see the adjoint's rounds
+  if (!c->kry_adj_xchg.p) {
+    B200RT_CUDA(c, c->kry_adj_xchg.ensure(sizeof(KryExchange)));
+    B200RT_CUDA(c, cudaMemsetAsync(c->kry_adj_xchg.p, 0, sizeof(KryExchange), c->stream));
+  }
+  void *block = c->kry_adj_xchg.p;
+  std::vector<int> rows(n);
+  for (int i = 0; i < n; i++) rows[i] = i;
+  KrySolver ks;
+  if (int rc = kry_open(c, rows, n, nu, c->kry_adj_work, c->kry_adj_round_base, &block, 0, 1, 0, n_rhs, ks)) return rc;
+  ks.trace = false;
+  cudaStream_t s = c->stream;
+  const size_t nb = (size_t) n_rhs * n * sizeof(double);
+  B200RT_CUDA(c, c->kry_kt.ensure((size_t) n * n * sizeof(double)));
+  B200RT_CUDA(c, c->kry_adj_io.ensure(2 * nb));
+  double *d_rhs = c->kry_adj_io.as<double>(), *d_lam = d_rhs + (size_t) n_rhs * n;
+  B200RT_CUDA(c, c->host_stage.ensure(nb));
+  std::memcpy(c->host_stage.p, rhs, nb);
+  B200RT_CUDA(c, cudaMemcpyAsync(d_rhs, c->host_stage.p, nb, cudaMemcpyHostToDevice, s));
+
+  // K^T on every call: K can change under the context without its knowledge (row sinks, b200rt_influence_dev)
+  {
+    PhaseTimer t(c, PH_TRANSPOSE);
+    const int tiles = (n + KT_TILE - 1) / KT_TILE;
+    kry_transpose<<<dim3(tiles, tiles), dim3(KT_TILE, KT_ROWS), 0, s>>>(K, n, c->kry_kt.as<double>());
+    B200RT_CUDA(c, cudaGetLastError());
+    t.stop(1);
+  }
+  const double *Kt = c->kry_kt.as<double>();
+  PhaseTimer t(c, PH_SOLVE);
+  int launches = 0, last = -1;
+  for (int k = 0; k < n_rhs; k++) {
+    if (zero[k]) {
+      B200RT_CUDA(c, cudaMemsetAsync(d_lam + (size_t) k * n, 0, (size_t) n * sizeof(double), s));
+      continue;
+    }
+    B200RT_CUDA(c, kry_reset(ks, s));
+    if (last < 0)
+      if (int rc = kry_setup(c, ks, Kt, branching, &launches)) return rc;
+    bool fused = false;
+    if (int rc = kry_iterate(c, ks, Kt, branching, d_rhs + (size_t) k * n, d_lam + (size_t) k * n, &launches, &fused)) return rc;
+    B200RT_CUDA(c, cudaMemcpyAsync(ks.h_st + 63 + k, ks.wk.st, sizeof(KryState), cudaMemcpyDeviceToHost, s));
+    last = k;
+  }
+  B200RT_CUDA(c, cudaGetLastError());
+  t.stop(launches);
+  B200RT_CUDA(c, cudaMemcpyAsync(c->host_stage.p, d_lam, nb, cudaMemcpyDeviceToHost, s));
+  B200RT_CUDA(c, cudaStreamSynchronize(s));
+  c->kry_adj_round_base = ks.h_st[63 + last].round;
+  for (int k = 0; k < n_rhs; k++) {
+    if (zero[k]) {
+      if (n_steps) n_steps[k] = 0;
+      if (residual) residual[k] = 0.0;
+      continue;
+    }
+    const KryState &fin = ks.h_st[63 + k];
+    if (int rc = kry_status(c, fin, "b200rt_solve_adjoint (right-hand side " + std::to_string(k) + ")", "")) return rc;
+    if (n_steps) n_steps[k] = fin.iter;
+    if (residual) residual[k] = fin.true_res;
+  }
+  std::memcpy(lambda, c->host_stage.p, nb);
   PhaseTimer::collect(c);
   return B200RT_OK;
 }

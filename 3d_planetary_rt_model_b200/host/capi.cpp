@@ -249,6 +249,13 @@ int obsfit_brightness_weights_get(void *h, long long *indptr, int *indices, doub
     g_weights.erase(it);
   });
 }
+// observation_fit::brightness_source_sensitivity: w[n_obs] -> out[n_vox] = d(sum_l w_l brightness_l) / dS0
+int obsfit_brightness_source_sensitivity(void *h, int e, int which, int n_obs, const double *w, double *out) {
+  return guard([&] {
+    auto s = static_cast<observation_fit *>(h)->brightness_source_sensitivity(e, std::vector<double>(w, w + n_obs), which);
+    std::memcpy(out, s.data(), s.size() * sizeof(double));
+  });
+}
 // out[n_sets][2][n_obs]
 int obsfit_brightness_batch(void *h, int n_sets, const double *nH, const double *T, int contexts_per_gpu, int n_gpus,
                             double *out, double *seconds) {

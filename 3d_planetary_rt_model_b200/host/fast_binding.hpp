@@ -65,4 +65,12 @@ inline void weights_copy(const observation_fit::csr_matrix *w, long long *indptr
 }
 inline void weights_free(observation_fit::csr_matrix *w) { delete w; }
 
+// observation_fit::brightness_source_sensitivity into a vector the caller keeps (new) and frees (vector_free)
+inline std::vector<double> *source_sensitivity(observation_fit *o, int e, const double *w, int n, int which) {
+  return new std::vector<double>(o->brightness_source_sensitivity(e, std::vector<double>(w, w + n), which));
+}
+inline int vector_size(const std::vector<double> *v) { return (int) v->size(); }
+inline void vector_copy(const std::vector<double> *v, double *out) { std::memcpy(out, v->data(), v->size() * sizeof(double)); }
+inline void vector_free(std::vector<double> *v) { delete v; }
+
 }  // namespace b200_fast

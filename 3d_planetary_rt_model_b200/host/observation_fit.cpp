@@ -441,6 +441,32 @@ observation_fit::csr_matrix observation_fit::brightness_weights(int e, int which
   return r;
 }
 
+vector<observation_fit::Real> observation_fit::brightness_source_sensitivity(int e, const vector<Real> &obs_weights,
+                                                                           int which) {
+  if (which == 2 || which == 3)
+    throw std::invalid_argument("brightness_source_sensitivity: the plane-parallel grid has no brightness (grid_plane_parallel.hpp:304-311)");
+  if (which != 0 && which != 1) throw std::invalid_argument("brightness_source_sensitivity: model must be 0 (H) or 1 (D)");
+  if (e < 0 || e >= n_hydrogen_emissions) throw std::invalid_argument("brightness_source_sensitivity: bad emission index");
+  singlet_model &m = singlet(which);
+  if (!m.have_S) throw std::runtime_error("observation_fit: generate a source function before asking for its sensitivity");
+  if (n_obs() == 0) throw std::runtime_error("there must be at least one observation to simulate");
+  if ((int) obs_weights.size() != n_obs())
+    throw std::invalid_argument("brightness_source_sensitivity: one weight per observation (" + std::to_string(n_obs()) + ")");
+  b200rt_ctx *c = m.ctx;
+  if (!m.los_uploaded) {
+    check(b200rt_los_upload(c, n_obs(), los[0].data(), los[1].data(), los[2].data(), los[3].data(), los[4].data(),
+                            los[5].data(), los[6].data(), los[7].data(), los[8].data()), c);
+    m.los_uploaded = true;
+  }
+  // W with brightness()'s n_subsamples, r = W^T w, then lambda = (I - w K)^-T r on the resident K: r . S = lambda . S0
+  check(b200rt_los_weights(c, 10, nullptr), c);
+  const vector<double> w(obs_weights.begin(), obs_weights.end());
+  vector<double> r((size_t) m.in.n_vox), lambda((size_t) m.in.n_vox);
+  check(b200rt_los_weights_apply(c, e, 1, w.data(), r.data()), c);
+  check(b200rt_solve_adjoint(c, e, 1, r.data(), lambda.data(), nullptr, nullptr), c);
+  return vector<Real>(lambda.begin(), lambda.end());
+}
+
 // deuterium_RT / deuterium_obs (observation_fit.cpp:591-637)
 vector<vector<observation_fit::Real>> observation_fit::D_brightness() {
   singlet_model &m = singlet(1);

@@ -157,6 +157,11 @@ public:
     std::vector<Real> data;          // [nnz]
   };
   csr_matrix brightness_weights(int i_emission, int which = 0);
+  // d(sum_l obs_weights[l] * brightness()[i_emission][l]) / dS0 over the voxels of the H (0) or D (1) model: W^T w,
+  // then one adjoint solve on the model's influence matrix, (I - w K)^T lambda = W^T w, so that the weighted brightness
+  // changes by lambda . dS0 for a change dS0 of the single-scattering source.  The IPH term does not depend on S0.
+  // obs_weights has one entry per observation; the plane-parallel models (2, 3) throw.
+  std::vector<Real> brightness_source_sensitivity(int i_emission, const std::vector<Real> &obs_weights, int which = 0);
 
 private:
   struct set_inputs;       // grid + the eight tables of each emission for one parameter set

@@ -29,6 +29,12 @@ cdef extern from "fast_binding.hpp" namespace "b200_fast" nogil:
     int b200_weights_cols "b200_fast::weights_cols"(const b200_csr *w)
     void b200_weights_copy "b200_fast::weights_copy"(const b200_csr *w, long long *indptr, int *indices, double *data)
     void b200_weights_free "b200_fast::weights_free"(b200_csr *w)
+    cppclass b200_dvec "std::vector<double>":
+        pass
+    b200_dvec *b200_source_sensitivity "b200_fast::source_sensitivity"(observation_fit *o, int e, const double *w, int n, int which) except +
+    int b200_vector_size "b200_fast::vector_size"(const b200_dvec *v)
+    void b200_vector_copy "b200_fast::vector_copy"(const b200_dvec *v, double *out)
+    void b200_vector_free "b200_fast::vector_free"(b200_dvec *v)
 
 
 cdef class Pyobservation_fit_b200(Pyobservation_fit):
@@ -129,3 +135,19 @@ cdef class Pyobservation_fit_b200(Pyobservation_fit):
         b200_weights_copy(w, &P[0], &I[0], &D[0])
         b200_weights_free(w)
         return indptr, indices[:nnz], data[:nnz]
+
+    def brightness_source_sensitivity(self, int i_emission, obs_weights, int which=0):
+        """d(sum_l obs_weights[l] * brightness_l) / dS0 over the voxels of the H (which = 0) or D (1) model: one
+        adjoint solve on the model's influence matrix (the IPH term does not depend on S0)"""
+        cdef double[::1] W = np.ascontiguousarray(obs_weights, dtype=np.float64)
+        cdef int n = W.shape[0]
+        cdef const double *wp = &W[0] if n > 0 else NULL
+        cdef b200_dvec *v
+        with nogil:
+            v = b200_source_sensitivity(self.thisptr, i_emission, wp, n, which)
+        out = np.empty(max(b200_vector_size(v), 1), dtype=np.float64)
+        cdef double[::1] O = out
+        b200_vector_copy(v, &O[0])
+        cdef int m = b200_vector_size(v)
+        b200_vector_free(v)
+        return out[:m]

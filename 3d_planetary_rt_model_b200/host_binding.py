@@ -56,6 +56,7 @@ SIGNATURES = {
     "obsfit_brightness_weights": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(C.c_longlong), C.POINTER(C.c_int),
                                             C.POINTER(C.c_int)]),
     "obsfit_brightness_weights_get": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "obsfit_brightness_source_sensitivity": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _dp, _dp]),
 }
 MODEL_H, MODEL_D, MODEL_H_PP, MODEL_D_PP = 0, 1, 2, 3
 _lib = None
@@ -286,6 +287,14 @@ class Pyobservation_fit:
         self._ck(self.lib.obsfit_brightness_weights_get(self.h, indptr.ctypes.data_as(_vp), indices.ctypes.data_as(_vp),
                                                         data.ctypes.data_as(_vp)))
         return indptr, indices[:nnz.value], data[:nnz.value], (nr.value, nc.value)
+
+    def brightness_source_sensitivity(self, e, obs_weights, which=MODEL_H):
+        """d(sum_l obs_weights[l] * brightness()[e][l]) / dS0 over the voxels of model `which` (H or D): one adjoint
+        solve on the model's influence matrix"""
+        w = np.ascontiguousarray(obs_weights, dtype=np.float64)
+        out = np.zeros(self.n_vox)
+        self._ck(self.lib.obsfit_brightness_source_sensitivity(self.h, e, which, len(w), w, out))
+        return out
 
     def radial_boundaries(self, which=MODEL_H):
         out = np.zeros(self.n_rb)

@@ -274,6 +274,30 @@ int b200rt_solve_exchange(b200rt_ctx *ctx, void **block_dev, void *ipc_handle64)
 int b200rt_solve_distributed(b200rt_ctx *ctx, int rank, int world, void *const *blocks);
 int b200rt_last_solve_steps(b200rt_ctx *ctx, int *n_steps);   /* GMRES steps of the last distributed solve */
 
+/* ---- adjoint solve ------------------------------------------------------------------
+ * The source function solves (I - w K) S = S0, S0 the single-scattering source (the solar photons first scattered in
+ * each voxel).  For any r, r . S = lambda . S0 with lambda = (I - w K)^-T r: one adjoint solve gives the sensitivity of
+ * r . S to every voxel's S0 at once.  With r = W_e^T w from b200rt_los_weights_apply(..., transpose = 1, ...),
+ * lambda = d(sum_l w_l brightness_e,l) / dS0_e: where the photons seen along the weighted lines of sight were first
+ * scattered (a multiple-scattering contribution function for w = e_l), or the gradient of a chi^2 through S0.  The
+ * sensitivity to K itself follows in closed form: d(r . S) / dK_ij = w lambda_i S_j (not computed here).
+ *   lambda[k] = (I - w K)^-T rhs[k] for k < n_rhs (singlet emission i_emission; a multiplet: (I - K)^-T over the n_el
+ *   element unknowns e = voxel * n_upper + state, i_emission = 0).  rhs, lambda: [n_rhs][n] doubles; n_steps, residual:
+ *   [n_rhs] (may be NULL) = GMRES steps and true relative residual |rhs - A^T lambda| / |rhs| of each.
+ * FP64 in both precisions (K is FP64).  The preconditioned GMRES of b200rt_solve_distributed (one rank) runs on K^T,
+ * which is rebuilt from the resident K on every call (b200rt_last_kernel_ms phase 9); phase 2 counts the
+ * preconditioner set-up, done once per call, and the iterations.  B200RT_KRYLOV_TOL / _MAXIT / _PC / _FUSED / _CTAS
+ * apply as in the forward solve.  A zero right-hand side gives lambda = 0 with 0 steps.  The forward state -- S,
+ * b200rt_last_residual, b200rt_last_solve_steps, the exchange block's round counters -- is left as it was (the adjoint
+ * has its own exchange block and work area).  A device group runs it on the member that holds every row of K (rows
+ * of a distributed build are gathered there first).
+ * Refused: B200RT_ERR_ARG a bad emission index, n_rhs < 1, rhs or lambda NULL; B200RT_ERR_CAPACITY
+ * n > B200RT_KRYLOV_MAX_N; B200RT_ERR_STATE K not built, or not built for every voxel by this context (a rank of a
+ * one-process-per-GPU distributed job, the rank 0 of the IPC row-sink form); B200RT_ERR_NOT_DOMINANT no convergence
+ * within B200RT_KRYLOV_MAXIT steps (the residual is in the message). */
+int b200rt_solve_adjoint(b200rt_ctx *ctx, int i_emission, int n_rhs, const double *rhs, double *lambda,
+                         int *n_steps, double *residual);
+
 /* ---- observations ---------------------------------------------------------------
  * host helper: observation::add_MSO_observation (observation.hpp:46-65) + atmo_point::xyz +
  * atmo_vector::ptxyz (atmo_vec.cpp:51-61,256-290): MSO position / look direction ->
@@ -378,7 +402,8 @@ int b200rt_traverse_los(b200rt_ctx *ctx, long long capacity,
  * device time (CUDA events on the ctx stream) of the kernels of the last call:
  * phase 0 = traversal, 1 = influence march, 2 = solve, 3 = brightness march (the march launches alone),
  * 4 = IPH, 5 = the longest-first ordering kernels of the lines of sight (3 launches per batch),
- * 6 / 7 / 8 = line-of-sight weights: structure passes (count, scan, fill), value pass, products (b200rt_los_weights*) */
+ * 6 / 7 / 8 = line-of-sight weights: structure passes (count, scan, fill), value pass, products (b200rt_los_weights*),
+ * 9 = the transposition of K of b200rt_solve_adjoint */
 int b200rt_last_kernel_ms(b200rt_ctx *ctx, int phase, float *ms, int *n_launches);
 int b200rt_synchronize(b200rt_ctx *ctx);
 /* measured FP64 peaks of this device (TFLOP/s): plain DFMA and DMMA.8x8x4 (mma.sync m8n8k4.f64).
