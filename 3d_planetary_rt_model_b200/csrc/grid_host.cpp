@@ -64,8 +64,9 @@ constexpr double MIRROR_COS_TOL = 0x1p-49;   // 1.8e-15
 //     ~4e-8 relative per contribution on the 100x60 grid.  In float, line_z rounds differently often enough that the
 //     lists of a near pair drift apart (segment lengths up to 100 % on that grid), so float folds bit-equal pairs only.
 // The lower index represents the pair; every other ray, and every ray of a set without mirror symmetry, stays single.
+// near_pairs = false folds bit-equal pairs only (upload_grid: grids with an SZA boundary at 90 degrees).
 template <class Real>
-int fold_pairs(const RayTables<Real> &rt, int *rep) {
+int fold_pairs(const RayTables<Real> &rt, int *rep, bool near_pairs = true) {
   const int n = (int) rt.cost.size();
   for (int k = 0; k < n; k++) rep[k] = k;
   int marched = 0;
@@ -77,7 +78,7 @@ int fold_pairs(const RayTables<Real> &rt, int *rep) {
           !same_bits(rt.dom[k], rt.dom[q]))
         continue;
       const bool exact = same_bits(rt.cp[k], rt.cp[q]);
-      const bool mirror = sizeof(Real) == sizeof(double) && rt.lower[k] != rt.lower[q] &&
+      const bool mirror = near_pairs && sizeof(Real) == sizeof(double) && rt.lower[k] != rt.lower[q] &&
                           std::fabs(rt.cp[k] - rt.cp[q]) <= MIRROR_COS_TOL;
       if (exact || mirror) { rep[q] = k; break; }
     }
@@ -174,8 +175,14 @@ int upload_grid(b200rt_ctx *c) {
 
   // march view: the representative rays of the mirror-pair fold (fold_pairs) in ascending order, domega * multiplicity
   // (doubling is exact).  The first ray of a polar-angle class is always a representative, so every class keeps one.
+  // An SZA boundary at 90 degrees (every odd n_sb) is the cone cos = 0 to rounding, i.e. the plane z = 0: whether a ray
+  // close to that plane crosses it turns on the last bits of the ray's direction.  The two rays of a near pair then cross
+  // different voxels beside the plane (128x131 grid: thousands of pairs, with segments of up to 37 % of the path in the
+  // other SZA voxel), so such grids fold bit-equal pairs only and march each ray as the reference does.
+  bool plane_cone = false;
+  for (int k = 0; k < n_sb - 2; k++) plane_cone = plane_cone || std::fabs((double) ccos[k]) < 1e-6;
   std::vector<int> rep(n_rays);
-  const int n_fold = fold_pairs<Real>(rt, rep.data());
+  const int n_fold = fold_pairs<Real>(rt, rep.data(), !plane_cone);
   std::vector<Real> fcost, fsint, fdom;
   std::vector<double> fcp;
   std::vector<int> fcls, fmult, fpos(n_rays, -1), fcls_ray(n_cls);

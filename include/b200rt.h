@@ -114,7 +114,8 @@ int b200rt_make_grid_pp(int precision, int n_rb, int n_theta, const double *radi
  * azimuthally symmetric grid the voxel-origin rays at phi and 2 pi - phi cross the same voxels over the same lengths, so
  * b200rt_influence* marches such a pair once and adds its contribution with twice the ray's domega.  Rays pair when
  * their uploaded cos/sin(theta), cos(phi) and domega are bit-equal, or (F64 only) when cos/sin(theta) and domega are
- * bit-equal, cos(phi) agrees to 1.8e-15 and sin(phi) has the opposite sign.  rep[n_rays]: the ray whose march stands for
+ * bit-equal, cos(phi) agrees to 1.8e-15 and sin(phi) has the opposite sign.  A grid with an SZA boundary at 90 degrees
+ * (odd n_sb) folds bit-equal pairs only: there the near pairs cross different voxels.  rep[n_rays]: the ray whose march stands for
  * ray k (k itself for a marched ray; a pair is represented by its lower index); n_marched: rays marched per voxel. */
 int b200rt_fold_rays(int precision, int n_rays, const double *ray_theta, const double *ray_phi,
                      const double *ray_domega, int *rep, int *n_marched);

@@ -41,8 +41,8 @@ def mixed_los(synth, scn, n, seed=11):
     return np.concatenate([locs, miss_locs, in_locs]), np.concatenate([dirs, miss_dirs, in_dirs])
 
 
-def model(synth, binding, shape, prec, **kw):
-    scn = synth.make_scenario(*shape, n_em=2, sza_T_contrast=0.1)
+def model(synth, binding, shape, prec, n_em=2, **kw):
+    scn = synth.make_scenario(*shape, n_em=n_em, sza_T_contrast=0.1)
     return scn, binding.GpuModel(scn, prec, **kw)
 
 
@@ -55,45 +55,51 @@ def csr(W, e, n_vox):
     return sp.csr_matrix((data[e], indices, indptr), shape=(len(indptr) - 1, n_vox))
 
 
-@pytest.mark.parametrize("prec", ["f64", "f32"])
+# one emission runs lw_value_kernel<Real, 1>, two run lw_value_kernel<Real, 2> (los_weights.cu, launch_lw_values)
+PREC_EM = pytest.mark.parametrize("prec,n_em", [("f64", 2), ("f32", 2), ("f64", 1), ("f32", 1)],
+                                  ids=["f64", "f32", "f64-one_emission", "f32-one_emission"])
+
+
+@PREC_EM
 @pytest.mark.parametrize("nsub", [10, 4, 0])
 @pytest.mark.parametrize("shape", [(8, 6, 4, 4), (12, 8, 5, 6), (20, 12, 6, 8)])
-def test_linear_in_S_matches_device_brightness(synth, binding, shape, prec, nsub):
-    scn, G = model(synth, binding, shape, prec)
+def test_linear_in_S_matches_device_brightness(synth, binding, shape, prec, n_em, nsub):
+    scn, G = model(synth, binding, shape, prec, n_em)
     locs, dirs = mixed_los(synth, scn, 2000)
     W = G.los_weights(locs, dirs, nsub)        # before any solve or source function
-    for e in range(2):
+    assert W[2].shape[0] == n_em
+    for e in range(n_em):
         G.set_sourcefn(e, random_S(G.n_vox, e))
     _, b = G.brightness(locs, dirs, nsub)
     assert (b[:, 2] == -1).any()               # planet hits are in the set
     tol = 1e-12 if prec == "f64" else 1e-4
-    for e in range(2):
+    for e in range(n_em):
         WS = csr(W, e, G.n_vox) @ random_S(G.n_vox, e)
         ref = b[e, 0]
         assert np.abs(ref).max() > 0
         assert np.abs(WS - ref).max() / np.abs(ref).max() < tol, (e, np.abs(WS - ref).max() / np.abs(ref).max())
 
 
-@pytest.mark.parametrize("prec", ["f64", "f32"])
-def test_entries_match_oracle(synth, binding, oraclebind, prec):
-    scn, G = model(synth, binding, (12, 8, 5, 6), prec)
+@PREC_EM
+def test_entries_match_oracle(synth, binding, oraclebind, prec, n_em):
+    scn, G = model(synth, binding, (12, 8, 5, 6), prec, n_em)
     locs, dirs = mixed_los(synth, scn, 100, seed=3)
     indptr, indices, data = G.los_weights(locs, dirs, 10)
     O = oraclebind.OracleModel(scn, prec)
     O.build_rows()
     O.solve()
     n, nv = len(locs), G.n_vox
-    dense_o = np.zeros((2, n, nv))
+    dense_o = np.zeros((n_em, n, nv))
     for v in range(nv):
         ev = np.zeros(nv)
         ev[v] = 1.0
-        for e in range(2):
+        for e in range(n_em):
             O.set_sourcefn(e, ev)
         _, bo = O.brightness(locs, dirs, 10)
         dense_o[:, :, v] = bo[:, 0]
     floor = 1e-300 if prec == "f64" else 1e-35
-    stored = csr((indptr, indices, np.ones((2, len(indices)))), 0, nv).toarray() != 0
-    for e in range(2):
+    stored = csr((indptr, indices, np.ones((1, len(indices)))), 0, nv).toarray() != 0
+    for e in range(n_em):
         Wg = csr((indptr, indices, data), e, nv).toarray()
         Wo = dense_o[e]
         assert not (np.abs(Wo) > floor)[~stored].any(), "an oracle nonzero is not a stored entry"

@@ -190,8 +190,20 @@ def test_production_size_one_context(synth, binding, monkeypatch):
     assert G.ctx.kernel_ms(binding.PH_SOLVE)[1] <= 5                   # the one-launch preconditioned GMRES
     steps = G.last_solve_steps()
     assert 3 <= steps <= 100
-    S, res = G.vectors()["S"].copy(), G.ctx.residual(0)
+    v = G.vectors()
+    S, S0, res = v["S"].copy(), v["S0"], G.ctx.residual(0)
     assert res < 1e-12
+    # the adjoint on the same K (a 4.37 GB K^T): the host residual of (I - K)^T lam = r from the downloaded K, and
+    # r . S = lam . S0 against the GMRES S
+    r = np.random.default_rng(29).uniform(-1.0, 1.0, (2, G.n_el))
+    lam, adj_steps, _ = G.solve_adjoint(r)
+    K = G.K()
+    assert np.abs(lam - lam @ K - r).max() <= 1e-12 * np.abs(r).max()
+    del K
+    for k in range(2):
+        assert abs(r[k] @ S - lam[k] @ S0) <= 1e-10 * np.abs(r[k]).dot(np.abs(S))
+    # A^T has the spectrum of A, and the preconditioner's blocks are the transposed ones: about the forward's steps
+    assert (np.abs(adj_steps - steps) <= 0.2 * steps).all(), (adj_steps, steps)
     monkeypatch.setenv("B200RT_SOLVER", "lu")
     G.solve()
     assert dev(S, G.vectors()["S"]) < 1e-9

@@ -48,6 +48,28 @@ def test_mirror_rays_cross_the_same_voxels(synth, oraclebind, shape):
     assert pairs == scn.n_vox * nt * (nph // 2)
 
 
+def test_plane_cone_breaks_the_premise(synth, oraclebind):
+    """an odd n_sb puts an SZA boundary at 90 degrees, a cone that is the plane z = 0 to rounding: near mirror pairs
+    cross different voxels beside it, so upload_grid (grid_host.cpp) folds only bit-equal pairs on such grids"""
+    scn = synth.make_scenario(20, 13, 6, 8, n_em=1)
+    O = oraclebind.OracleModel(scn, "f64")
+    assert abs(np.cos(O.grid()["sza_boundaries"][(scn.n_sb - 1) // 2])) < 1e-6
+    nt, nph, ns = scn.n_theta, scn.n_phi, scn.n_sb - 1
+    ln, eb, ent, dist = O.traverse_voxel_rays()
+    off = np.concatenate([[0], np.cumsum(ln)])
+    differ = 0
+    for v in range(scn.n_vox):
+        for i in range(nt):
+            for j in range(nph // 2):
+                a = (v * nt + i) * nph + j
+                b = (v * nt + i) * nph + nph - 1 - j
+                ea, eb_ = set(ent[off[a]:off[a + 1]]), set(ent[off[b]:off[b + 1]])
+                if ln[a] != ln[b] or ea != eb_:
+                    differ += 1
+                    assert all(x % ns in (ns // 2 - 1, ns // 2) for x in ea ^ eb_ if x >= 0), (v, i, j)
+    assert differ > 0
+
+
 # ------------------------------------------------------------------ CPU: the fold rule
 @pytest.mark.parametrize("n_phi", [2, 4, 6, 12, 16, 32, 64, 128, 256, 512])
 @pytest.mark.parametrize("raymethod", [0, 1])
@@ -126,6 +148,19 @@ def test_folded_singlet_build_matches_oracle(synth, binding, oraclebind, prec):
         vo, vg = O.vectors(e), G.vectors(e, want_S=False)
         for k in ("S0", "tau_species_ss", "tau_absorber_ss"):
             assert rel_err(vo[k], vg[k], floor=UNDERFLOW[prec]) < tol, k
+
+
+@pytest.mark.gpu
+def test_plane_cone_grid_build_matches_oracle(synth, binding, oraclebind):
+    """20x13x6x8: an SZA boundary at 90 degrees, so only bit-equal pairs fold and every other ray is marched"""
+    scn = synth.make_scenario(20, 13, 6, 8, n_em=1, sza_T_contrast=0.1)
+    O = oraclebind.OracleModel(scn, "f64")
+    G = binding.GpuModel(scn, "f64")
+    O.build_rows()
+    G.build_rows()
+    Ko, Kg = O.K(0), G.K(0)
+    assert np.array_equal(np.abs(Ko) > 1e-290, np.abs(Kg) > 1e-290)
+    assert rel_err(np.where(np.abs(Ko) > 1e-290, Ko, 0), np.where(np.abs(Kg) > 1e-290, Kg, 0)) < TOL["f64"]
 
 
 @pytest.mark.gpu
